@@ -312,6 +312,32 @@ def mix_stats(env, stride, torch, steps: int = 64) -> dict:
             "ply_min_q1_median_q3_max": [int(x) for x in q.tolist()], "sampled_plies": steps}
 
 
+DUMP_SAMPLE_GAMES = 256  # planes + mask of 256 games: 29 MB of the 462 MB a step writes
+
+
+def snapshot_outputs(env) -> dict:
+    """What the timed step hands its caller, copied on the device (no host round trip between timed regions): the board
+    records after the move, legal-move counts, status words, game ids and plies of every game, and the f32 planes and
+    mask (of the positions before the move) of a fixed, seeded sample of games, whose indices go to sample_games."""
+    import numpy as np
+    import torch
+    rows = np.sort(np.random.default_rng(SEED).choice(env.n, DUMP_SAMPLE_GAMES, replace=False))
+    idx = torch.from_numpy(rows).to(env.device)
+    return {"boards": env.boards.clone(), "counts": env.counts.clone(), "status": env.status.clone(),
+            "game": env.game.clone(), "ply": env.ply.clone(), "planes": env.planes_buffer().index_select(0, idx),
+            "mask": env.mask_buffer().index_select(0, idx), "sample_games": idx}
+
+
+def write_outputs(snapshot: dict, out_dir: str) -> None:
+    """snapshot_outputs() as DIR/<name>.npy: float32 for the f32 tensors and the u8 board records, float64 for the
+    integers (all exact)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in snapshot.items():
+        a = t.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype in (np.float32, np.uint8) else np.float64))
+
+
 def run_ours(args) -> None:
     import numpy as np
     import torch
@@ -374,6 +400,8 @@ def run_ours(args) -> None:
     clocks = sampler.stop() if rank == 0 else None
     ms = e0.elapsed_time(e1)
     positions_a = env.counters.clone()
+    # region A's last step, copied on the device here and written to files after the last timed leg
+    outputs = snapshot_outputs(env) if args.dump_outputs and rank == 0 else None
     # ---- timed region B (the dominant kernel's launch duration): the same K steps again with CUDA events around
     #      every expand_kernel / rules_kernel launch on the streams they run on (fpc_profile_*).  Kept out of region A
     #      because the instrumentation is not free: four timestamped event records per step drain the internal streams
@@ -608,6 +636,8 @@ def run_ours(args) -> None:
                 shard["note"] = ("one GPU's share of configs[4] (8,192 games x 800 simulations): compare with `mcts` of "
                                  "the runs at N = 2, 4, 8, which sum this over the ranks; fp32 is a 100-simulation sample")
                 out["mcts_configs4_shard"] = shard
+        if outputs is not None:
+            write_outputs(outputs, args.dump_outputs)
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
@@ -769,7 +799,7 @@ def perft_leg(local: int) -> dict:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=400)
+    ap.add_argument("--steps", type=int, default=400, help="timed steps per trial")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -777,7 +807,14 @@ def main():
     ap.add_argument("--no-dropin", action="store_true")
     ap.add_argument("--ff", type=int, default=FAST_FORWARD,
                     help="untimed rules-only plies that spread the resident games over whole games (profiling runs shorten it)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last step of the headline timed region computed as DIR/<name>.npy (rank 0's games; "
+                         "planes and mask of a fixed sample of them), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
