@@ -5,6 +5,7 @@
 #include <math_constants.h>
 #include <stdint.h>
 
+#include <cfloat>
 #include <string>
 
 #include "../../include/fpc.h"
@@ -252,8 +253,10 @@ __global__ void __launch_bounds__(EXP_THREADS, 8) tree_expand_backup_kernel(cons
       }
     }
     // ---- softmax over the whole action space (mcts.py:67): ONE streaming pass, online max / sum; four independent
-    //      16-byte loads per thread and iteration keep enough bytes in flight to stream at the HBM rate -------------
-    float m = -CUDART_INF_F, s = 0.0f;
+    //      16-byte loads per thread and iteration keep enough bytes in flight to stream at the HBM rate.  The running
+    //      maximum starts at -FLT_MAX, not -inf: a group of -inf logits (a masked policy) then rescales by
+    //      exp(-inf - -FLT_MAX) = 0 instead of exp(-inf - -inf) = NaN, and -inf entries get a zero prior ----------
+    float m = -FLT_MAX, s = 0.0f;
     const float4 *lg4 = reinterpret_cast<const float4 *>(lg);
     constexpr int N4 = G::ASZ / 4;
     int i = tid;

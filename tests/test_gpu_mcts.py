@@ -10,6 +10,7 @@ import numpy as np
 import pytest
 import torch
 
+from alphazero_4_player_chess_b200._lib import FPC_MAX_MOVES, FpcError
 from alphazero_4_player_chess_b200.fen import start_record
 from alphazero_4_player_chess_b200.geometry import GEOMETRIES
 from alphazero_4_player_chess_b200.mcts import BatchedMCTS
@@ -48,23 +49,31 @@ def test_against_reference_mcts_fixtures(R, case):
     assert m.n_nodes.cpu().numpy().tolist() == z[f"{case}_n_nodes"].tolist()
 
 
-@pytest.mark.parametrize("name,R,n_games,sims", [("STANDARD", 14, 24, 48), ("EIGHT_SIMPLE", 8, 32, 80), ("TEN", 10, 16, 40)])
-@pytest.mark.parametrize("batch_rotation", [True, False])
-def test_whole_trees_match_the_oracle(name, R, n_games, sims, batch_rotation):
-    g = GEOMETRIES[R]
+def search_roots(name, R, n_games):
     o = oracle_for(R)
     pool = mixed_positions(name, 600)
     # late positions: short games at 8x8 put terminal leaves (root dropping) inside the search horizon
     roots = np.ascontiguousarray(pool[len(pool) // 3:: max(1, len(pool) // (2 * n_games))][:n_games])
-    roots = np.stack([r for r in roots if o.game_result(r)[0] == 0])
+    return np.stack([r for r in roots if o.game_result(r)[0] == 0])
+
+
+@pytest.mark.parametrize("name,R,n_games,sims", [("STANDARD", 14, 24, 48), ("EIGHT_SIMPLE", 8, 32, 80), ("TEN", 10, 16, 40),
+                                                 ("THIRTEEN", 13, 16, 40)])
+@pytest.mark.parametrize("batch_rotation", [True, False])
+def test_whole_trees_match_the_oracle(name, R, n_games, sims, batch_rotation):
+    o = oracle_for(R)
+    roots = search_roots(name, R, n_games)
     trees = oracle_search(o, FakeNet(R), roots, 3, sims, batch_rotation=batch_rotation)
     m = run_gpu(R, roots, sims, batch_rotation)
+    assert_trees_equal(m, trees)
+    print(f"{name} rot={batch_rotation}: {len(trees)} games, {int(m.n_nodes.sum())} nodes, {int(m.dropped.sum())} dropped roots")
+
+
+def assert_trees_equal(m, trees):
     n_nodes = m.n_nodes.cpu().numpy()
     parent, move_flat, visits = m.parent.cpu().numpy(), m.move_flat.cpu().numpy(), m.visits.cpu().numpy()
     value_sum, prior = m.value_sum.cpu().numpy(), m.prior.cpu().numpy()
     first_child, n_children = m.first_child.cpu().numpy(), m.n_children.cpu().numpy()
-    dropped = m.dropped.cpu().numpy()
-    n_dropped = 0
     for gi, t in enumerate(trees):
         nn = len(t.parent)
         assert n_nodes[gi] == nn, gi
@@ -78,8 +87,67 @@ def test_whole_trees_match_the_oracle(name, R, n_games, sims, batch_rotation):
             assert n_children[gi, node] == len(ch)
             if ch:
                 assert first_child[gi, node] == ch[0] and ch == list(range(ch[0], ch[0] + len(ch)))
-        n_dropped += int(dropped[gi])
-    print(f"{name} rot={batch_rotation}: {len(trees)} games, {int(n_nodes.sum())} nodes, {n_dropped} dropped roots")
+
+
+class SharpMaskedNet(FakeNet):
+    """FakeNet with logits x 8 (spread 64, so legal priors range down to e^-64) and -inf on every entry whose index is
+    below 4 modulo 128 and on the eight planes no move reaches (8(R-1)+8 and up).  The first pattern covers the first
+    16-value group lane 0 of every warp of tree_expand_backup_kernel streams, which is where a running maximum that
+    starts at -inf turns into NaN.  At x16 the spread (128) would pass the f32 exponential's normal range (~87): priors
+    then go through denormal intermediates, whose absolute precision no relative tolerance between two f32 pipelines
+    can follow."""
+
+    def __call__(self, encoded):
+        logits, value = super().__call__(encoded)
+        logits = logits * 8.0
+        logits[:, (torch.arange(self.ASZ, device=logits.device) % 128) < 4] = -float("inf")
+        logits[:, 8 * self.R * self.R * self.R:] = -float("inf")
+        return logits, value
+
+
+@pytest.mark.parametrize("batch_rotation", [True, False])
+def test_sharp_masked_network_trees_match_the_oracle(batch_rotation):
+    """A policy with -inf entries and a wide logit spread (before the soft-max started its running maximum at -FLT_MAX,
+    every child got a NaN prior here and the next descent stopped the search with error bit 4)."""
+    R, sims = 14, 48
+    o = oracle_for(R)
+    roots = search_roots("STANDARD", R, 24)
+    trees = oracle_search(o, SharpMaskedNet(R), roots, 3, sims, batch_rotation=batch_rotation)
+    for t in trees:  # every expanded leaf kept an unmasked legal move: finite priors that sum to 1
+        for node, ch in enumerate(t.children):
+            if ch:
+                pr = np.array([t.prior[c] for c in ch])
+                assert len(ch) <= FPC_MAX_MOVES and np.isfinite(pr).all() and abs(pr.sum() - 1.0) < 1e-5, node
+    net = SharpMaskedNet(R, device="cuda")
+    m = BatchedMCTS(R, len(roots), net, {"C": 3, "num_searches": sims}, batch_rotation=batch_rotation)
+    m.search(torch.from_numpy(roots))
+    torch.cuda.synchronize()
+    assert_trees_equal(m, trees)
+    print(f"sharp masked rot={batch_rotation}: {len(trees)} games, {int(m.n_nodes.sum())} nodes")
+
+
+def test_fully_underflowing_policy_stops_the_search():
+    """Every legal logit 200 below the row's maximum (which sits on a plane no move reaches): the soft-max underflows to 0
+    on every legal move and the renormalisation divides 0 by 0, in the reference's f32 pipeline as in the kernel.  The
+    leaf gets its children with NaN priors, the next descent can select none of them, and the search raises instead of
+    returning a tree."""
+    R = 8
+    g = GEOMETRIES[R]
+
+    def net(planes):
+        logits = torch.zeros((planes.shape[0], g.action_space_size), device=planes.device)
+        logits[:, -1] = 200.0
+        return logits, torch.zeros((planes.shape[0], 1), device=planes.device)
+
+    roots = np.stack([start_record("EIGHT_SIMPLE")] * 3)
+    m = BatchedMCTS(R, 3, net, {"C": 3, "num_searches": 3})
+    with pytest.raises(FpcError, match="tree error bits 0x4"):
+        m.search(torch.from_numpy(roots))
+    flat, _, prior, cnt = m.root_children()
+    n_legal = len(set(oracle_for(R).move_flat_index(mv) for mv in oracle_for(R).legal_moves(roots[0])))
+    assert cnt.tolist() == [n_legal] * 3
+    assert torch.isnan(prior[:, :n_legal]).all()
+    assert (m.error == 4).all() and (m.leaf == -1).all() and (m.dropped == 1).all()
 
 
 def test_batch_rotation_ignores_terminal_leaves():
