@@ -16,6 +16,7 @@ STATUS_RESULT_MASK, STATUS_IN_CHECK, STATUS_CAN_TAKE_KING = 0x3, 0x100, 0x200
 STATUS_OVERFLOW, STATUS_FINISHED, STATUS_CHECK = 0x400, 0x800, 0x1000
 FLAG_ASYNC_DENSE = 1
 FLAG_INCREMENTAL = 2
+TREE_ADVANCE_MAX_NODE_CAP = 524288
 
 _vp, _i, _u64 = C.c_void_p, C.c_int, C.c_uint64
 
@@ -50,6 +51,7 @@ SIGNATURES = {
     "fpc_playout_step_tracked": (_i, [_vp, _i, _vp, _i, _u64, _vp, _vp, _vp, _i, _u64, _vp, _vp, _vp, _vp, _vp, _i, _vp,
                                       _vp, _i, _vp]),
     "fpc_tree_reset": (_i, [_vp, _vp, _vp]),
+    "fpc_tree_advance": (_i, [_vp, _vp, _vp, C.c_int32, C.c_int32, _vp, _vp]),
     "fpc_tree_select": (_i, [_vp, _i, _vp, _i, _vp, _vp]),
     "fpc_tree_expand_backup": (_i, [_vp, _vp, _vp, _vp]),
     "fpc_ctx_create": (_vp, [_i, _i, _i]),

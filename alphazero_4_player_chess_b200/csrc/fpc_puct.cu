@@ -25,9 +25,10 @@ int cuda_check(cudaError_t e, const char *what);
 constexpr int SEL_WARPS = 4;
 constexpr int ERR_NODE_CAP = 1, ERR_BOARD_CAP = 2, ERR_NO_CHILD = 4, ERR_MOVE = 8;
 
+// A fresh root for game g: node 0 = `root` (one record), visit_count 1, no children; per-game state cleared.  Run by
+// every thread of one CTA.
 template <class G>
-__global__ void __launch_bounds__(256) tree_reset_kernel(const fpc_tree T, const uint8_t *roots) {
-  const int g = blockIdx.x;
+__device__ __forceinline__ void write_fresh_root(const fpc_tree &T, int g, const uint8_t *root) {
   const size_t slab = (size_t)g * T.node_cap;
   if (threadIdx.x == 0) {
     T.parent[slab] = -1;
@@ -44,8 +45,218 @@ __global__ void __launch_bounds__(256) tree_reset_kernel(const fpc_tree T, const
     T.dropped[g] = 0;
     T.error[g] = 0;
   }
-  for (int i = threadIdx.x; i < G::REC; i += blockDim.x)
-    T.boards[(size_t)g * T.board_cap * G::REC + i] = roots[(size_t)g * G::REC + i];
+  for (int i = threadIdx.x; i < G::REC; i += blockDim.x) T.boards[(size_t)g * T.board_cap * G::REC + i] = root[i];
+}
+
+template <class G>
+__global__ void __launch_bounds__(256) tree_reset_kernel(const fpc_tree T, const uint8_t *roots) {
+  write_fresh_root<G>(T, blockIdx.x, roots + (size_t)blockIdx.x * G::REC);
+}
+
+// ---- re-rooting on the played move (fpc_tree_advance), one CTA per game -------------------------------------------
+// Invariants of a slab written by the kernels of this file, which the in-place compaction relies on:
+//  (1) parent[i] < i for every node but the root: children are appended at n_nodes when their parent is expanded;
+//  (2) hence the new root c has the smallest index of its subtree, and renumbering the kept nodes in ascending order of
+//      their old index maps c to 0 and never raises an index (new <= old);
+//  (3) a node is materialised before it can be expanded, so c's board slot, when it has one, is the smallest among the
+//      subtree's boards and lands in slot 0; a c without a board was never selected and has no descendants.
+// A gather in ascending chunks of old indices, each chunk read completely before a barrier and written after it, is
+// therefore safe in place: every write lands at or below the chunk it came from, never on an entry not yet read.
+// The old -> new map is a bitmap of the kept entries plus an exclusive prefix count per 32-entry word in dynamic shared
+// memory (node_cap / 4 bytes); after the nodes it is rebuilt over the board slots.
+constexpr int ADV_THREADS = 256, ADV_WARPS = ADV_THREADS / 32;
+constexpr int ADV_ITEMS = 4;                          // nodes per thread and chunk: four independent loads in flight
+constexpr int ADV_CHUNK = ADV_THREADS * ADV_ITEMS;    // 1,024 nodes = 32 map words
+
+__device__ __forceinline__ bool map_bit(const uint32_t *bits, int b) { return (bits[b >> 5] >> (b & 31)) & 1u; }
+
+// new index of kept entry b = the number of kept entries below it
+__device__ __forceinline__ int map_rank(const uint32_t *bits, const uint32_t *pre, int b) {
+  return (int)pre[b >> 5] + __popc(bits[b >> 5] & ((1u << (b & 31)) - 1u));
+}
+
+// pre[w] = exclusive prefix sum of popc(bits[w]) for w < nw; returns the total to every thread
+__device__ int scan_map(const uint32_t *bits, uint32_t *pre, int nw, int *red) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int carry = 0;
+  for (int base = 0; base < nw; base += ADV_THREADS) {
+    const int w = base + threadIdx.x;
+    const int v = w < nw ? __popc(bits[w]) : 0;
+    int x = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int y = __shfl_up_sync(FULL, x, o);
+      if (lane >= o) x += y;
+    }
+    if (lane == 31) red[warp] = x;
+    __syncthreads();
+    int before = 0, tot = 0;
+#pragma unroll
+    for (int k = 0; k < ADV_WARPS; ++k) {
+      const int n = red[k];
+      before += k < warp ? n : 0;
+      tot += n;
+    }
+    if (w < nw) pre[w] = carry + before + x - v;
+    carry += tot;
+    __syncthreads();
+  }
+  return carry;
+}
+
+template <class G>
+__global__ void __launch_bounds__(ADV_THREADS) tree_advance_kernel(const fpc_tree T, const int32_t *actions, const uint8_t *roots,
+                                                                   int max_nodes, int max_boards, int32_t *kept_out) {
+  extern __shared__ uint32_t s_map[];  // [map_words] bits, then [map_words] prefix counts
+  __shared__ int red[ADV_WARPS];
+  __shared__ int s_c, s_mat;
+  const int map_words = (T.node_cap + 31) >> 5;
+  uint32_t *bits = s_map, *pre = s_map + map_words;
+  const int g = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const size_t slab = (size_t)g * T.node_cap;
+  const uint8_t *root = roots + (size_t)g * G::REC;
+  uint4 *pool = reinterpret_cast<uint4 *>(T.boards + (size_t)g * T.board_cap * G::REC);
+  constexpr int V = G::REC / 16;  // 16-byte words per record
+  const int action = actions[g];
+  const int nn = T.n_nodes[g], nb_old = T.n_boards[g];
+  const int nc0 = T.n_children[slab], fc0 = T.first_child[slab];
+  if (tid == 0) s_c = -1, s_mat = 0;
+  __syncthreads();
+  // 1. c = the root child that made the move (the flat indices of siblings are unique: promotions share one child)
+  if (action >= 0)
+    for (int i = tid; i < nc0; i += ADV_THREADS)
+      if (T.move_flat[slab + fc0 + i] == action) s_c = fc0 + i;
+  __syncthreads();
+  const int c = s_c;
+  bool keep = c > 0;
+  int c_slot = -1;
+  if (keep) {  // uniform over the CTA
+    // c's board, when it has one, must be the caller's position (a full move with promotion is not the index-built one)
+    c_slot = T.board_idx[slab + c];
+    bool diff = false;
+    if (c_slot >= 0)
+      for (int i = tid; i < V; i += ADV_THREADS) {
+        const uint4 a = pool[(size_t)c_slot * V + i], b = reinterpret_cast<const uint4 *>(root)[i];
+        diff |= a.x != b.x || a.y != b.y || a.z != b.z || a.w != b.w;
+      }
+    keep = !__syncthreads_or(diff);
+  }
+  // 2. subtree membership over [c, nn) (offsets r = i - c), in ascending chunks: a node's parent lies in an earlier chunk
+  //    (its bit is final) or in this one, where the walk climbs on until it leaves the chunk or meets c.  Every warp's
+  //    ballot is one map word.
+  const int span = keep ? nn - c : 0;
+  for (int base = 0; base < span; base += ADV_CHUNK) {
+    int par[ADV_ITEMS], bix[ADV_ITEMS];
+#pragma unroll
+    for (int q = 0; q < ADV_ITEMS; ++q) {
+      const int r = base + q * ADV_THREADS + tid;
+      par[q] = r < span ? T.parent[slab + c + r] : -1;
+      bix[q] = r < span ? T.board_idx[slab + c + r] : -1;
+    }
+    int n_mat = 0;
+#pragma unroll
+    for (int q = 0; q < ADV_ITEMS; ++q) {
+      const int r = base + q * ADV_THREADS + tid;
+      bool in = r == 0;
+      if (r > 0 && r < span) {
+        int p = par[q];
+        while (p >= c + base && p != c) p = T.parent[slab + p];
+        in = p == c || (p > c && map_bit(bits, p - c));
+      }
+      const unsigned w = __ballot_sync(FULL, in);
+      n_mat += __popc(__ballot_sync(FULL, in && bix[q] >= 0));
+      const int word = (base + q * ADV_THREADS) / 32 + warp;
+      if (lane == 0 && word * 32 < span) bits[word] = w;
+    }
+    if (lane == 0 && n_mat) atomicAdd(&s_mat, n_mat);
+    __syncthreads();
+  }
+  int kept = 0;
+  if (keep) {
+    kept = scan_map(bits, pre, (span + 31) >> 5, red);
+    keep = kept <= max_nodes && s_mat <= max_boards;
+  }
+  if (!keep) {  // every read of the old tree is behind a barrier by now
+    write_fresh_root<G>(T, g, root);
+    if (tid == 0 && kept_out) kept_out[g] = 0;
+    return;
+  }
+  // 3. gather the kept nodes in place; parent and first_child through the map, the rest unchanged but for the root
+  for (int base = 0; base < span; base += ADV_CHUNK) {
+    int dst[ADV_ITEMS], par[ADV_ITEMS], fc[ADV_ITEMS], nch[ADV_ITEMS], vis[ADV_ITEMS], mv[ADV_ITEMS], bix[ADV_ITEMS];
+    double vs[ADV_ITEMS];
+    float pr[ADV_ITEMS];
+#pragma unroll
+    for (int q = 0; q < ADV_ITEMS; ++q) {
+      const int r = base + q * ADV_THREADS + tid;
+      dst[q] = -1;
+      if (r < span && map_bit(bits, r)) {
+        const size_t i = slab + c + r;
+        dst[q] = map_rank(bits, pre, r);
+        par[q] = T.parent[i], fc[q] = T.first_child[i], nch[q] = T.n_children[i], vis[q] = T.visits[i];
+        mv[q] = T.move_flat[i], bix[q] = T.board_idx[i], vs[q] = T.value_sum[i], pr[q] = T.prior[i];
+      }
+    }
+#pragma unroll
+    for (int q = 0; q < ADV_ITEMS; ++q) {
+      if (dst[q] < 0) continue;
+      if (dst[q] == 0) {
+        par[q] = -1, mv[q] = -1, pr[q] = 0.0f;
+      } else {
+        par[q] = map_rank(bits, pre, par[q] - c);
+      }
+      fc[q] = nch[q] > 0 ? map_rank(bits, pre, fc[q] - c) : 0;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int q = 0; q < ADV_ITEMS; ++q) {
+      if (dst[q] < 0) continue;
+      const size_t j = slab + dst[q];
+      T.parent[j] = par[q], T.first_child[j] = fc[q], T.n_children[j] = nch[q], T.visits[j] = vis[q];
+      T.move_flat[j] = mv[q], T.board_idx[j] = bix[q], T.value_sum[j] = vs[q], T.prior[j] = pr[q];
+    }
+    __syncthreads();
+  }
+  // 4. boards: the map is rebuilt over the slots the kept nodes own and the boards gathered the same way.  An
+  //    unmaterialised c owns none of them; it gets the caller's board in slot 0 and every kept slot moves up by one.
+  const int off = c_slot < 0;
+  const int n_slots = min(nb_old, map_words * 32);
+  const int slot_words = (n_slots + 31) >> 5;
+  for (int w = tid; w < slot_words; w += ADV_THREADS) bits[w] = 0;
+  __syncthreads();
+  for (int j = tid; j < kept; j += ADV_THREADS) {
+    const int b = T.board_idx[slab + j];
+    if (b >= 0 && b < n_slots) atomicOr(&bits[b >> 5], 1u << (b & 31));
+  }
+  __syncthreads();
+  const int kept_boards = scan_map(bits, pre, slot_words, red);
+  for (int j = tid; j < kept; j += ADV_THREADS) {
+    const int b = T.board_idx[slab + j];
+    T.board_idx[slab + j] = j == 0 ? 0 : b >= 0 ? off + map_rank(bits, pre, b) : -1;
+  }
+  constexpr int BPC = ADV_THREADS / V;  // boards per chunk
+  for (int base = 0; base < n_slots; base += BPC) {
+    const int s = base + tid / V, part = tid % V;
+    int dst = -1;
+    uint4 v;
+    if (tid < BPC * V && s < n_slots && map_bit(bits, s)) {
+      v = pool[(size_t)s * V + part];
+      dst = off + map_rank(bits, pre, s);
+    }
+    __syncthreads();
+    if (dst >= 0) pool[(size_t)dst * V + part] = v;
+    __syncthreads();
+  }
+  if (off)
+    for (int i = tid; i < V; i += ADV_THREADS) pool[i] = reinterpret_cast<const uint4 *>(root)[i];
+  if (tid == 0) {
+    T.n_nodes[g] = kept;
+    T.n_boards[g] = kept_boards + off;
+    T.leaf[g] = -1;
+    T.dropped[g] = 0;
+    T.error[g] = 0;
+    if (kept_out) kept_out[g] = kept;
+  }
 }
 
 // Node::ChooseLeaf's descent (node.cpp:21-26) + Node::SelectChild (node.cpp:49-78).
@@ -408,6 +619,16 @@ static int check_tree(const fpc_tree *t, const char *who) {
   return FPC_OK;
 }
 
+template <class G>
+static int launch_advance(const fpc_tree &t, const int32_t *actions, const uint8_t *roots, int max_nodes, int max_boards,
+                          int32_t *kept, cudaStream_t st) {
+  const size_t smem = 2 * sizeof(uint32_t) * (size_t)((t.node_cap + 31) / 32);
+  if (smem > 48 * 1024)
+    CK(cudaFuncSetAttribute(tree_advance_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  tree_advance_kernel<G><<<t.n_games, ADV_THREADS, smem, st>>>(t, actions, roots, max_nodes, max_boards, kept);
+  return cuda_check(cudaGetLastError(), "tree_advance_kernel launch");
+}
+
 }  // namespace fpc
 
 using namespace fpc;
@@ -422,6 +643,22 @@ int fpc_tree_reset(const fpc_tree *t, const uint8_t *d_root_boards, void *stream
   cudaStream_t st = (cudaStream_t)stream;
   FPC_DISPATCH(t->R, (tree_reset_kernel<G><<<t->n_games, 256, 0, st>>>(*t, d_root_boards)));
   return cuda_check(cudaGetLastError(), "tree_reset_kernel launch");
+}
+
+int fpc_tree_advance(const fpc_tree *t, const int32_t *d_actions, const uint8_t *d_root_boards, int32_t max_keep_nodes,
+                     int32_t max_keep_boards, int32_t *d_kept, void *stream) {
+  int rc = check_tree(t, "fpc_tree_advance");
+  if (rc != FPC_OK) return rc;
+  if (t->node_cap > FPC_TREE_ADVANCE_MAX_NODE_CAP)
+    return fail(FPC_ERR_ARG, "fpc_tree_advance: node_cap " + std::to_string(t->node_cap) + " above " +
+                                 std::to_string(FPC_TREE_ADVANCE_MAX_NODE_CAP));
+  if (max_keep_nodes < 0 || max_keep_boards < 0) return fail(FPC_ERR_ARG, "fpc_tree_advance: negative limit");
+  if (t->n_games == 0) return FPC_OK;
+  if (!d_actions || !d_root_boards) return fail(FPC_ERR_ARG, "fpc_tree_advance: null actions / roots");
+  if (reinterpret_cast<uintptr_t>(d_root_boards) & 15) return fail(FPC_ERR_ARG, "root boards must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  FPC_DISPATCH(t->R, (rc = launch_advance<G>(*t, d_actions, d_root_boards, max_keep_nodes, max_keep_boards, d_kept, st)));
+  return rc;
 }
 
 int fpc_tree_select(const fpc_tree *t, int batch_rotation, float *d_planes, int flags, fpc_dense_track *track, void *stream) {

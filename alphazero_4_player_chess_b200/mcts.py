@@ -18,16 +18,22 @@ from ._lib import FPC_MAX_MOVES, TreeDesc, check
 from .geometry import GEOMETRIES, NUM_STATE_CHANNELS
 
 ERR_NODE_CAP, ERR_BOARD_CAP, ERR_NO_CHILD, ERR_MOVE = 1, 2, 4, 8
+# node slots per simulation: a leaf adds at most FPC_MAX_MOVES children; the legal-move average is ~19-38 at 14x14
+NODES_PER_SIM = 96
 
 
 class BatchedMCTS:
     def __init__(self, R: int, n_games: int, neural_net, args: dict, device: str | torch.device = "cuda",
-                 batch_rotation: bool = False, node_cap: int | None = None, cuda_graph: bool = False):
+                 batch_rotation: bool = False, node_cap: int | None = None, cuda_graph: bool = False,
+                 reuse_tree: bool = False):
         """args: the reference's dict (`alphazero.py:291-306`): uses "C" and "num_searches".
         batch_rotation=True reproduces the reference bit for bit (a whole leaf batch is rotated by the
         colour of its first expandable state); False rotates every leaf by its own side to move.
         cuda_graph=True captures one whole simulation (select -> network -> expand/backup) in a CUDA graph after
-        three eager ones and replays it: the ~70 launches of a simulation become one."""
+        three eager ones and replays it: the ~70 launches of a simulation become one.
+        reuse_tree=True sizes the default capacities for `advance` (keeping the played move's subtree between moves):
+        room for a kept subtree plus a full new search.  It changes nothing else; `advance` works either way, it only
+        keeps less with the smaller default arenas."""
         self.geom = GEOMETRIES[R]
         self.R, self.n = R, int(n_games)
         self.net = neural_net
@@ -40,9 +46,10 @@ class BatchedMCTS:
         self._graph = None
         self.L = _lib.lib()
         sims = int(args["num_searches"])
-        # a leaf adds at most FPC_MAX_MOVES children; the legal-move average is ~19-38 at 14x14
-        self.node_cap = int(node_cap) if node_cap else 1 + sims * 96
-        self.board_cap = sims + 2
+        reuse = 2 if reuse_tree else 1
+        self.node_cap = int(node_cap) if node_cap else 1 + reuse * NODES_PER_SIM * sims
+        self.board_cap = reuse * sims + 2
+        self._has_tree = False
         n, nc, dev = self.n, self.node_cap, self.device
         i32 = dict(dtype=torch.int32, device=dev)
         self.parent = torch.empty((n, nc), **i32)
@@ -88,6 +95,29 @@ class BatchedMCTS:
         with torch.cuda.device(self.device):
             check(self.L.fpc_tree_reset(C.byref(self.desc), roots.data_ptr(), self._stream()))
         self._roots = roots  # keep alive until the kernel has run
+        self._has_tree = True
+
+    def advance(self, actions: torch.Tensor, root_boards: torch.Tensor) -> torch.Tensor:
+        """Re-root every game's tree on the root child that played actions[g] (i32 flat index; -1 = none), keeping
+        that child's subtree -- its visits, value sums, priors and boards -- for the next search.  root_boards = the
+        positions after the move, made with the index-built move (`BatchedEnv.make_index`).  A game whose child is
+        missing, whose subtree would leave less headroom than a fresh tree has (more than node_cap - 96 * sims nodes or
+        board_cap - sims boards) or whose child's board differs from root_boards[g] gets a fresh root instead, as
+        reset() makes it.  Returns kept [n] i32: the nodes carried over per game, 0 for a fresh root."""
+        if not self._has_tree:
+            raise _lib.FpcError("advance() needs a tree: call reset() or search(root_boards) first")
+        acts = actions.to(self.device, torch.int32).contiguous()
+        roots = root_boards.to(self.device, torch.uint8).contiguous()
+        assert acts.shape == (self.n,) and roots.shape == (self.n, self.geom.record_bytes)
+        sims = int(self.args["num_searches"])
+        max_nodes = max(0, self.node_cap - NODES_PER_SIM * sims)
+        max_boards = max(0, self.board_cap - sims)
+        kept = torch.empty(self.n, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.L.fpc_tree_advance(C.byref(self.desc), acts.data_ptr(), roots.data_ptr(), max_nodes, max_boards,
+                                          kept.data_ptr(), self._stream()))
+        self._roots, self._acts = roots, acts  # keep alive until the kernel has run
+        return kept
 
     def select(self) -> torch.Tensor:
         """Node.ChooseLeaf for every live game; returns the encoded leaf batch [n,24,R,R]."""
@@ -125,11 +155,16 @@ class BatchedMCTS:
         self.expand_backup(logits, value)
 
     @torch.no_grad()
-    def search(self, root_boards: torch.Tensor, record=None, check: bool = True) -> "BatchedMCTS":
-        """record: optional callable(sim, logits, value) called after every network forward (eager mode only), e.g.
+    def search(self, root_boards: torch.Tensor | None = None, record=None, check: bool = True) -> "BatchedMCTS":
+        """num_searches simulations from fresh roots at root_boards, or, with root_boards=None, on top of the current
+        trees (after advance(), or to add simulations to a finished search).
+        record: optional callable(sim, logits, value) called after every network forward (eager mode only), e.g.
         to keep the outputs of some games for a replay on the CPU oracle.  check: raise on tree errors (arena full ...)
         instead of leaving them in `self.error`."""
-        self.reset(root_boards)
+        if root_boards is not None:
+            self.reset(root_boards)
+        elif not self._has_tree:
+            raise _lib.FpcError("search(None) continues the current trees, but there are none: pass root_boards")
         sims = int(self.args["num_searches"])
         done = 0
         if self.cuda_graph and record is None:

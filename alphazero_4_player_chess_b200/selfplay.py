@@ -24,14 +24,19 @@ from .mcts import BatchedMCTS
 
 class SelfPlay:
     def __init__(self, R: int, n_games: int, neural_net, args: dict, start_record, device="cuda",
-                 batch_rotation: bool = False):
+                 batch_rotation: bool = False, reuse_tree: bool = False):
         """args: the reference's dict (`alphazero.py:291-306`); uses C, num_searches, temperature,
-        max_game_length, heuristic_weight."""
+        max_game_length, heuristic_weight.  reuse_tree=True keeps the played move's subtree for the next move's search
+        (`BatchedMCTS.advance`) where the reference starts every move from a fresh root: num_searches simulations are
+        still added per move, on top of the visits carried over, and the policy targets are the root children's visit
+        counts including those."""
         self.geom = GEOMETRIES[R]
         self.R, self.n, self.args = R, int(n_games), args
         self.device = torch.device(device)
         self.env = BatchedEnv(R, self.n, device=self.device)
-        self.mcts = BatchedMCTS(R, self.n, neural_net, args, device=self.device, batch_rotation=batch_rotation)
+        self.reuse_tree = bool(reuse_tree)
+        self.mcts = BatchedMCTS(R, self.n, neural_net, args, device=self.device, batch_rotation=batch_rotation,
+                                reuse_tree=self.reuse_tree)
         self.start = torch.as_tensor(start_record, dtype=torch.uint8)
         T = int(args["max_game_length"])
         i32 = dict(dtype=torch.int32, device=self.device)
@@ -69,7 +74,10 @@ class SelfPlay:
         losing_team = torch.full((n,), -1, dtype=torch.int64, device=self.device)
         self.hist_valid.zero_()
         for t in range(T):
-            self.mcts.reset(self.env.boards)
+            if self.reuse_tree and t > 0:
+                self.mcts.advance(actions, self.env.boards)
+            else:
+                self.mcts.reset(self.env.boards)
             self.mcts.dropped.copy_((~running).int())  # finished games take no part in the search
             for _ in range(int(self.args["num_searches"])):
                 planes = self.mcts.select()

@@ -201,6 +201,14 @@ int fpc_attack_maps(int R, const uint8_t *d_boards, int n, uint8_t *d_out, void 
  *
  * One simulation for all games = fpc_tree_select -> network forward on `d_planes` (PyTorch) ->
  * fpc_tree_expand_backup.
+ *
+ * Invariants of every slab the calls below write (fpc_tree_advance relies on them):
+ *   - parent[i] < i for every node but the root: children are appended at n_nodes when their parent is expanded,
+ *     so a node has the smallest index of its subtree;
+ *   - first_child = 0 and n_children = 0 for a node that is not expanded;
+ *   - a node is materialised (board_idx >= 0) before it is expanded, so its board slot is below those of its
+ *     descendants; slot 0 is the root's;
+ *   - n_boards <= n_nodes <= node_cap.
  */
 typedef struct fpc_tree {
   int32_t R, n_games, node_cap, board_cap;
@@ -232,6 +240,26 @@ typedef struct fpc_tree {
 
 /* Roots: node 0 of every game = d_root_boards[g], visit_count 1 (mcts.py:30), no children. */
 int fpc_tree_reset(const fpc_tree *t, const uint8_t *d_root_boards, void *stream);
+
+/* Tree reuse between moves (outside the reference, which builds a fresh Node per move, mcts.py:28-31): re-root every
+ * game's tree on the root child whose move_flat == d_actions[g], in place.  d_root_boards [n_games][record] (16-byte
+ * aligned) = the positions after the move, made with the index-built move (fpc_make_index).  The subtree of that child
+ * c is kept when c exists, the subtree has at most max_keep_nodes nodes and at most max_keep_boards materialised
+ * boards, and c's board (if materialised) is byte-equal to d_root_boards[g].  Then:
+ *   - the kept nodes are renumbered in ascending order of their old index (c becomes node 0); children stay
+ *     contiguous and in ascending flat order; parent and first_child are remapped; visits, value_sum, prior,
+ *     move_flat and n_children are unchanged, except that node 0 gets parent -1, move_flat -1, prior 0 and
+ *     board_idx 0;
+ *   - the kept boards are compacted in ascending order of their old slot and board_idx is remapped; slot 0 holds
+ *     d_root_boards[g];
+ *   - n_nodes / n_boards = the kept counts, leaf = -1, dropped = 0, error = 0.
+ * Otherwise (action -1, no such child, a limit exceeded, a board mismatch) the game gets a fresh root from
+ * d_root_boards[g], exactly as fpc_tree_reset writes it; that is not an error.  d_kept[g] (may be NULL) = the number
+ * of nodes carried over, 0 for a fresh root.  node_cap above FPC_TREE_ADVANCE_MAX_NODE_CAP (the old -> new index
+ * map lives in node_cap / 4 bytes of shared memory) and negative limits are FPC_ERR_ARG, before any launch. */
+#define FPC_TREE_ADVANCE_MAX_NODE_CAP 524288
+int fpc_tree_advance(const fpc_tree *t, const int32_t *d_actions, const uint8_t *d_root_boards, int32_t max_keep_nodes,
+                     int32_t max_keep_boards, int32_t *d_kept, void *stream);
 
 /* Node::ChooseLeaf (node.cpp:19-47) for every live game: descend with Node::SelectChild
  * (node.cpp:49-78: argmax of Q + C*sqrt(ln(sqrt(N))/(1+n))*P in double, first maximum wins),
