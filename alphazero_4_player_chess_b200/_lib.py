@@ -8,7 +8,8 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("FPC_LIB_PATH") or os.path.join(_HERE, "libfpc.so")  # FPC_LIB_PATH: diagnostics builds (tools/)
+# FPC_LIB_PATH loads another build of the library instead, e.g. to compare two builds with bench.py
+LIB_PATH = os.environ.get("FPC_LIB_PATH") or os.path.join(_HERE, "libfpc.so")
 
 FPC_MAX_MOVES = 300
 FPC_OK, FPC_ERR_ARG, FPC_ERR_CUDA, FPC_ERR_MOVE, FPC_ERR_OVERFLOW = 0, -1, -2, -3, -4

@@ -2,7 +2,6 @@
 // See include/fpc.h for the boundary and fpc_device.cuh for the rules.
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -10,12 +9,10 @@
 #include <vector>
 
 #include "../../include/fpc.h"
+#include "fpc_host.h"
 #include "fpc_rules.cuh"
 
 namespace fpc {
-
-int fail(int code, const std::string &msg);
-int cuda_check(cudaError_t e, const char *what);
 
 constexpr int WARPS_PER_BLOCK = 4;  // one warp per game
 constexpr int BLOCK_THREADS = WARPS_PER_BLOCK * 32;
@@ -32,19 +29,13 @@ static_assert(STATUS_IN_CHECK == FPC_STATUS_IN_CHECK && STATUS_CAN_TAKE_KING == 
                   STATUS_CHECK == FPC_STATUS_CHECK,
               "status bits of fpc_rules.cuh and include/fpc.h");
 
-#define CK(expr)                                   \
-  do {                                             \
-    int rc_ = cuda_check((expr), #expr);           \
-    if (rc_ != FPC_OK) return rc_;                 \
-  } while (0)
-
 // The rules kernel: one warp per game (fpc_rules.cuh).  Legal moves, result, the bit sets of the dense outputs,
 // and (playout) the move choice and make-move.  It touches only the board store and compact per-game outputs.
-template <class G, int WPB = WARPS_PER_BLOCK>
-__global__ void __launch_bounds__(WPB * 32) rules_kernel(const __grid_constant__ ObserveParams P) {
-  __shared__ RulesScratch<G> scratch[WPB];
+template <class G>
+__global__ void __launch_bounds__(BLOCK_THREADS) rules_kernel(const __grid_constant__ ObserveParams P) {
+  __shared__ RulesScratch<G> scratch[WARPS_PER_BLOCK];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  const int g = blockIdx.x * WPB + wib;
+  const int g = blockIdx.x * WARPS_PER_BLOCK + wib;
   if (g >= P.n) return;
   rules_warp<G>(P, scratch[wib], g, lane);
 }
@@ -219,18 +210,12 @@ static int side_state(SideState **out) {
   if (!S.side) {
     int least = 0, greatest = 0;
     CK(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-#ifdef FPC_EXPERIMENT
-    if (getenv("FPC_X_NOPRIO") && atoi(getenv("FPC_X_NOPRIO"))) greatest = least = 0;
-#endif
     CK(cudaStreamCreateWithPriority(&S.side, cudaStreamNonBlocking, least));
     CK(cudaStreamCreateWithPriority(&S.hi, cudaStreamNonBlocking, greatest));
-    // FPC_EVT (diagnostics): bit 0 expand_done, bit 1 rules_done, bit 2 fork created WITH timing
-    const char *evt_env = getenv("FPC_EVT");
-    const int evt = evt_env ? atoi(evt_env) : 0;
-    CK(cudaEventCreateWithFlags(&S.fork, (evt & 4) ? cudaEventDefault : cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&S.fork, cudaEventDisableTiming));
     for (int i = 0; i < 2; ++i) {
-      CK(cudaEventCreateWithFlags(&S.rules_done[i], (evt & 2) ? cudaEventDefault : cudaEventDisableTiming));
-      CK(cudaEventCreateWithFlags(&S.expand_done_plain[i], (evt & 1) ? cudaEventDefault : cudaEventDisableTiming));
+      CK(cudaEventCreateWithFlags(&S.rules_done[i], cudaEventDisableTiming));
+      CK(cudaEventCreateWithFlags(&S.expand_done_plain[i], cudaEventDisableTiming));
       CK(cudaEventCreateWithFlags(&S.expand_done_stamped[i], cudaEventDefault));
       S.expand_done[i] = S.expand_done_plain[i];
     }
@@ -288,53 +273,6 @@ struct DenseOut {
   fpc_dense_track *track;
 };
 
-#ifndef FPC_EXPERIMENT
-static inline int prof_mask() { return 15; }
-#endif
-// FPC_NO_STARTUP_STAMPS=1 (diagnostics) switches the start-up behaviour of launch_observe off
-static bool startup_probe_enabled() {
-  static const bool on = !(getenv("FPC_NO_STARTUP_STAMPS") && atoi(getenv("FPC_NO_STARTUP_STAMPS")));
-  return on;
-}
-#ifdef FPC_EXPERIMENT
-// Diagnostics build only (tools/overlap_probe.py): knobs that change how the two kernels of a dense step are launched.
-static int xknob(const char *name) {
-  const char *e = getenv(name);
-  return e ? atoi(e) : 0;
-}
-// FPC_X_PROFMASK: which of the four timing records of an instrumented step are issued (1 rules start, 2 rules end,
-// 4 expand start, 8 expand end); fpc_profile_read then only counts launches
-static int prof_mask() {
-  const char *e = getenv("FPC_X_PROFMASK");
-  return e ? atoi(e) : 15;
-}
-__global__ void delay_kernel(int us) {
-  const long long t0 = clock64();
-  while (clock64() - t0 < (long long)us * 1965) __nanosleep(200);
-}
-template <class G>
-static void launch_rules_x(int n, cudaStream_t st, const ObserveParams &p_in) {
-  ObserveParams p = p_in;
-  if (xknob("FPC_X_NOCOUNTERS")) p.counters = nullptr;  // no global atomics on the eight shared counters
-  // FPC_X_RDELAY = microseconds the rules kernel is held back on its stream (one idle thread spins first)
-  if (xknob("FPC_X_RDELAY")) delay_kernel<<<1, 1, 0, st>>>(xknob("FPC_X_RDELAY"));
-  // FPC_X_RSMEM = KB of (unused) dynamic shared memory per rules CTA: caps how many of them an SM holds
-  const int dyn = xknob("FPC_X_RSMEM") * 1024;
-  if (dyn) {
-    static bool set = false;
-    if (!set) cudaFuncSetAttribute(rules_kernel<G, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024), set = true;
-    rules_kernel<G, 4><<<(n + 3) / 4, 128, dyn, st>>>(p);
-    return;
-  }
-  switch (xknob("FPC_X_RWARPS")) {
-    case 1: rules_kernel<G, 1><<<n, 32, 0, st>>>(p); break;
-    case 2: rules_kernel<G, 2><<<(n + 1) / 2, 64, 0, st>>>(p); break;
-    case 8: rules_kernel<G, 8><<<(n + 7) / 8, 256, 0, st>>>(p); break;
-    default: rules_kernel<G, 4><<<(n + 3) / 4, 128, 0, st>>>(p); break;
-  }
-}
-#endif
-
 // rules_kernel on a high-priority stream forked from the caller's; expand_kernel on the side stream once the rules
 // kernel has written the records.  Unless FPC_FLAG_ASYNC_DENSE is set the caller's stream then waits for the
 // expansion.  after_rules (may be a no-op) runs right after the rules kernel is enqueued: the host-buffer entry
@@ -385,7 +323,7 @@ static int launch_observe(ObserveParams p, DenseOut d, cudaStream_t st, F after_
   {
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) cudaGetLastError(), cap = cudaStreamCaptureStatusActive;
-    if (cap == cudaStreamCaptureStatusNone && startup_probe_enabled()) {
+    if (cap == cudaStreamCaptureStatusNone) {
       side_was_idle = cudaStreamQuery(S->side) == cudaSuccess || cudaStreamQuery(S->hi) == cudaSuccess;
       cudaGetLastError();  // "not ready" is reported through the error state
     }
@@ -412,9 +350,6 @@ static int launch_observe(ObserveParams p, DenseOut d, cudaStream_t st, F after_
   CK(cudaEventRecord(S->fork, st));
   CK(cudaStreamWaitEvent(S->hi, S->fork, 0));
   if (S->expand_recorded[b]) CK(cudaStreamWaitEvent(S->hi, S->expand_done[b], 0));
-#ifdef FPC_EXPERIMENT
-  if (xknob("FPC_X_SERIAL") && S->last >= 0) CK(cudaStreamWaitEvent(S->hi, S->expand_done[S->last], 0));
-#endif
   // Both kernels ask for the same shared-memory carveout: CTAs of rules_kernel (14 KB of shared memory each) and of
   // expand_kernel (none) share SMs, and an SM only changes its L1 / shared split when it is empty.
   {
@@ -428,37 +363,32 @@ static int launch_observe(ObserveParams p, DenseOut d, cudaStream_t st, F after_
     }
   }
   const bool prof = S->prof_on && S->prof_n < PROF_MAX;
-  if (prof && (prof_mask() & 1)) CK(cudaEventRecord(S->prof_ev_r[2 * S->prof_n], S->hi));
-#ifdef FPC_EXPERIMENT
-  if (!xknob("FPC_X_SKIPRULES")) launch_rules_x<G>(p.n, S->hi, p);
-#else
+  if (prof) CK(cudaEventRecord(S->prof_ev_r[2 * S->prof_n], S->hi));
   rules_kernel<G><<<blocks, BLOCK_THREADS, 0, S->hi>>>(p);
-#endif
   CK(cudaGetLastError());
-  if (prof && (prof_mask() & 2)) CK(cudaEventRecord(S->prof_ev_r[2 * S->prof_n + 1], S->hi));
+  if (prof) CK(cudaEventRecord(S->prof_ev_r[2 * S->prof_n + 1], S->hi));
   CK(cudaEventRecord(S->rules_done[b], S->hi));
   CK(cudaStreamWaitEvent(st, S->rules_done[b], 0));
   rc = after_rules();
   if (rc != FPC_OK) return rc;
   CK(cudaStreamWaitEvent(S->side, S->rules_done[b], 0));
-  if (prof && (prof_mask() & 4)) CK(cudaEventRecord(S->prof_ev[2 * S->prof_n], S->side));
+  if (prof) CK(cudaEventRecord(S->prof_ev[2 * S->prof_n], S->side));
   {
     static thread_local int sms[MAX_DEVICES] = {0};
     int dev = 0;
     CK(cudaGetDevice(&dev));
     if (!sms[dev]) CK(cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev));
     const int grid = p.n < sms[dev] ? p.n : sms[dev];
-#ifdef FPC_EXPERIMENT
-    if (!xknob("FPC_X_NOEXPAND"))
-#endif
     expand_kernel<G><<<grid, EXPAND_THREADS, 0, S->side>>>(p.cells, d.planes, p.flats, d.mask, p.n);
   }
   CK(cudaGetLastError());
-  if (prof && (prof_mask() & 8)) CK(cudaEventRecord(S->prof_ev[2 * S->prof_n + 1], S->side));
-  if (prof) ++S->prof_n;
+  if (prof) {
+    CK(cudaEventRecord(S->prof_ev[2 * S->prof_n + 1], S->side));
+    ++S->prof_n;
+  }
   // Which event marks the end of this expansion.  A TIMESTAMPED record is the robust one: measured on B200
-  // (tools/overlap_probe.py, gpurun_out/xrun23.log, xrun26.log) it costs ~2 us per step against a plain record when the
-  // caller runs far ahead of the device (76.3 vs 74.2 us per step), but with the plain record a loop that starts from
+  // (tools/overlap_probe.py, DESIGN.md section 3 item 5) it costs ~2 us per step against a plain record when the caller
+  // runs far ahead of the device (76.3 vs 74.2 us per step), but with the plain record a loop that starts from
   // an idle device loses ~250 us (20 steps: ~90 vs 79 us per step), and a caller that waits for every step's results
   // before issuing the next one falls into a mode of 176 us per step (83 us with the timestamped record).  So: the
   // timestamped record whenever a call finds an internal stream idle, and for the STARTUP_CALLS calls after that; the
@@ -581,33 +511,22 @@ static int launch_attack_maps(const uint8_t *in, int n, uint8_t *out, cudaStream
   return cuda_check(cudaGetLastError(), "attack_map_kernel launch");
 }
 
-#define FPC_DISPATCH(R, CALL)                                              \
-  switch (R) {                                                             \
-    case 14: { using G = Geo<14, 3>; return CALL; }                        \
-    case 13: { using G = Geo<13, 3>; return CALL; }                        \
-    case 10: { using G = Geo<10, 2>; return CALL; }                        \
-    case 8: { using G = Geo<8, 2>; return CALL; }                          \
-    default: return fail(FPC_ERR_ARG, "unsupported board size R=" + std::to_string(R)); \
-  }
-
-static int ia_of(int R) { return R == 14 || R == 13 ? 3 : (R == 10 || R == 8 ? 2 : -1); }
-
 template <class F>
 static int do_observe(int R, const ObserveParams &p, DenseOut d, cudaStream_t st, F after_rules) {
-  FPC_DISPATCH(R, (launch_observe<G>(p, d, st, after_rules)));
+  return dispatch(R, [&](auto g) { return launch_observe<decltype(g)>(p, d, st, after_rules); });
 }
 static int do_observe(int R, const ObserveParams &p, DenseOut d, cudaStream_t st) {
   return do_observe(R, p, d, st, [] { return FPC_OK; });
 }
 static int do_make(int R, const uint8_t *in, const uint64_t *moves, const int32_t *flat, int n, uint8_t *out,
                    int32_t *err, cudaStream_t st) {
-  FPC_DISPATCH(R, launch_make<G>(in, moves, flat, n, out, err, st));
+  return dispatch(R, [&](auto g) { return launch_make<decltype(g)>(in, moves, flat, n, out, err, st); });
 }
 static int do_heuristic(int R, const uint8_t *in, int n, int32_t *v, cudaStream_t st) {
-  FPC_DISPATCH(R, launch_heuristic<G>(in, n, v, st));
+  return dispatch(R, [&](auto g) { return launch_heuristic<decltype(g)>(in, n, v, st); });
 }
 static int do_attack_maps(int R, const uint8_t *in, int n, uint8_t *out, cudaStream_t st) {
-  FPC_DISPATCH(R, launch_attack_maps<G>(in, n, out, st));
+  return dispatch(R, [&](auto g) { return launch_attack_maps<decltype(g)>(in, n, out, st); });
 }
 
 }  // namespace fpc
@@ -748,7 +667,7 @@ int fpc_profile_read(int *launches, double *expand_ms, double *rules_ms) {
   CK(cudaStreamSynchronize(S->side));
   CK(cudaStreamSynchronize(S->hi));
   double total = 0, total_r = 0;
-  for (int i = 0; i < S->prof_n && prof_mask() == 15; ++i) {
+  for (int i = 0; i < S->prof_n; ++i) {
     float ms = 0;
     CK(cudaEventElapsedTime(&ms, S->prof_ev[2 * i], S->prof_ev[2 * i + 1]));
     total += ms;

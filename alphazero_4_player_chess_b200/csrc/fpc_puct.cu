@@ -10,17 +10,9 @@
 
 #include "../../include/fpc.h"
 #include "fpc_device.cuh"
+#include "fpc_host.h"
 
 namespace fpc {
-
-int fail(int code, const std::string &msg);  // fpc_kernels.cu
-int cuda_check(cudaError_t e, const char *what);
-
-#define CK(expr)                                   \
-  do {                                             \
-    int rc_ = cuda_check((expr), #expr);           \
-    if (rc_ != FPC_OK) return rc_;                 \
-  } while (0)
 
 constexpr int SEL_WARPS = 4;
 constexpr int ERR_NODE_CAP = 1, ERR_BOARD_CAP = 2, ERR_NO_CHILD = 4, ERR_MOVE = 8;
@@ -598,15 +590,6 @@ __global__ void __launch_bounds__(EXP_THREADS, 8) tree_expand_backup_kernel(cons
   }
 }
 
-#define FPC_DISPATCH(R, CALL)                                              \
-  switch (R) {                                                             \
-    case 14: { using G = Geo<14, 3>; CALL; break; }                        \
-    case 13: { using G = Geo<13, 3>; CALL; break; }                        \
-    case 10: { using G = Geo<10, 2>; CALL; break; }                        \
-    case 8: { using G = Geo<8, 2>; CALL; break; }                          \
-    default: return fail(FPC_ERR_ARG, "unsupported board size R=" + std::to_string(R)); \
-  }
-
 static int check_tree(const fpc_tree *t, const char *who) {
   if (!t) return fail(FPC_ERR_ARG, std::string(who) + ": null tree");
   if (!fpc_supported(t->R) || t->n_games < 0 || t->node_cap < 1 || t->board_cap < 1)
@@ -641,8 +624,10 @@ int fpc_tree_reset(const fpc_tree *t, const uint8_t *d_root_boards, void *stream
   if (t->n_games == 0) return FPC_OK;
   if (!d_root_boards) return fail(FPC_ERR_ARG, "fpc_tree_reset: null roots");
   cudaStream_t st = (cudaStream_t)stream;
-  FPC_DISPATCH(t->R, (tree_reset_kernel<G><<<t->n_games, 256, 0, st>>>(*t, d_root_boards)));
-  return cuda_check(cudaGetLastError(), "tree_reset_kernel launch");
+  return dispatch(t->R, [&](auto g) {
+    tree_reset_kernel<decltype(g)><<<t->n_games, 256, 0, st>>>(*t, d_root_boards);
+    return cuda_check(cudaGetLastError(), "tree_reset_kernel launch");
+  });
 }
 
 int fpc_tree_advance(const fpc_tree *t, const int32_t *d_actions, const uint8_t *d_root_boards, int32_t max_keep_nodes,
@@ -657,8 +642,9 @@ int fpc_tree_advance(const fpc_tree *t, const int32_t *d_actions, const uint8_t 
   if (!d_actions || !d_root_boards) return fail(FPC_ERR_ARG, "fpc_tree_advance: null actions / roots");
   if (reinterpret_cast<uintptr_t>(d_root_boards) & 15) return fail(FPC_ERR_ARG, "root boards must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
-  FPC_DISPATCH(t->R, (rc = launch_advance<G>(*t, d_actions, d_root_boards, max_keep_nodes, max_keep_boards, d_kept, st)));
-  return rc;
+  return dispatch(t->R, [&](auto g) {
+    return launch_advance<decltype(g)>(*t, d_actions, d_root_boards, max_keep_nodes, max_keep_boards, d_kept, st);
+  });
 }
 
 int fpc_tree_select(const fpc_tree *t, int batch_rotation, float *d_planes, int flags, fpc_dense_track *track, void *stream) {
@@ -667,15 +653,21 @@ int fpc_tree_select(const fpc_tree *t, int batch_rotation, float *d_planes, int 
   if (t->n_games == 0) return FPC_OK;
   cudaStream_t st = (cudaStream_t)stream;
   const int blocks = (t->n_games + SEL_WARPS - 1) / SEL_WARPS;
-  FPC_DISPATCH(t->R, (tree_descend_kernel<G><<<blocks, SEL_WARPS * 32, 0, st>>>(*t)));
-  CK(cudaGetLastError());
+  rc = dispatch(t->R, [&](auto g) {
+    tree_descend_kernel<decltype(g)><<<blocks, SEL_WARPS * 32, 0, st>>>(*t);
+    return cuda_check(cudaGetLastError(), "tree_descend_kernel launch");
+  });
+  if (rc != FPC_OK) return rc;
   if (batch_rotation) {
     // the batch rotation is that of the first NON-terminal leaf: results first, then k, then the planes
     rc = fpc_observe(t->R, t->leaf_boards, t->n_games, nullptr, t->leaf_flat, t->leaf_counts, t->leaf_status, nullptr,
                      nullptr, 0, nullptr, 0, stream);
     if (rc != FPC_OK) return rc;
-    FPC_DISPATCH(t->R, (tree_batch_k_kernel<G><<<1, 1024, 0, st>>>(*t)));
-    CK(cudaGetLastError());
+    rc = dispatch(t->R, [&](auto g) {
+      tree_batch_k_kernel<decltype(g)><<<1, 1024, 0, st>>>(*t);
+      return cuda_check(cudaGetLastError(), "tree_batch_k_kernel launch");
+    });
+    if (rc != FPC_OK) return rc;
     return fpc_observe_tracked(track, t->R, t->leaf_boards, t->n_games, nullptr, nullptr, nullptr, nullptr, d_planes, t->k, 0,
                                nullptr, flags, stream);
   }
@@ -691,8 +683,10 @@ int fpc_tree_expand_backup(const fpc_tree *t, const float *d_logits, const float
   if (!d_logits || !d_values) return fail(FPC_ERR_ARG, "fpc_tree_expand_backup: null logits / values");
   if (reinterpret_cast<uintptr_t>(d_logits) & 15) return fail(FPC_ERR_ARG, "logits must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
-  FPC_DISPATCH(t->R, (tree_expand_backup_kernel<G><<<t->n_games, EXP_THREADS, 0, st>>>(*t, d_logits, d_values)));
-  return cuda_check(cudaGetLastError(), "tree_expand_backup_kernel launch");
+  return dispatch(t->R, [&](auto g) {
+    tree_expand_backup_kernel<decltype(g)><<<t->n_games, EXP_THREADS, 0, st>>>(*t, d_logits, d_values);
+    return cuda_check(cudaGetLastError(), "tree_expand_backup_kernel launch");
+  });
 }
 
 }  // extern "C"

@@ -1,5 +1,5 @@
-"""Diagnostics: the dense playout step (rules_kernel + expand_kernel) under the launch knobs of the FPC_EXPERIMENT
-build (tools/build_experiment.sh -> tools/libfpc_x.so).  usage: FPC_LIB_PATH=tools/libfpc_x.so FPC_X_...=1 python
+"""Diagnostics: times the pipelined dense playout step (rules_kernel + expand_kernel) under the caller patterns set by
+the FPC_P_* variables below; FPC_LIB_PATH points it at another build of the library.  usage: [FPC_P_...=1] python
 tools/overlap_probe.py [steps] [fast_forward_plies]"""
 import ctypes, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -34,7 +34,8 @@ for _ in range(20):
 env.join()
 torch.cuda.synchronize()
 noprof = int(os.environ.get("FPC_P_NOPROF", "0"))  # 1: no per-launch CUDA events around the two kernels
-_lib.check(L.fpc_profile_enable(0 if noprof else int(os.environ.get("FPC_P_PROF", "1"))))  # FPC_P_PROF = N: every N-th launch timed
+prof = not noprof and int(os.environ.get("FPC_P_PROF", "1")) != 0  # FPC_P_PROF=0: the same as FPC_P_NOPROF=1
+_lib.check(L.fpc_profile_enable(int(prof)))
 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
 env.counters.zero_()
 sync_each = int(os.environ.get("FPC_P_SYNC", "0"))  # 1: the host waits for every step's compact results (rules kernel)
@@ -70,7 +71,7 @@ for _ in range(steps):
     env.playout_step(planes=False, mask=False)
 r1.record()
 torch.cuda.synchronize()
-knobs = {k: v for k, v in os.environ.items() if k.startswith("FPC_X_") or k.startswith("FPC_P_")}
+knobs = {k: v for k, v in os.environ.items() if k.startswith("FPC_P_")}
 c = env.counters.cpu()
 print(f"{knobs}: step {e0.elapsed_time(e1) / steps * 1e3:.1f} us, expand in-loop {ex.value / max(n.value, 1) * 1e3:.1f} us, "
       f"rules in-loop {ru.value / max(n.value, 1) * 1e3:.1f} us, rules-only step {r0.elapsed_time(r1) / steps * 1e3:.1f} us, "
