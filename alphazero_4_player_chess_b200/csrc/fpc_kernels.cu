@@ -149,11 +149,12 @@ int cuda_check(cudaError_t e, const char *what) {
   return fail(FPC_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
 }
 
-// One record pair (plane cells / mask flats) per game, double-buffered: rules_kernel of step t+1 writes one buffer
-// while expand_kernel of step t still reads the other.
+// One record pair (plane cells / mask flats) per game, double-buffered: rules_kernel of a full rewrite writes one half
+// while expand_kernel of an earlier call may still read the other.  cur_*: the half with the tensor's latest record.
 struct Records {
   uint16_t *cells[2] = {nullptr, nullptr}, *flats[2] = {nullptr, nullptr};
   size_t games = 0;
+  int cur_cells = 0, cur_flats = 0;
   int release() {
     for (int i = 0; i < 2; ++i) {
       cudaFree(cells[i]);
@@ -175,39 +176,48 @@ struct Records {
   }
 };
 
-// Per host thread and device: the streams the two kernels of a dense call run on, their events, and the record
-// workspace between rules_kernel and expand_kernel for calls without a fpc_dense_track.
-struct SideState {
+// Optional CUDA-event timing of one dense call's two launches on their own streams (fpc_profile_enable / _read).
+struct LaunchTimes {
+  cudaEvent_t rules[2], expand[2];  // start, stop
+};
+constexpr int PROF_MAX = 4096;
+
+// Per host thread and device: the streams the two kernels of a dense call run on, their events, and the records of
+// calls without a fpc_dense_track.
+struct DeviceState {
+  int device = -1;
+  int sms = 0;                  // multiprocessors: the grid of expand_kernel
   cudaStream_t side = nullptr;  // expand_kernel: lowest priority
   cudaStream_t hi = nullptr;    // rules_kernel when dense outputs are wanted: highest priority, so that its
                                 // CTAs are dispatched ahead of the remaining CTAs of a running expansion
   cudaEvent_t fork = nullptr;
   cudaEvent_t rules_done[2] = {nullptr, nullptr}, expand_done[2] = {nullptr, nullptr};
-  // expand_done[b] is whichever of these two was recorded last for buffer b: the plain one (no timing) in steady state,
-  // the timestamped one while a pipeline of dense calls is starting up (see launch_observe)
+  // expand_done[b] is whichever of these two was recorded last for slot b: the plain one (no timing) in steady state,
+  // the timestamped one while a pipeline of dense calls is starting up (end_event)
   cudaEvent_t expand_done_plain[2] = {nullptr, nullptr}, expand_done_stamped[2] = {nullptr, nullptr};
   int startup_left = 0;
   bool expand_recorded[2] = {false, false};
-  Records ws;
-  int parity = 0;
-  int last = -1;           // event slot of the most recent expansion (fpc_join)
+  int parity = 0;           // event slot of the next full rewrite
+  int last = -1;            // event slot of the most recent expansion (fpc_join)
   bool last_async = false;  // ... which the caller's stream has not been made to wait for (FPC_FLAG_ASYNC_DENSE)
-  // optional CUDA-event timing of expand_kernel on its own stream (fpc_profile_enable / _read)
+  unsigned carveout_set = 0;  // bit R: the shared-memory carveout of board size R's two kernels is requested
+  Records ws;
   bool prof_on = false;
   int prof_n = 0;
-  std::vector<cudaEvent_t> prof_ev;   // expand_kernel: start/stop pairs
-  std::vector<cudaEvent_t> prof_ev_r; // rules_kernel (dense path): start/stop pairs
+  std::vector<LaunchTimes> prof;
 };
-constexpr int PROF_MAX = 4096;
 constexpr int MAX_DEVICES = 16;
-static thread_local SideState g_side[MAX_DEVICES];
+static thread_local DeviceState g_dev[MAX_DEVICES];
 
-static int side_state(SideState **out) {
+// The calling thread's state on the current device.  With `create`, its streams and events are made on first use.
+static int device_state(DeviceState **out, bool create) {
   int dev = 0;
   CK(cudaGetDevice(&dev));
   if (dev < 0 || dev >= MAX_DEVICES) return fail(FPC_ERR_ARG, "device ordinal out of range");
-  SideState &S = g_side[dev];
-  if (!S.side) {
+  DeviceState &S = g_dev[dev];
+  if (create && !S.side) {
+    S.device = dev;
+    CK(cudaDeviceGetAttribute(&S.sms, cudaDevAttrMultiProcessorCount, dev));
     int least = 0, greatest = 0;
     CK(cudaDeviceGetStreamPriorityRange(&least, &greatest));
     CK(cudaStreamCreateWithPriority(&S.side, cudaStreamNonBlocking, least));
@@ -224,31 +234,6 @@ static int side_state(SideState **out) {
   return FPC_OK;
 }
 
-// Releases everything this host thread holds on the current device (fpc_shutdown).
-static int side_release() {
-  int dev = 0;
-  CK(cudaGetDevice(&dev));
-  if (dev < 0 || dev >= MAX_DEVICES) return fail(FPC_ERR_ARG, "device ordinal out of range");
-  SideState &S = g_side[dev];
-  if (S.side) {
-    CK(cudaStreamSynchronize(S.side));
-    CK(cudaStreamSynchronize(S.hi));
-    cudaStreamDestroy(S.side);
-    cudaStreamDestroy(S.hi);
-    cudaEventDestroy(S.fork);
-    for (int i = 0; i < 2; ++i) {
-      cudaEventDestroy(S.rules_done[i]);
-      cudaEventDestroy(S.expand_done_plain[i]);
-      cudaEventDestroy(S.expand_done_stamped[i]);
-    }
-  }
-  S.ws.release();
-  for (auto &e : S.prof_ev) cudaEventDestroy(e);
-  for (auto &e : S.prof_ev_r) cudaEventDestroy(e);
-  S = SideState();
-  return FPC_OK;
-}
-
 }  // namespace fpc
 
 // Explicit handle for resident dense tensors (FPC_FLAG_INCREMENTAL): it owns the records of the ones the latest dense
@@ -258,9 +243,8 @@ struct fpc_dense_track {
   unsigned magic;
   int device, R, n;
   fpc::Records rec;
-  // per tensor: the pointer the record describes, which buffer holds the record, whether the content is known
+  // per tensor: the pointer the record describes, whether the content is known
   const float *planes, *mask;
-  int cur_cells, cur_flats;
   bool known_planes, known_mask;
 };
 
@@ -273,136 +257,137 @@ struct DenseOut {
   fpc_dense_track *track;
 };
 
-// rules_kernel on a high-priority stream forked from the caller's; expand_kernel on the side stream once the rules
-// kernel has written the records.  Unless FPC_FLAG_ASYNC_DENSE is set the caller's stream then waits for the
-// expansion.  after_rules (may be a no-op) runs right after the rules kernel is enqueued: the host-buffer entry
-// points start their device-to-host copies of the compact results there.
+// Incremental update: the tensors hold exactly the recorded ones, so the rules kernel clears those and sets the new
+// ones on the caller's stream, with no expansion.  A still running expansion into the same tensors (an earlier
+// FPC_FLAG_ASYNC_DENSE call) must finish first.
+template <class G, class F>
+static int launch_incremental(ObserveParams p, DenseOut d, const DeviceState &S, cudaStream_t st, F after_rules) {
+  if (S.last >= 0 && S.last_async) CK(cudaStreamWaitEvent(st, S.expand_done[S.last], 0));
+  const Records &r = d.track->rec;
+  p.cells = d.planes ? r.cells[r.cur_cells] : nullptr;
+  p.flats = d.mask ? r.flats[r.cur_flats] : nullptr;
+  p.inc_planes = d.planes;
+  p.inc_mask = d.mask;
+  rules_kernel<G><<<(p.n + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK, BLOCK_THREADS, 0, st>>>(p);
+  CK(cudaGetLastError());
+  return after_rules();
+}
+
+// Is the caller running ahead of the device (both internal streams still have work queued), or does this call find
+// one of them idle -- a run of dense calls starting up, or a host that waits for every step's results?  Asked before
+// the call enqueues anything; never during stream capture, where querying a stream is not allowed (a captured call
+// counts as running ahead).
+static bool finds_stream_idle(const DeviceState &S, cudaStream_t st) {
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) cudaGetLastError(), cap = cudaStreamCaptureStatusActive;
+  if (cap != cudaStreamCaptureStatusNone) return false;
+  const bool idle = cudaStreamQuery(S.side) == cudaSuccess || cudaStreamQuery(S.hi) == cudaSuccess;
+  cudaGetLastError();  // "not ready" is reported through the error state
+  return idle;
+}
+
+// Which event marks the end of the expansion in slot b.  A TIMESTAMPED record is the robust one: measured on B200
+// (tools/overlap_probe.py, DESIGN.md section 3 item 5) it costs ~2 us per step against a plain record when the caller
+// runs far ahead of the device (76.3 vs 74.2 us per step), but with the plain record a loop that starts from
+// an idle device loses ~250 us (20 steps: ~90 vs 79 us per step), and a caller that waits for every step's results
+// before issuing the next one falls into a mode of 176 us per step (83 us with the timestamped record).  So: the
+// timestamped record whenever a call finds an internal stream idle, and for the STARTUP_CALLS calls after that; the
+// plain one only while the caller keeps both streams busy.
+static cudaEvent_t end_event(DeviceState &S, int b, bool found_idle) {
+  constexpr int STARTUP_CALLS = 8;
+  if (found_idle) S.startup_left = STARTUP_CALLS;
+  S.expand_done[b] = S.startup_left > 0 ? S.expand_done_stamped[b] : S.expand_done_plain[b];
+  if (S.startup_left > 0) --S.startup_left;
+  return S.expand_done[b];
+}
+
+// Full rewrite: rules_kernel on the high-priority stream forked from the caller's, expand_kernel on the side stream
+// once the records exist; unless FPC_FLAG_ASYNC_DENSE is set the caller's stream then waits for the expansion.
+template <class G, class F>
+static int launch_full(ObserveParams p, DenseOut d, DeviceState &S, cudaStream_t st, F after_rules) {
+  const bool found_idle = finds_stream_idle(S, st);
+  const int b = S.parity;
+  S.parity ^= 1;
+  // growing the handle-less records (a handle's fit its batch): earlier launches may still use the old ones
+  Records &r = d.track ? d.track->rec : S.ws;
+  if ((size_t)p.n > r.games) {
+    CK(cudaStreamSynchronize(st));
+    CK(cudaStreamSynchronize(S.side));
+    CK(cudaStreamSynchronize(S.hi));
+    int rc = r.reserve((size_t)p.n);
+    if (rc != FPC_OK) return rc;
+  }
+  if (d.planes) r.cur_cells ^= 1, p.cells = r.cells[r.cur_cells];
+  if (d.mask) r.cur_flats ^= 1, p.flats = r.flats[r.cur_flats];
+  CK(cudaEventRecord(S.fork, st));
+  CK(cudaStreamWaitEvent(S.hi, S.fork, 0));
+  // The half of the records this call writes was last read by an expansion at least two full rewrites earlier on this
+  // thread and device: each tensor's records alternate halves, and only full rewrites flip them.  All those expansions
+  // run in order on the one side stream, so waiting for the expansion two calls back (slot b) covers it.  Incremental
+  // calls read the records on the caller's stream, which the fork orders.
+  if (S.expand_recorded[b]) CK(cudaStreamWaitEvent(S.hi, S.expand_done[b], 0));
+  // Both kernels ask for the same shared-memory carveout: CTAs of rules_kernel (14 KB of shared memory each) and of
+  // expand_kernel (none) share SMs, and an SM only changes its L1 / shared split when it is empty.
+  if (!((S.carveout_set >> G::R) & 1u)) {
+    CK(cudaFuncSetAttribute(rules_kernel<G>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+    CK(cudaFuncSetAttribute(expand_kernel<G>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+    S.carveout_set |= 1u << G::R;
+  }
+  LaunchTimes *t = S.prof_on && S.prof_n < PROF_MAX ? &S.prof[S.prof_n] : nullptr;
+  if (t) CK(cudaEventRecord(t->rules[0], S.hi));
+  rules_kernel<G><<<(p.n + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK, BLOCK_THREADS, 0, S.hi>>>(p);
+  CK(cudaGetLastError());
+  if (t) CK(cudaEventRecord(t->rules[1], S.hi));
+  CK(cudaEventRecord(S.rules_done[b], S.hi));
+  CK(cudaStreamWaitEvent(st, S.rules_done[b], 0));
+  const int rc = after_rules();
+  if (rc != FPC_OK) return rc;
+  CK(cudaStreamWaitEvent(S.side, S.rules_done[b], 0));
+  if (t) CK(cudaEventRecord(t->expand[0], S.side));
+  expand_kernel<G><<<p.n < S.sms ? p.n : S.sms, EXPAND_THREADS, 0, S.side>>>(p.cells, d.planes, p.flats, d.mask, p.n);
+  CK(cudaGetLastError());
+  if (t) {
+    CK(cudaEventRecord(t->expand[1], S.side));
+    ++S.prof_n;
+  }
+  const cudaEvent_t done = end_event(S, b, found_idle);
+  CK(cudaEventRecord(done, S.side));
+  S.expand_recorded[b] = true;
+  S.last = b;
+  S.last_async = (d.flags & FPC_FLAG_ASYNC_DENSE) != 0;
+  if (!S.last_async) CK(cudaStreamWaitEvent(st, done, 0));
+  return FPC_OK;
+}
+
+// after_rules (may be a no-op) runs right after the rules kernel is enqueued: the host-buffer entry points start their
+// device-to-host copies of the compact results there.
 template <class G, class F>
 static int launch_observe(ObserveParams p, DenseOut d, cudaStream_t st, F after_rules) {
   if (p.n == 0) return FPC_OK;
-  const bool dense = d.planes || d.mask;
-  const int blocks = (p.n + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
-  if (!dense) {
-    rules_kernel<G><<<blocks, BLOCK_THREADS, 0, st>>>(p);
+  if (!d.planes && !d.mask) {  // rules only: one launch on the caller's stream
+    rules_kernel<G><<<(p.n + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK, BLOCK_THREADS, 0, st>>>(p);
     CK(cudaGetLastError());
     return after_rules();
   }
   if ((reinterpret_cast<uintptr_t>(d.planes) | reinterpret_cast<uintptr_t>(d.mask)) & 15)
     return fail(FPC_ERR_ARG, "planes / mask must be 16-byte aligned");
-  SideState *S = nullptr;
-  int rc = side_state(&S);
+  DeviceState *S = nullptr;
+  int rc = device_state(&S, true);
   if (rc != FPC_OK) return rc;
   fpc_dense_track *T = d.track;
   if (T) {
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
     if (T->magic != TRACK_MAGIC) return fail(FPC_ERR_ARG, "fpc_dense_track: not a live handle");
-    if (T->device != dev || T->R != G::R || T->n != p.n) return fail(FPC_ERR_ARG, "fpc_dense_track: made for another device / board size / batch");
+    if (T->device != S->device || T->R != G::R || T->n != p.n) return fail(FPC_ERR_ARG, "fpc_dense_track: made for another device / board size / batch");
     // a handle follows one planes tensor and one mask tensor; being used with another one starts over for that tensor
     if (d.planes && d.planes != T->planes) T->planes = d.planes, T->known_planes = false;
     if (d.mask && d.mask != T->mask) T->mask = d.mask, T->known_mask = false;
-    const bool inc = (d.flags & FPC_FLAG_INCREMENTAL) && (!d.planes || T->known_planes) && (!d.mask || T->known_mask);
-    if (inc) {
-      // the tensors hold exactly the recorded ones: clear those, set the new ones, no expansion.  A still running
-      // expansion into the same tensors (an earlier FPC_FLAG_ASYNC_DENSE call) must finish first.
-      if (S->last >= 0 && S->last_async) CK(cudaStreamWaitEvent(st, S->expand_done[S->last], 0));
-      p.cells = d.planes ? T->rec.cells[T->cur_cells] : nullptr;
-      p.flats = d.mask ? T->rec.flats[T->cur_flats] : nullptr;
-      p.inc_planes = d.planes;
-      p.inc_mask = d.mask;
-      rules_kernel<G><<<blocks, BLOCK_THREADS, 0, st>>>(p);
-      CK(cudaGetLastError());
-      return after_rules();
-    }
+    if ((d.flags & FPC_FLAG_INCREMENTAL) && (!d.planes || T->known_planes) && (!d.mask || T->known_mask))
+      return launch_incremental<G>(p, d, *S, st, after_rules);
+    // the full rewrite leaves each tensor it writes holding exactly its new record
+    if (d.planes) T->known_planes = true;
+    if (d.mask) T->known_mask = true;
   }
-  // Is the caller running ahead of the device (both internal streams still have work queued), or does this call find
-  // one of them idle -- a run of dense calls starting up, or a host that waits for every step's results?  Asked before
-  // this call enqueues anything; never during stream capture, where querying a stream is not allowed (a captured call
-  // counts as running ahead).
-  bool side_was_idle = false;
-  {
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) cudaGetLastError(), cap = cudaStreamCaptureStatusActive;
-    if (cap == cudaStreamCaptureStatusNone) {
-      side_was_idle = cudaStreamQuery(S->side) == cudaSuccess || cudaStreamQuery(S->hi) == cudaSuccess;
-      cudaGetLastError();  // "not ready" is reported through the error state
-    }
-  }
-  // full rewrite: the records go to the buffer the previous expansion is not reading
-  const int b = S->parity;
-  S->parity ^= 1;
-  if (T) {
-    if (d.planes) T->cur_cells ^= 1, p.cells = T->rec.cells[T->cur_cells], T->known_planes = true;
-    if (d.mask) T->cur_flats ^= 1, p.flats = T->rec.flats[T->cur_flats], T->known_mask = true;
-  } else {
-    if ((size_t)p.n > S->ws.games) {  // growing the workspace: earlier launches may still use the old one
-      CK(cudaStreamSynchronize(st));
-      CK(cudaStreamSynchronize(S->side));
-      CK(cudaStreamSynchronize(S->hi));
-      rc = S->ws.reserve((size_t)p.n);
-      if (rc != FPC_OK) return rc;
-    }
-    p.cells = d.planes ? S->ws.cells[b] : nullptr;
-    p.flats = d.mask ? S->ws.flats[b] : nullptr;
-  }
-  // fork: caller's stream -> high-priority stream (rules) -> back to the caller's stream; the expansion that last
-  // read this record buffer (two dense calls ago) must be done before the rules kernel rewrites it
-  CK(cudaEventRecord(S->fork, st));
-  CK(cudaStreamWaitEvent(S->hi, S->fork, 0));
-  if (S->expand_recorded[b]) CK(cudaStreamWaitEvent(S->hi, S->expand_done[b], 0));
-  // Both kernels ask for the same shared-memory carveout: CTAs of rules_kernel (14 KB of shared memory each) and of
-  // expand_kernel (none) share SMs, and an SM only changes its L1 / shared split when it is empty.
-  {
-    static thread_local bool carveout_set[MAX_DEVICES] = {false};
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (dev >= 0 && dev < MAX_DEVICES && !carveout_set[dev]) {
-      CK(cudaFuncSetAttribute(rules_kernel<G>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-      CK(cudaFuncSetAttribute(expand_kernel<G>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-      carveout_set[dev] = true;
-    }
-  }
-  const bool prof = S->prof_on && S->prof_n < PROF_MAX;
-  if (prof) CK(cudaEventRecord(S->prof_ev_r[2 * S->prof_n], S->hi));
-  rules_kernel<G><<<blocks, BLOCK_THREADS, 0, S->hi>>>(p);
-  CK(cudaGetLastError());
-  if (prof) CK(cudaEventRecord(S->prof_ev_r[2 * S->prof_n + 1], S->hi));
-  CK(cudaEventRecord(S->rules_done[b], S->hi));
-  CK(cudaStreamWaitEvent(st, S->rules_done[b], 0));
-  rc = after_rules();
-  if (rc != FPC_OK) return rc;
-  CK(cudaStreamWaitEvent(S->side, S->rules_done[b], 0));
-  if (prof) CK(cudaEventRecord(S->prof_ev[2 * S->prof_n], S->side));
-  {
-    static thread_local int sms[MAX_DEVICES] = {0};
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (!sms[dev]) CK(cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev));
-    const int grid = p.n < sms[dev] ? p.n : sms[dev];
-    expand_kernel<G><<<grid, EXPAND_THREADS, 0, S->side>>>(p.cells, d.planes, p.flats, d.mask, p.n);
-  }
-  CK(cudaGetLastError());
-  if (prof) {
-    CK(cudaEventRecord(S->prof_ev[2 * S->prof_n + 1], S->side));
-    ++S->prof_n;
-  }
-  // Which event marks the end of this expansion.  A TIMESTAMPED record is the robust one: measured on B200
-  // (tools/overlap_probe.py, DESIGN.md section 3 item 5) it costs ~2 us per step against a plain record when the caller
-  // runs far ahead of the device (76.3 vs 74.2 us per step), but with the plain record a loop that starts from
-  // an idle device loses ~250 us (20 steps: ~90 vs 79 us per step), and a caller that waits for every step's results
-  // before issuing the next one falls into a mode of 176 us per step (83 us with the timestamped record).  So: the
-  // timestamped record whenever a call finds an internal stream idle, and for the STARTUP_CALLS calls after that; the
-  // plain one only while the caller keeps both streams busy.
-  constexpr int STARTUP_CALLS = 8;
-  if (side_was_idle) S->startup_left = STARTUP_CALLS;
-  S->expand_done[b] = S->startup_left > 0 ? S->expand_done_stamped[b] : S->expand_done_plain[b];
-  if (S->startup_left > 0) --S->startup_left;
-  CK(cudaEventRecord(S->expand_done[b], S->side));
-  S->expand_recorded[b] = true;
-  S->last = b;
-  S->last_async = (d.flags & FPC_FLAG_ASYNC_DENSE) != 0;
-  if (!S->last_async) CK(cudaStreamWaitEvent(st, S->expand_done[b], 0));
-  return FPC_OK;
+  return launch_full<G>(p, d, *S, st, after_rules);
 }
 template <class G>
 static int launch_make(const uint8_t *in, const uint64_t *moves, const int32_t *flat, int n, uint8_t *out,
@@ -646,14 +631,16 @@ int fpc_record_from_fen(int R, const char *fen, int honour_castling, uint8_t *h_
 }
 
 int fpc_profile_enable(int on) {
-  SideState *S = nullptr;
-  int rc = side_state(&S);
+  DeviceState *S = nullptr;
+  int rc = device_state(&S, true);
   if (rc != FPC_OK) return rc;
-  if (on && S->prof_ev.empty()) {
-    S->prof_ev.resize(2 * PROF_MAX);
-    for (auto &e : S->prof_ev) CK(cudaEventCreate(&e));
-    S->prof_ev_r.resize(2 * PROF_MAX);
-    for (auto &e : S->prof_ev_r) CK(cudaEventCreate(&e));
+  if (on && S->prof.empty()) {
+    S->prof.resize(PROF_MAX);
+    for (LaunchTimes &t : S->prof)
+      for (int i = 0; i < 2; ++i) {
+        CK(cudaEventCreate(&t.rules[i]));
+        CK(cudaEventCreate(&t.expand[i]));
+      }
   }
   S->prof_on = on != 0;
   S->prof_n = 0;
@@ -661,17 +648,18 @@ int fpc_profile_enable(int on) {
 }
 
 int fpc_profile_read(int *launches, double *expand_ms, double *rules_ms) {
-  SideState *S = nullptr;
-  int rc = side_state(&S);
+  DeviceState *S = nullptr;
+  int rc = device_state(&S, true);
   if (rc != FPC_OK) return rc;
   CK(cudaStreamSynchronize(S->side));
   CK(cudaStreamSynchronize(S->hi));
   double total = 0, total_r = 0;
   for (int i = 0; i < S->prof_n; ++i) {
+    const LaunchTimes &t = S->prof[i];
     float ms = 0;
-    CK(cudaEventElapsedTime(&ms, S->prof_ev[2 * i], S->prof_ev[2 * i + 1]));
+    CK(cudaEventElapsedTime(&ms, t.expand[0], t.expand[1]));
     total += ms;
-    CK(cudaEventElapsedTime(&ms, S->prof_ev_r[2 * i], S->prof_ev_r[2 * i + 1]));
+    CK(cudaEventElapsedTime(&ms, t.rules[0], t.rules[1]));
     total_r += ms;
   }
   if (launches) *launches = S->prof_n;
@@ -681,15 +669,36 @@ int fpc_profile_read(int *launches, double *expand_ms, double *rules_ms) {
 }
 
 int fpc_join(void *stream) {
-  int dev = 0;
-  CK(cudaGetDevice(&dev));
-  if (dev < 0 || dev >= MAX_DEVICES) return fail(FPC_ERR_ARG, "device ordinal out of range");
-  SideState &S = g_side[dev];
-  if (S.last >= 0) CK(cudaStreamWaitEvent((cudaStream_t)stream, S.expand_done[S.last], 0));
+  DeviceState *S = nullptr;
+  int rc = device_state(&S, false);
+  if (rc != FPC_OK) return rc;
+  if (S->last >= 0) CK(cudaStreamWaitEvent((cudaStream_t)stream, S->expand_done[S->last], 0));
   return FPC_OK;
 }
 
-int fpc_shutdown(void) { return side_release(); }
+// Releases everything this host thread holds on the current device.
+int fpc_shutdown(void) {
+  DeviceState *S = nullptr;
+  int rc = device_state(&S, false);
+  if (rc != FPC_OK) return rc;
+  if (S->side) {
+    CK(cudaStreamSynchronize(S->side));
+    CK(cudaStreamSynchronize(S->hi));
+    cudaStreamDestroy(S->side);
+    cudaStreamDestroy(S->hi);
+    cudaEventDestroy(S->fork);
+    for (int i = 0; i < 2; ++i) {
+      cudaEventDestroy(S->rules_done[i]);
+      cudaEventDestroy(S->expand_done_plain[i]);
+      cudaEventDestroy(S->expand_done_stamped[i]);
+    }
+  }
+  S->ws.release();
+  for (LaunchTimes &t : S->prof)
+    for (int i = 0; i < 2; ++i) cudaEventDestroy(t.rules[i]), cudaEventDestroy(t.expand[i]);
+  *S = DeviceState();
+  return FPC_OK;
+}
 
 fpc_dense_track *fpc_dense_track_create(int R, int n) {
   if (!fpc_supported(R) || n <= 0) {
@@ -702,7 +711,6 @@ fpc_dense_track *fpc_dense_track_create(int R, int n) {
   t->magic = TRACK_MAGIC;
   t->device = dev, t->R = R, t->n = n;
   t->planes = t->mask = nullptr;
-  t->cur_cells = t->cur_flats = 0;
   t->known_planes = t->known_mask = false;
   if (t->rec.reserve((size_t)n) != FPC_OK) {
     t->rec.release();
