@@ -18,6 +18,8 @@ STATUS_OVERFLOW, STATUS_FINISHED, STATUS_CHECK = 0x400, 0x800, 0x1000
 FLAG_ASYNC_DENSE = 1
 FLAG_INCREMENTAL = 2
 TREE_ADVANCE_MAX_NODE_CAP = 524288
+MAX_LEAVES_PER_GAME = 256
+SLOT_EMPTY, SLOT_LEAF, SLOT_COLLISION = 0, 1, 2
 
 _vp, _i, _u64 = C.c_void_p, C.c_int, C.c_uint64
 
@@ -55,6 +57,8 @@ SIGNATURES = {
     "fpc_tree_advance": (_i, [_vp, _vp, _vp, C.c_int32, C.c_int32, _vp, _vp]),
     "fpc_tree_select": (_i, [_vp, _i, _vp, _i, _vp, _vp]),
     "fpc_tree_expand_backup": (_i, [_vp, _vp, _vp, _vp]),
+    "fpc_tree_select_leaves": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp]),
+    "fpc_tree_expand_backup_leaves": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "fpc_ctx_create": (_vp, [_i, _i, _i]),
     "fpc_ctx_destroy": (None, [_vp]),
     "fpc_ctx_stream": (_vp, [_vp]),
@@ -95,6 +99,14 @@ class TreeDesc(C.Structure):
                  ("parent", "first_child", "n_children", "visits", "move_flat", "board_idx", "value_sum", "prior",
                   "n_nodes", "n_boards", "leaf", "dropped", "error", "boards", "leaf_boards", "leaf_flat",
                   "leaf_counts", "leaf_status", "k")])
+
+
+class LeafBatchDesc(C.Structure):
+    """struct fpc_leaf_batch (include/fpc.h): the leaf-parallel batch's device arrays."""
+    _fields_ = ([("L", C.c_int32), ("virtual_loss", C.c_int32)] +
+                [(name, C.c_void_p) for name in
+                 ("in_flight", "slot_node", "slot_kind", "leaf_boards", "leaf_flat", "leaf_counts", "leaf_status", "k",
+                  "priors", "collisions")])
 
 
 _LIB = None

@@ -590,6 +590,408 @@ __global__ void __launch_bounds__(EXP_THREADS, 8) tree_expand_backup_kernel(cons
   }
 }
 
+// ---- leaf-parallel PUCT (fpc_tree_select_leaves / fpc_tree_expand_backup_leaves; semantics in include/fpc.h) -------
+constexpr int LB_PATH = 64;  // path nodes a descent keeps in shared memory for its marks; deeper ones are re-walked
+
+// One warp per game, its L descents one after the other: slot j must see the marks of slots < j.  Each level is one
+// memory round as in tree_descend_kernel, with in_flight read beside visits; after the first descent the upper levels
+// come from the cache.
+template <class G>
+__global__ void __launch_bounds__(SEL_WARPS * 32) leaves_descend_kernel(const fpc_tree T, const fpc_leaf_batch B) {
+  __shared__ alignas(16) uint8_t recs[SEL_WARPS][256];
+  __shared__ int paths[SEL_WARPS][LB_PATH];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int g = blockIdx.x * SEL_WARPS + wib;
+  if (g >= T.n_games) return;
+  const int L = B.L, VL = B.virtual_loss;
+  const size_t s0 = (size_t)g * L, slab = (size_t)g * T.node_cap;
+  const int32_t *visits = T.visits + slab, *first_child = T.first_child + slab, *n_children = T.n_children + slab;
+  const double *value_sum = T.value_sum + slab;
+  const float *prior = T.prior + slab;
+  int32_t *in_flight = B.in_flight + slab;
+  uint8_t *pool = T.boards + (size_t)g * T.board_cap * G::REC;
+  int *path = paths[wib];
+  uint8_t *b = recs[wib];
+  int n_boards = T.n_boards[g], n_coll = 0, j = 0;
+  bool live = !T.dropped[g];
+  if (lane == 0) T.leaf[g] = -1;
+  for (; live && j < L; ++j) {
+    int node = 0, depth = 0, err = 0;
+    int nc = n_children[0], fc = first_child[0], nv = visits[0] + VL * in_flight[0];
+    if (lane == 0) path[0] = 0;
+    while (nc > 0) {
+      const double lg = log(sqrt((double)nv));
+      double best = -CUDART_INF;
+      int best_i = 0x7fffffff, b_nc = 0, b_fc = 0, b_nv = 0;
+      for (int i = lane; i < nc; i += 32) {
+        const int vl = VL * in_flight[fc + i];
+        const int n = visits[fc + i] + vl;
+        const int c_nc = n_children[fc + i], c_fc = first_child[fc + i];
+        const double q = n > 0 ? (value_sum[fc + i] - (double)vl) / (double)n : 0.0;
+        const double ucb = q + T.C * sqrt(lg / (double)(1 + n)) * (double)prior[fc + i];
+        if (ucb > best) {  // strict: the first maximum wins
+          best = ucb;
+          best_i = i;
+          b_nc = c_nc, b_fc = c_fc, b_nv = n;
+        }
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        const double ob = __shfl_xor_sync(FULL, best, o);
+        const int oi = __shfl_xor_sync(FULL, best_i, o);
+        const int o_nc = __shfl_xor_sync(FULL, b_nc, o), o_fc = __shfl_xor_sync(FULL, b_fc, o), o_nv = __shfl_xor_sync(FULL, b_nv, o);
+        if (oi != 0x7fffffff && (best_i == 0x7fffffff || ob > best || (ob == best && oi < best_i))) {
+          best = ob;
+          best_i = oi;
+          b_nc = o_nc, b_fc = o_fc, b_nv = o_nv;
+        }
+      }
+      if (best_i == 0x7fffffff) {  // "Failed to select a child." (node.cpp:72-75)
+        err = ERR_NO_CHILD;
+        break;
+      }
+      node = fc + best_i;
+      ++depth;
+      if (lane == 0 && depth < LB_PATH) path[depth] = node;
+      nc = b_nc, fc = b_fc, nv = b_nv;
+    }
+    const bool coll = !err && in_flight[node] > 0;
+    if (!err) {
+      int bi = T.board_idx[slab + node];
+      if (bi < 0) {  // a LEAF reached for the first time (a collision's endpoint was materialised by an earlier slot)
+        const int pb = T.board_idx[slab + T.parent[slab + node]];
+        if (lane < G::REC / 16) reinterpret_cast<uint4 *>(b)[lane] = reinterpret_cast<const uint4 *>(pool + (size_t)pb * G::REC)[lane];
+        __syncwarp();
+        int ok = 1;
+        if (lane == 0) {
+          int from, to;
+          decode_flat_move<G>(T.move_flat[slab + node], from, to);
+          ok = apply_move_record<G>(b, from, to, NO_PIECE, G::NSQ, G::NSQ, 0) ? 1 : 0;
+        }
+        ok = __shfl_sync(FULL, ok, 0);
+        bi = n_boards;
+        if (bi >= T.board_cap || !ok) {
+          err = ok ? ERR_BOARD_CAP : ERR_MOVE;
+        } else {
+          __syncwarp();
+          if (lane < G::REC / 16) reinterpret_cast<uint4 *>(pool + (size_t)bi * G::REC)[lane] = reinterpret_cast<const uint4 *>(b)[lane];
+          if (lane == 0) T.board_idx[slab + node] = bi;
+          n_boards = bi + 1;
+        }
+      } else {
+        if (lane < G::REC / 16) reinterpret_cast<uint4 *>(b)[lane] = reinterpret_cast<const uint4 *>(pool + (size_t)bi * G::REC)[lane];
+        __syncwarp();
+      }
+    }
+    if (err) {  // this slot and the later ones stay EMPTY; the earlier slots keep their marks
+      if (lane == 0) {
+        T.error[g] |= err;
+        T.dropped[g] = 1;
+      }
+      live = false;
+      break;
+    }
+    const size_t s = s0 + j;
+    if (lane < G::REC / 16) reinterpret_cast<uint4 *>(B.leaf_boards + s * G::REC)[lane] = reinterpret_cast<const uint4 *>(b)[lane];
+    if (lane == 0) {
+      B.slot_node[s] = node;
+      B.slot_kind[s] = coll ? FPC_SLOT_COLLISION : FPC_SLOT_LEAF;
+      B.k[s] = b[G::OFF_TURN] & 3;
+      if (j == 0 && !coll) T.leaf[g] = node;
+    }
+    n_coll += coll;
+    // the marks: the first LB_PATH levels from shared memory in one round, a deeper rest by a walk up from the endpoint
+    __syncwarp();
+    const int top = min(depth, LB_PATH - 1);
+    for (int i = lane; i <= top; i += 32) in_flight[path[i]] += 1;
+    if (lane == 0 && depth > top)
+      for (int x = node; x != path[top]; x = T.parent[slab + x]) in_flight[x] += 1;
+    __syncwarp();  // the next descent reads these marks
+  }
+  for (int jj = j + lane; jj < L; jj += 32) {
+    B.slot_node[s0 + jj] = -1;
+    B.slot_kind[s0 + jj] = FPC_SLOT_EMPTY;
+    B.k[s0 + jj] = 0;
+  }
+  if (lane == 0) {
+    T.n_boards[g] = n_boards;
+    if (n_coll) B.collisions[g] += n_coll;
+  }
+}
+
+// tree_batch_k_kernel over the slots: k <- side to move of the first LEAF slot whose status says IN_PROGRESS
+template <class G>
+__global__ void __launch_bounds__(1024) leaves_batch_k_kernel(const fpc_leaf_batch B, int n_slots) {
+  __shared__ int first;
+  if (threadIdx.x == 0) first = 0x7fffffff;
+  __syncthreads();
+  int mine = 0x7fffffff;
+  for (int s = threadIdx.x; s < n_slots; s += blockDim.x)
+    if (B.slot_kind[s] == FPC_SLOT_LEAF && (B.leaf_status[s] & FPC_STATUS_RESULT_MASK) == 0) {
+      mine = s;
+      break;
+    }
+  if (mine != 0x7fffffff) atomicMin(&first, mine);
+  __syncthreads();
+  if (first == 0x7fffffff) return;
+  const int k = B.leaf_boards[(size_t)first * G::REC + G::OFF_TURN] & 3;
+  for (int s = threadIdx.x; s < n_slots; s += blockDim.x) B.k[s] = k;
+}
+
+// Per-slot priors, one CTA per LEAF slot that is in progress: tree_expand_backup_kernel's soft-max, un-rotation, mask
+// and renormalisation, statement for statement (so the priors are its bits), into B.priors[slot][i] for the legal
+// entries i < count; 0 where no child is made (a repeated promotion index).
+template <class G>
+__global__ void __launch_bounds__(EXP_THREADS, 8) leaves_priors_kernel(const fpc_leaf_batch B, const float *logits) {
+  __shared__ float red_m[EXP_WARPS], red_s[EXP_WARPS];
+  __shared__ double red_d[EXP_WARPS];
+  __shared__ float s_max, s_sum;
+  __shared__ double s_msum;
+  const size_t s = blockIdx.x;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (B.slot_kind[s] != FPC_SLOT_LEAF || (B.leaf_status[s] & FPC_STATUS_RESULT_MASK) != 0) return;
+  const int cnt = B.leaf_counts[s];
+  const int k = B.k[s] & 3;
+  constexpr int PER = (MAX_MOVES + EXP_THREADS - 1) / EXP_THREADS;
+  const float *lg = logits + s * G::ASZ;
+  int flat[PER];
+  float lgt[PER];
+  bool first[PER];
+#pragma unroll
+  for (int q = 0; q < PER; ++q) {
+    const int i = tid + q * EXP_THREADS;
+    flat[q] = -1, lgt[q] = 0.0f, first[q] = false;
+    if (i < cnt) {
+      flat[q] = B.leaf_flat[s * MAX_MOVES + i];
+      first[q] = i == 0 || B.leaf_flat[s * MAX_MOVES + i - 1] != flat[q];  // promotions share an index
+      if (first[q]) {
+        const int plane = flat[q] / G::NSQ, sq = flat[q] - plane * G::NSQ;
+        int r = sq / G::R, c = sq - r * G::R;
+        for (int t = 0; t < k; ++t) {
+          const int nr = G::R - 1 - c;
+          c = r;
+          r = nr;
+        }
+        lgt[q] = __ldg(lg + plane * G::NSQ + r * G::R + c);
+      }
+    }
+  }
+  float m = -FLT_MAX, s_ = 0.0f;
+  const float4 *lg4 = reinterpret_cast<const float4 *>(lg);
+  constexpr int N4 = G::ASZ / 4;
+  int i = tid;
+  for (; i + 3 * EXP_THREADS < N4; i += 4 * EXP_THREADS) {
+    const float4 a = __ldcs(lg4 + i), b = __ldcs(lg4 + i + EXP_THREADS), c = __ldcs(lg4 + i + 2 * EXP_THREADS),
+                 d = __ldcs(lg4 + i + 3 * EXP_THREADS);
+    const float mx = fmaxf(fmaxf(fmaxf(fmaxf(a.x, a.y), fmaxf(a.z, a.w)), fmaxf(fmaxf(b.x, b.y), fmaxf(b.z, b.w))),
+                           fmaxf(fmaxf(fmaxf(c.x, c.y), fmaxf(c.z, c.w)), fmaxf(fmaxf(d.x, d.y), fmaxf(d.z, d.w))));
+    const float nm = fmaxf(m, mx);
+    s_ = s_ * __expf(m - nm) + ((__expf(a.x - nm) + __expf(a.y - nm)) + (__expf(a.z - nm) + __expf(a.w - nm))) +
+         ((__expf(b.x - nm) + __expf(b.y - nm)) + (__expf(b.z - nm) + __expf(b.w - nm))) +
+         ((__expf(c.x - nm) + __expf(c.y - nm)) + (__expf(c.z - nm) + __expf(c.w - nm))) +
+         ((__expf(d.x - nm) + __expf(d.y - nm)) + (__expf(d.z - nm) + __expf(d.w - nm)));
+    m = nm;
+  }
+  for (; i < N4; i += EXP_THREADS) {
+    const float4 a = __ldcs(lg4 + i);
+    const float nm = fmaxf(m, fmaxf(fmaxf(a.x, a.y), fmaxf(a.z, a.w)));
+    s_ = s_ * __expf(m - nm) + ((__expf(a.x - nm) + __expf(a.y - nm)) + (__expf(a.z - nm) + __expf(a.w - nm)));
+    m = nm;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) softmax_merge(m, s_, __shfl_xor_sync(FULL, m, o), __shfl_xor_sync(FULL, s_, o));
+  if (lane == 0) {
+    red_m[warp] = m;
+    red_s[warp] = s_;
+  }
+  __syncthreads();
+  if (tid == 0) {
+    float M = red_m[0];
+    for (int w = 1; w < EXP_WARPS; ++w) M = fmaxf(M, red_m[w]);
+    double S = 0.0;
+    for (int w = 0; w < EXP_WARPS; ++w)
+      if (red_s[w] > 0.0f) S += (double)red_s[w] * (double)expf(red_m[w] - M);
+    s_max = M;
+    s_sum = (float)S;
+  }
+  __syncthreads();
+  float p[PER];
+  double psum = 0.0;
+#pragma unroll
+  for (int q = 0; q < PER; ++q) {
+    p[q] = first[q] ? expf(lgt[q] - s_max) / s_sum : 0.0f;
+    psum += (double)p[q];
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) psum += __shfl_xor_sync(FULL, psum, o);
+  if (lane == 0) red_d[warp] = psum;
+  __syncthreads();
+  if (tid == 0) {
+    double t = 0.0;
+    for (int w = 0; w < EXP_WARPS; ++w) t += red_d[w];
+    s_msum = t;
+  }
+  __syncthreads();
+#pragma unroll
+  for (int q = 0; q < PER; ++q) {
+    const int i = tid + q * EXP_THREADS;
+    if (i < cnt) B.priors[s * MAX_MOVES + i] = first[q] ? (float)((double)p[q] / s_msum) : 0.0f;
+  }
+}
+
+// Per-game commit, one CTA per game: children slot by slot against the running node count, then the backup of every
+// LEAF slot.  The backup gathers one (node, slot, sign) entry per node of each LEAF path, sorts them by (node, slot) in
+// shared memory and lets one thread add each node's entries in ascending slot order: the bits of a sequential
+// slot-by-slot backup without a serial walk of L paths.  More entries than LB_ENTRIES (very deep paths) take that
+// serial walk instead.  The same walks clear in_flight on every path of the batch.
+constexpr int LB_THREADS = 256, LB_WARPS = LB_THREADS / 32;
+constexpr int LB_ENTRIES = 4096;  // 32 KB of keys
+static_assert(FPC_MAX_LEAVES_PER_GAME <= (1 << 30), "slot index and sign share the low 32 bits of a key");
+
+template <class G>
+__global__ void __launch_bounds__(LB_THREADS) leaves_commit_kernel(const fpc_tree T, const fpc_leaf_batch B, const float *values) {
+  __shared__ unsigned long long s_ent[LB_ENTRIES];
+  __shared__ int s_node[FPC_MAX_LEAVES_PER_GAME], s_cnt[FPC_MAX_LEAVES_PER_GAME], s_base[FPC_MAX_LEAVES_PER_GAME];
+  __shared__ float s_val[FPC_MAX_LEAVES_PER_GAME];
+  __shared__ int8_t s_what[FPC_MAX_LEAVES_PER_GAME];  // 0 no backup, 1 terminal LEAF, 2 LEAF in progress
+  __shared__ int s_ne;
+  const int g = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int L = B.L;
+  const size_t s0 = (size_t)g * L, slab = (size_t)g * T.node_cap;
+  if (tid == 0) s_ne = 0;
+  for (int j = tid; j < L; j += LB_THREADS) {
+    const int kind = B.slot_kind[s0 + j];
+    const int result = B.leaf_status[s0 + j] & FPC_STATUS_RESULT_MASK;
+    int what = 0;
+    float v = 0.0f;
+    if (kind == FPC_SLOT_LEAF) {
+      what = result ? 1 : 2;
+      v = result == 3 ? 0.0f : result ? -1.0f : values[s0 + j];
+    }
+    s_node[j] = kind == FPC_SLOT_EMPTY ? -1 : B.slot_node[s0 + j];
+    s_what[j] = (int8_t)what;
+    s_val[j] = v;
+  }
+  __syncthreads();
+  // children per slot (one per non-zero prior), one warp per slot
+  for (int j = warp; j < L; j += LB_WARPS) {
+    int n = 0;
+    if (s_what[j] == 2) {
+      const int cnt = B.leaf_counts[s0 + j];
+      for (int i0 = 0; i0 < cnt; i0 += 32) {
+        const int i = i0 + lane;
+        n += __popc(__ballot_sync(FULL, i < cnt && B.priors[(s0 + j) * MAX_MOVES + i] != 0.0f));
+      }
+    }
+    if (lane == 0) s_cnt[j] = n;
+  }
+  __syncthreads();
+  if (tid == 0) {  // allocation in slot order, each slot checked against the running count
+    int nn = T.n_nodes[g], err = 0, drop = 0;
+    for (int j = 0; j < L; ++j) {
+      s_base[j] = -1;
+      drop |= s_what[j] == 1;
+      if (s_what[j] != 2) continue;
+      if (nn + s_cnt[j] > T.node_cap) {
+        err = ERR_NODE_CAP;
+      } else {
+        s_base[j] = nn;
+        nn += s_cnt[j];
+      }
+    }
+    T.n_nodes[g] = nn;
+    if (err) T.error[g] |= err;
+    if (drop) T.dropped[g] = 1;
+  }
+  __syncthreads();
+  for (int j = warp; j < L; j += LB_WARPS) {
+    const int base = s_base[j];
+    if (base < 0) continue;
+    const int leaf = s_node[j], cnt = B.leaf_counts[s0 + j];
+    int written = 0;
+    for (int i0 = 0; i0 < cnt; i0 += 32) {
+      const int i = i0 + lane;
+      const float prior = i < cnt ? B.priors[(s0 + j) * MAX_MOVES + i] : 0.0f;
+      const bool make = i < cnt && prior != 0.0f;
+      const unsigned bal = __ballot_sync(FULL, make);
+      if (make) {
+        const size_t c = slab + base + written + __popc(bal & ((1u << lane) - 1u));
+        T.parent[c] = leaf;
+        T.first_child[c] = 0;
+        T.n_children[c] = 0;
+        T.visits[c] = 1;  // node.h:28
+        T.move_flat[c] = B.leaf_flat[(s0 + j) * MAX_MOVES + i];
+        T.board_idx[c] = -1;
+        T.value_sum[c] = 0.0;
+        T.prior[c] = prior;
+      }
+      written += __popc(bal);
+    }
+    if (lane == 0) {
+      T.first_child[slab + leaf] = base;
+      T.n_children[slab + leaf] = s_cnt[j];
+    }
+  }
+  // the paths, one thread per slot: clear the marks; gather the backup entries of the LEAF slots
+  for (int j = tid; j < L; j += LB_THREADS) {
+    const bool backup = s_what[j] != 0;
+    unsigned par = 0;
+    for (int node = s_node[j]; node >= 0; node = T.parent[slab + node], par ^= 1u) {
+      B.in_flight[slab + node] = 0;
+      if (backup) {
+        const int e = atomicAdd(&s_ne, 1);
+        if (e < LB_ENTRIES) s_ent[e] = (unsigned long long)node << 32 | (unsigned)j << 1 | par;
+      }
+    }
+  }
+  __syncthreads();
+  const int ne = s_ne;
+  if (ne > LB_ENTRIES) {  // Node::Backpropagate slot by slot
+    if (tid == 0)
+      for (int j = 0; j < L; ++j) {
+        if (!s_what[j]) continue;
+        double v = (double)s_val[j];
+        for (int node = s_node[j]; node >= 0; node = T.parent[slab + node]) {
+          T.value_sum[slab + node] += v;
+          T.visits[slab + node] += 1;
+          v = -v;
+        }
+      }
+    return;
+  }
+  int np = 1;
+  while (np < ne) np <<= 1;
+  for (int e = ne + tid; e < np; e += LB_THREADS) s_ent[e] = ~0ull;
+  __syncthreads();
+  for (int kk = 2; kk <= np; kk <<= 1)  // bitonic sort, ascending
+    for (int jj = kk >> 1; jj > 0; jj >>= 1) {
+      for (int e = tid; e < np; e += LB_THREADS) {
+        const int o = e ^ jj;
+        if (o > e) {
+          const unsigned long long a = s_ent[e], b = s_ent[o];
+          if ((a > b) == ((e & kk) == 0)) {
+            s_ent[e] = b;
+            s_ent[o] = a;
+          }
+        }
+      }
+      __syncthreads();
+    }
+  for (int e = tid; e < ne; e += LB_THREADS) {
+    const int node = (int)(s_ent[e] >> 32);
+    if (e > 0 && (int)(s_ent[e - 1] >> 32) == node) continue;
+    double acc = T.value_sum[slab + node];
+    int n = 0;
+    for (int t = e; t < ne && (int)(s_ent[t] >> 32) == node; ++t, ++n) {
+      const unsigned lo = (unsigned)s_ent[t];
+      const double v = (double)s_val[lo >> 1];
+      acc += (lo & 1u) ? -v : v;
+    }
+    T.value_sum[slab + node] = acc;
+    T.visits[slab + node] += n;
+  }
+}
+
 static int check_tree(const fpc_tree *t, const char *who) {
   if (!t) return fail(FPC_ERR_ARG, std::string(who) + ": null tree");
   if (!fpc_supported(t->R) || t->n_games < 0 || t->node_cap < 1 || t->board_cap < 1)
@@ -599,6 +1001,19 @@ static int check_tree(const fpc_tree *t, const char *who) {
        !t->value_sum || !t->prior || !t->n_nodes || !t->n_boards || !t->leaf || !t->dropped || !t->error ||
        !t->boards || !t->leaf_boards || !t->leaf_flat || !t->leaf_counts || !t->leaf_status || !t->k))
     return fail(FPC_ERR_ARG, std::string(who) + ": null tree array");
+  return FPC_OK;
+}
+
+static int check_batch(const fpc_tree *t, const fpc_leaf_batch *b, const char *who) {
+  if (!b) return fail(FPC_ERR_ARG, std::string(who) + ": null leaf batch");
+  if (b->L < 1 || b->L > FPC_MAX_LEAVES_PER_GAME)
+    return fail(FPC_ERR_ARG, std::string(who) + ": L = " + std::to_string(b->L) + " outside 1 .. " +
+                                 std::to_string(FPC_MAX_LEAVES_PER_GAME));
+  if (b->virtual_loss < 1) return fail(FPC_ERR_ARG, std::string(who) + ": virtual_loss below 1");
+  if ((int64_t)t->n_games * b->L > INT32_MAX) return fail(FPC_ERR_ARG, std::string(who) + ": n_games * L too large");
+  if (t->n_games > 0 && (!b->in_flight || !b->slot_node || !b->slot_kind || !b->leaf_boards || !b->leaf_flat ||
+                         !b->leaf_counts || !b->leaf_status || !b->k || !b->priors || !b->collisions))
+    return fail(FPC_ERR_ARG, std::string(who) + ": null leaf-batch array");
   return FPC_OK;
 }
 
@@ -686,6 +1101,53 @@ int fpc_tree_expand_backup(const fpc_tree *t, const float *d_logits, const float
   return dispatch(t->R, [&](auto g) {
     tree_expand_backup_kernel<decltype(g)><<<t->n_games, EXP_THREADS, 0, st>>>(*t, d_logits, d_values);
     return cuda_check(cudaGetLastError(), "tree_expand_backup_kernel launch");
+  });
+}
+
+int fpc_tree_select_leaves(const fpc_tree *t, const fpc_leaf_batch *b, int batch_rotation, float *d_planes, int flags,
+                           fpc_dense_track *track, void *stream) {
+  int rc = check_tree(t, "fpc_tree_select_leaves");
+  if (rc == FPC_OK) rc = check_batch(t, b, "fpc_tree_select_leaves");
+  if (rc != FPC_OK) return rc;
+  if (t->n_games == 0) return FPC_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int n_slots = t->n_games * b->L;
+  const int blocks = (t->n_games + SEL_WARPS - 1) / SEL_WARPS;
+  rc = dispatch(t->R, [&](auto g) {
+    leaves_descend_kernel<decltype(g)><<<blocks, SEL_WARPS * 32, 0, st>>>(*t, *b);
+    return cuda_check(cudaGetLastError(), "leaves_descend_kernel launch");
+  });
+  if (rc != FPC_OK) return rc;
+  if (batch_rotation) {
+    rc = fpc_observe(t->R, b->leaf_boards, n_slots, nullptr, b->leaf_flat, b->leaf_counts, b->leaf_status, nullptr,
+                     nullptr, 0, nullptr, 0, stream);
+    if (rc != FPC_OK) return rc;
+    rc = dispatch(t->R, [&](auto g) {
+      leaves_batch_k_kernel<decltype(g)><<<1, 1024, 0, st>>>(*b, n_slots);
+      return cuda_check(cudaGetLastError(), "leaves_batch_k_kernel launch");
+    });
+    if (rc != FPC_OK) return rc;
+    return fpc_observe_tracked(track, t->R, b->leaf_boards, n_slots, nullptr, nullptr, nullptr, nullptr, d_planes, b->k, 0,
+                               nullptr, flags, stream);
+  }
+  return fpc_observe_tracked(track, t->R, b->leaf_boards, n_slots, nullptr, b->leaf_flat, b->leaf_counts, b->leaf_status,
+                             d_planes, b->k, 0, nullptr, flags, stream);
+}
+
+int fpc_tree_expand_backup_leaves(const fpc_tree *t, const fpc_leaf_batch *b, const float *d_logits,
+                                  const float *d_values, void *stream) {
+  int rc = check_tree(t, "fpc_tree_expand_backup_leaves");
+  if (rc == FPC_OK) rc = check_batch(t, b, "fpc_tree_expand_backup_leaves");
+  if (rc != FPC_OK) return rc;
+  if (t->n_games == 0) return FPC_OK;
+  if (!d_logits || !d_values) return fail(FPC_ERR_ARG, "fpc_tree_expand_backup_leaves: null logits / values");
+  if (reinterpret_cast<uintptr_t>(d_logits) & 15) return fail(FPC_ERR_ARG, "logits must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  return dispatch(t->R, [&](auto g) {
+    leaves_priors_kernel<decltype(g)><<<t->n_games * b->L, EXP_THREADS, 0, st>>>(*b, d_logits);
+    CK(cudaGetLastError());
+    leaves_commit_kernel<decltype(g)><<<t->n_games, LB_THREADS, 0, st>>>(*t, *b, d_values);
+    return cuda_check(cudaGetLastError(), "leaves_commit_kernel launch");
   });
 }
 

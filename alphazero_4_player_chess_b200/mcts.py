@@ -14,7 +14,7 @@ import ctypes as C
 import torch
 
 from . import _lib
-from ._lib import FPC_MAX_MOVES, TreeDesc, check
+from ._lib import FPC_MAX_MOVES, MAX_LEAVES_PER_GAME, LeafBatchDesc, TreeDesc, check
 from .geometry import GEOMETRIES, NUM_STATE_CHANNELS
 
 ERR_NODE_CAP, ERR_BOARD_CAP, ERR_NO_CHILD, ERR_MOVE = 1, 2, 4, 8
@@ -25,7 +25,7 @@ NODES_PER_SIM = 96
 class BatchedMCTS:
     def __init__(self, R: int, n_games: int, neural_net, args: dict, device: str | torch.device = "cuda",
                  batch_rotation: bool = False, node_cap: int | None = None, cuda_graph: bool = False,
-                 reuse_tree: bool = False):
+                 reuse_tree: bool = False, leaves_per_game: int = 1, virtual_loss: int = 1):
         """args: the reference's dict (`alphazero.py:291-306`): uses "C" and "num_searches".
         batch_rotation=True reproduces the reference bit for bit (a whole leaf batch is rotated by the
         colour of its first expandable state); False rotates every leaf by its own side to move.
@@ -33,7 +33,13 @@ class BatchedMCTS:
         three eager ones and replays it: the ~70 launches of a simulation become one.
         reuse_tree=True sizes the default capacities for `advance` (keeping the played move's subtree between moves):
         room for a kept subtree plus a full new search.  It changes nothing else; `advance` works either way, it only
-        keeps less with the smaller default arenas."""
+        keeps less with the smaller default arenas.
+        leaves_per_game=L > 1 evaluates L leaf slots per game in every network call (leaf parallelism, outside the
+        reference): each game descends L times per batch, every pending descent adding `virtual_loss` lost visits along
+        its path so that later descents of the batch pick other leaves; a descent that ends on a leaf already taken in
+        the batch is a collision and spends its slot without a visit (counted in `self.collisions`).  A search is then
+        num_searches / L batches of n_games * L network rows; L must divide num_searches.  The first batch after a
+        reset reaches the unexpanded root in every slot: one leaf and L - 1 collisions.  L = 1 is the one-leaf path."""
         self.geom = GEOMETRIES[R]
         self.R, self.n = R, int(n_games)
         self.net = neural_net
@@ -46,6 +52,14 @@ class BatchedMCTS:
         self._graph = None
         self.L = _lib.lib()
         sims = int(args["num_searches"])
+        self.leaves, self.virtual_loss = int(leaves_per_game), int(virtual_loss)
+        if not 1 <= self.leaves <= MAX_LEAVES_PER_GAME:
+            raise ValueError(f"leaves_per_game must be in 1 .. {MAX_LEAVES_PER_GAME}, got {self.leaves}")
+        if self.virtual_loss < 1:
+            raise ValueError(f"virtual_loss must be at least 1, got {self.virtual_loss}")
+        if sims % self.leaves:
+            raise ValueError(f"leaves_per_game={self.leaves} does not divide num_searches={sims}")
+        self._open = False  # a leaf batch was selected and not yet expanded: its in_flight marks are still set
         reuse = 2 if reuse_tree else 1
         self.node_cap = int(node_cap) if node_cap else 1 + reuse * NODES_PER_SIM * sims
         self.board_cap = reuse * sims + 2
@@ -72,9 +86,10 @@ class BatchedMCTS:
         self.leaf_counts = torch.zeros(n, **i32)
         self.leaf_status = torch.zeros(n, **i32)
         self.k = torch.zeros(n, **i32)
-        self.planes = torch.empty((n, NUM_STATE_CHANNELS, R, R), dtype=torch.float32, device=dev)
+        slots = n * self.leaves
+        self.planes = torch.empty((slots, NUM_STATE_CHANNELS, R, R), dtype=torch.float32, device=dev)
         with torch.cuda.device(self.device):
-            self._track = self.L.fpc_dense_track_create(R, n)  # lets select() update self.planes in place
+            self._track = self.L.fpc_dense_track_create(R, slots)  # lets select() update self.planes in place
         if not self._track:
             raise _lib.FpcError(self.L.fpc_last_error().decode())
         d = TreeDesc()
@@ -84,12 +99,43 @@ class BatchedMCTS:
                      "leaf_counts", "leaf_status", "k"):
             setattr(d, name, getattr(self, name).data_ptr())
         self.desc = d
+        self.batch = None
+        self.collisions = torch.zeros(n, **i32)  # collision slots since the last reset / advance (none at L = 1)
+        if self.leaves > 1:
+            # the leaf batch (struct fpc_leaf_batch): per-slot arrays for n * L slots, slot s = g * L + j
+            self.in_flight = torch.zeros((n, nc), **i32)  # zero between batches; the two leaf calls keep it so
+            self.slot_node = torch.full((slots,), -1, **i32)
+            self.slot_kind = torch.zeros(slots, **i32)
+            self.slot_boards = torch.zeros((slots, rec), dtype=torch.uint8, device=dev)
+            self.slot_flat = torch.zeros((slots, FPC_MAX_MOVES), **i32)
+            self.slot_counts = torch.zeros(slots, **i32)
+            self.slot_status = torch.zeros(slots, **i32)
+            self.slot_k = torch.zeros(slots, **i32)
+            self.slot_priors = torch.zeros((slots, FPC_MAX_MOVES), dtype=torch.float32, device=dev)
+            b = LeafBatchDesc()
+            b.L, b.virtual_loss = self.leaves, self.virtual_loss
+            for field, name in (("in_flight", "in_flight"), ("slot_node", "slot_node"), ("slot_kind", "slot_kind"),
+                                ("leaf_boards", "slot_boards"), ("leaf_flat", "slot_flat"),
+                                ("leaf_counts", "slot_counts"), ("leaf_status", "slot_status"), ("k", "slot_k"),
+                                ("priors", "slot_priors"), ("collisions", "collisions")):
+                setattr(b, field, getattr(self, name).data_ptr())
+            self.batch = b
 
     def _stream(self):
         return torch.cuda.current_stream(self.device).cuda_stream
 
+    def _close_batch(self) -> None:
+        """Before the trees are replaced or re-rooted: clear the marks of a leaf batch that was selected and never
+        expanded, and restart the collision count."""
+        if self._open:
+            self.in_flight.zero_()
+            self._open = False
+        if self.batch is not None:
+            self.collisions.zero_()
+
     # ---- the three device steps ----------------------------------------------------------------
     def reset(self, root_boards: torch.Tensor) -> None:
+        self._close_batch()
         roots = root_boards.to(self.device, torch.uint8).contiguous()
         assert roots.shape == (self.n, self.geom.record_bytes)
         with torch.cuda.device(self.device):
@@ -113,6 +159,7 @@ class BatchedMCTS:
         max_nodes = max(0, self.node_cap - NODES_PER_SIM * sims)
         max_boards = max(0, self.board_cap - sims)
         kept = torch.empty(self.n, dtype=torch.int32, device=self.device)
+        self._close_batch()
         with torch.cuda.device(self.device):
             check(self.L.fpc_tree_advance(C.byref(self.desc), acts.data_ptr(), roots.data_ptr(), max_nodes, max_boards,
                                           kept.data_ptr(), self._stream()))
@@ -120,12 +167,19 @@ class BatchedMCTS:
         return kept
 
     def select(self) -> torch.Tensor:
-        """Node.ChooseLeaf for every live game; returns the encoded leaf batch [n,24,R,R]."""
+        """Node.ChooseLeaf for every live game; returns the encoded leaf batch [n,24,R,R] ([n*L,24,R,R] with L leaf slots
+        per game, slot s = g*L + j; the rows of collision and empty slots are evaluated and ignored)."""
         # the planes tensor is resident and only read by the network between selects: after the first full encode
         # through this instance's handle it is updated in place (FPC_FLAG_INCREMENTAL)
         with torch.cuda.device(self.device):
-            check(self.L.fpc_tree_select(C.byref(self.desc), int(self.batch_rotation), self.planes.data_ptr(),
-                                         _lib.FLAG_INCREMENTAL, self._track, self._stream()))
+            if self.batch is None:
+                check(self.L.fpc_tree_select(C.byref(self.desc), int(self.batch_rotation), self.planes.data_ptr(),
+                                             _lib.FLAG_INCREMENTAL, self._track, self._stream()))
+            else:
+                check(self.L.fpc_tree_select_leaves(C.byref(self.desc), C.byref(self.batch), int(self.batch_rotation),
+                                                    self.planes.data_ptr(), _lib.FLAG_INCREMENTAL, self._track,
+                                                    self._stream()))
+                self._open = True
         return self.planes
 
     def close(self) -> None:
@@ -142,14 +196,21 @@ class BatchedMCTS:
     def expand_backup(self, logits: torch.Tensor, values: torch.Tensor) -> None:
         logits = logits.to(torch.float32).contiguous()
         values = values.to(torch.float32).reshape(-1).contiguous()
-        assert logits.shape == (self.n, self.geom.action_space_size) and values.shape == (self.n,)
+        rows = self.n * self.leaves
+        assert logits.shape == (rows, self.geom.action_space_size) and values.shape == (rows,)
         with torch.cuda.device(self.device):
-            check(self.L.fpc_tree_expand_backup(C.byref(self.desc), logits.data_ptr(), values.data_ptr(),
-                                                self._stream()))
+            if self.batch is None:
+                check(self.L.fpc_tree_expand_backup(C.byref(self.desc), logits.data_ptr(), values.data_ptr(),
+                                                    self._stream()))
+            else:
+                check(self.L.fpc_tree_expand_backup_leaves(C.byref(self.desc), C.byref(self.batch), logits.data_ptr(),
+                                                           values.data_ptr(), self._stream()))
+                self._open = False
 
     # ---- MCTS.search (mcts.py:17-43) -------------------------------------------------------------
     def simulate(self) -> None:
-        """One simulation for every live game (`MCTS.step` + `MCTS.expand`, mcts.py:59-89)."""
+        """One simulation for every live game (`MCTS.step` + `MCTS.expand`, mcts.py:59-89); with L leaf slots per game,
+        one batch of L slots per game."""
         planes = self.select()
         logits, value = self.net(planes)
         self.expand_backup(logits, value)
@@ -159,13 +220,17 @@ class BatchedMCTS:
         """num_searches simulations from fresh roots at root_boards, or, with root_boards=None, on top of the current
         trees (after advance(), or to add simulations to a finished search).
         record: optional callable(sim, logits, value) called after every network forward (eager mode only), e.g.
-        to keep the outputs of some games for a replay on the CPU oracle.  check: raise on tree errors (arena full ...)
+        to keep the outputs of some games for a replay on the CPU oracle (with L leaf slots per game: sim = the batch,
+        rows g*L + j).  check: raise on tree errors (arena full ...)
         instead of leaving them in `self.error`."""
         if root_boards is not None:
             self.reset(root_boards)
         elif not self._has_tree:
             raise _lib.FpcError("search(None) continues the current trees, but there are none: pass root_boards")
         sims = int(self.args["num_searches"])
+        if sims % self.leaves:
+            raise ValueError(f"leaves_per_game={self.leaves} does not divide num_searches={sims}")
+        sims //= self.leaves  # network batches
         done = 0
         if self.cuda_graph and record is None:
             # eager warm-up (the first select writes the planes in full; cuDNN / cuBLAS pick their kernels), then capture

@@ -24,19 +24,22 @@ from .mcts import BatchedMCTS
 
 class SelfPlay:
     def __init__(self, R: int, n_games: int, neural_net, args: dict, start_record, device="cuda",
-                 batch_rotation: bool = False, reuse_tree: bool = False):
+                 batch_rotation: bool = False, reuse_tree: bool = False, leaves_per_game: int = 1,
+                 virtual_loss: int = 1):
         """args: the reference's dict (`alphazero.py:291-306`); uses C, num_searches, temperature,
         max_game_length, heuristic_weight.  reuse_tree=True keeps the played move's subtree for the next move's search
         (`BatchedMCTS.advance`) where the reference starts every move from a fresh root: num_searches simulations are
         still added per move, on top of the visits carried over, and the policy targets are the root children's visit
-        counts including those."""
+        counts including those.  leaves_per_game / virtual_loss: leaf-parallel search (BatchedMCTS), num_searches / L
+        network batches of n_games * L leaf slots per move."""
         self.geom = GEOMETRIES[R]
         self.R, self.n, self.args = R, int(n_games), args
         self.device = torch.device(device)
         self.env = BatchedEnv(R, self.n, device=self.device)
         self.reuse_tree = bool(reuse_tree)
         self.mcts = BatchedMCTS(R, self.n, neural_net, args, device=self.device, batch_rotation=batch_rotation,
-                                reuse_tree=self.reuse_tree)
+                                reuse_tree=self.reuse_tree, leaves_per_game=leaves_per_game,
+                                virtual_loss=virtual_loss)
         self.start = torch.as_tensor(start_record, dtype=torch.uint8)
         T = int(args["max_game_length"])
         i32 = dict(dtype=torch.int32, device=self.device)
@@ -79,7 +82,7 @@ class SelfPlay:
             else:
                 self.mcts.reset(self.env.boards)
             self.mcts.dropped.copy_((~running).int())  # finished games take no part in the search
-            for _ in range(int(self.args["num_searches"])):
+            for _ in range(int(self.args["num_searches"]) // self.mcts.leaves):
                 planes = self.mcts.select()
                 logits, value = self.mcts.net(planes)
                 self.mcts.expand_backup(logits, value)

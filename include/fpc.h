@@ -278,6 +278,73 @@ int fpc_tree_select(const fpc_tree *t, int batch_rotation, float *d_planes, int 
  * node.h:28).  d_logits [n_games][A*R*R] f32 in the network's (rotated) frame, d_values [n_games]. */
 int fpc_tree_expand_backup(const fpc_tree *t, const float *d_logits, const float *d_values, void *stream);
 
+/* ---- leaf-parallel PUCT: several leaves per game in one network batch, with a virtual loss --------------------------
+ *
+ * Outside the reference (one leaf per game and simulation, mcts.py:17-43).  Every live game descends L times per batch,
+ * one slot after the other; in_flight[x] counts the earlier slots of the current batch whose path went through node x,
+ * and a descent sees the effective statistics
+ *   N_eff(x) = visits[x] + VL*in_flight[x],   W_eff(x) = value_sum[x] - (double)(VL*in_flight[x])
+ * in Node::SelectChild's arithmetic (q = n > 0 ? W_eff(c)/n : 0 with n = N_eff(c); ucb = q +
+ * C*sqrt(ln(sqrt(N_eff(x)))/(1+n))*P(c) in double; the first maximum wins).  With in_flight all zero this is
+ * fpc_tree_select's arithmetic to the bit, so slot 0 (and every slot at L = 1) selects what fpc_tree_select selects.
+ *
+ * Selection, game g, slots j = 0 .. L-1 in ascending order (slot s = g*L + j):
+ *   - the endpoint e is the first node with n_children == 0.  in_flight[e] > 0: a COLLISION (not evaluated; its slot
+ *     is spent without a visit).  Otherwise a LEAF, whose board is materialised as fpc_tree_select does it;
+ *   - in_flight += 1 on every node of the root -> e path, e and the root included (collisions too: that is what steers
+ *     later slots away);
+ *   - a descent error (no selectable child, board_cap, index-built move) sets the error bits of fpc_tree_select and
+ *     drops the game; slot j and every later slot of the game are EMPTY and add no marks.  A dropped game's slots are
+ *     all EMPTY.
+ * Every leaf and collision slot then goes through the rules kernel and the encoder (a collision carries its
+ * endpoint's board), into d_planes [n_games*L][24][R][R]: the network sees a static batch, so CUDA graphs work.
+ * batch_rotation != 0: k = the side to move of the first LEAF slot (ascending s) whose status is IN_PROGRESS.
+ * leaf[g] = the node of slot g*L when it is a LEAF, else -1 (at L = 1 what fpc_tree_select writes).
+ *
+ * Expand / backup, game g, slots in ascending j (the outputs of COLLISION and EMPTY slots are ignored):
+ *   - LEAF, terminal: Backpropagate(0 | -1); the game is dropped after this batch (its later slots still count: they
+ *     ran concurrently);
+ *   - LEAF, in progress: Backpropagate(value), then one child per non-zero prior appended at n_nodes, the priors
+ *     bit-identical to fpc_tree_expand_backup's for the same logits, k and legal list.  The node_cap check is made per
+ *     slot against the running n_nodes: a slot that does not fit sets error bit 0 and is backed up without children;
+ *   - the f64 additions to any one node's value_sum happen in ascending slot order: the bits of a sequential
+ *     slot-by-slot backup;
+ *   - afterwards in_flight is zero on every node again, whatever errors occurred.
+ * num_searches simulations are num_searches / L batches.  The first batch after a reset reaches the unexpanded root in
+ * every slot: one leaf, L-1 collisions.  Arena sizes per batch: at most one new board and one expansion per slot.
+ *
+ * fpc_tree_reset and fpc_tree_advance do not touch in_flight: the caller zeroes it once and the two calls below keep
+ * it zero.  L outside 1 .. FPC_MAX_LEAVES_PER_GAME, virtual_loss < 1, null arrays and misaligned logits are
+ * FPC_ERR_ARG, before any launch. */
+#define FPC_MAX_LEAVES_PER_GAME 256
+#define FPC_SLOT_EMPTY 0
+#define FPC_SLOT_LEAF 1
+#define FPC_SLOT_COLLISION 2
+typedef struct fpc_leaf_batch {
+  int32_t L;              /* leaf slots per game and batch */
+  int32_t virtual_loss;   /* VL >= 1 */
+  int32_t *in_flight;     /* [n_games][node_cap], zero between batches */
+  /* per slot, [n_games*L] */
+  int32_t *slot_node;     /* the endpoint of the slot's descent, -1 for an EMPTY slot */
+  int32_t *slot_kind;     /* FPC_SLOT_* */
+  uint8_t *leaf_boards;   /* [n_games*L][record] */
+  int32_t *leaf_flat;     /* [n_games*L][FPC_MAX_MOVES] */
+  int32_t *leaf_counts;
+  int32_t *leaf_status;
+  int32_t *k;
+  float *priors;          /* [n_games*L][FPC_MAX_MOVES] scratch of fpc_tree_expand_backup_leaves */
+  /* per game, [n_games] */
+  int32_t *collisions;    /* += the COLLISION slots of every select; the caller zeroes it */
+} fpc_leaf_batch;
+
+/* One batch's selection (see above), the rules kernel and the planes; flags + track as in fpc_tree_select (the track
+ * handle sized for n_games*L). */
+int fpc_tree_select_leaves(const fpc_tree *t, const fpc_leaf_batch *b, int batch_rotation, float *d_planes, int flags,
+                           fpc_dense_track *track, void *stream);
+/* The batch's expand / backup (see above).  d_logits [n_games*L][A*R*R] f32 (16-byte aligned), d_values [n_games*L]. */
+int fpc_tree_expand_backup_leaves(const fpc_tree *t, const fpc_leaf_batch *b, const float *d_logits,
+                                  const float *d_values, void *stream);
+
 /* ---- host-buffer operations (per-object calls of the binding; e2e measurement) ------------- */
 
 typedef struct fpc_ctx fpc_ctx;
