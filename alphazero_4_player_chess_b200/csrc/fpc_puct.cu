@@ -6,6 +6,7 @@
 #include <stdint.h>
 
 #include <cfloat>
+#include <cmath>
 #include <string>
 
 #include "../../include/fpc.h"
@@ -992,6 +993,69 @@ __global__ void __launch_bounds__(LB_THREADS) leaves_commit_kernel(const fpc_tre
   }
 }
 
+// ---- Dirichlet noise on the root's children (fpc_tree_root_noise; the recipe is stated in include/fpc.h) ------------
+constexpr int NOISE_ATTEMPTS = 64;  // Marsaglia-Tsang attempts before the deterministic fallback
+constexpr double TWO_PI = 6.283185307179586;
+
+// Uniform j of child i of the game with this key: never 0, so every log below is finite
+__device__ __forceinline__ double noise_uniform(uint64_t seed, uint64_t key, int i, int j) {
+  return ((double)(mix64(seed, key, (uint64_t)i << 32 | (uint32_t)j) >> 11) + 0.5) * 0x1p-53;
+}
+
+// Gamma(alpha, 1) for child i.  Attempt t reads uniforms 3t (Box-Muller radius), 3t+1 (angle) and 3t+2 (acceptance);
+// the alpha < 1 boost reads uniform 3 * NOISE_ATTEMPTS, so the draws of a child never depend on which attempt accepted.
+__device__ __noinline__ double noise_gamma(uint64_t seed, uint64_t key, int i, double alpha) {
+  const double a = alpha < 1.0 ? alpha + 1.0 : alpha;
+  const double d = a - 1.0 / 3.0, c = 1.0 / sqrt(9.0 * d);
+  double g = d;
+  for (int t = 0; t < NOISE_ATTEMPTS; ++t) {
+    const double x = sqrt(-2.0 * log(noise_uniform(seed, key, i, 3 * t))) * cos(TWO_PI * noise_uniform(seed, key, i, 3 * t + 1));
+    const double v = 1.0 + c * x;
+    if (v <= 0.0) continue;
+    const double v3 = v * v * v;
+    if (log(noise_uniform(seed, key, i, 3 * t + 2)) < 0.5 * x * x + d - d * v3 + d * log(v3)) {
+      g = d * v3;
+      break;
+    }
+  }
+  if (alpha < 1.0) g *= pow(noise_uniform(seed, key, i, 3 * NOISE_ATTEMPTS), 1.0 / alpha);
+  return g;
+}
+
+// One warp per game, child i on lane i % 32: the draws, the f64 sum in a fixed order (lane-wise ascending i, then the
+// xor tree), and the mix into the f32 priors.
+__global__ void __launch_bounds__(SEL_WARPS * 32) tree_root_noise_kernel(const fpc_tree T, uint64_t seed, const int64_t *keys,
+                                                                         double alpha, double eps, int32_t *done) {
+  const int lane = threadIdx.x & 31;
+  const int g = blockIdx.x * SEL_WARPS + (threadIdx.x >> 5);
+  if (g >= T.n_games || done[g] || T.dropped[g]) return;
+  const size_t slab = (size_t)g * T.node_cap;
+  const int k = T.n_children[slab], fc = T.first_child[slab];
+  if (k <= 0) return;
+  const uint64_t key = (uint64_t)keys[g];
+  constexpr int PER = (MAX_MOVES + 31) / 32;
+  double gam[PER];
+  double sum = 0.0;
+#pragma unroll
+  for (int q = 0; q < PER; ++q) {
+    const int i = lane + 32 * q;
+    gam[q] = i < k ? noise_gamma(seed, key, i, alpha) : 0.0;
+    sum += gam[q];
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(FULL, sum, o);
+#pragma unroll
+  for (int q = 0; q < PER; ++q) {
+    const int i = lane + 32 * q;
+    if (i < k) {
+      const double eta = sum > 0.0 ? gam[q] / sum : 1.0 / k;  // sum 0: every draw underflowed (alpha below ~0.05)
+      float *p = T.prior + slab + fc + i;
+      *p = (float)((1.0 - eps) * (double)*p + eps * eta);
+    }
+  }
+  if (lane == 0) done[g] = 1;
+}
+
 static int check_tree(const fpc_tree *t, const char *who) {
   if (!t) return fail(FPC_ERR_ARG, std::string(who) + ": null tree");
   if (!fpc_supported(t->R) || t->n_games < 0 || t->node_cap < 1 || t->board_cap < 1)
@@ -1149,6 +1213,22 @@ int fpc_tree_expand_backup_leaves(const fpc_tree *t, const fpc_leaf_batch *b, co
     leaves_commit_kernel<decltype(g)><<<t->n_games, LB_THREADS, 0, st>>>(*t, *b, d_values);
     return cuda_check(cudaGetLastError(), "leaves_commit_kernel launch");
   });
+}
+
+int fpc_tree_root_noise(const fpc_tree *t, uint64_t seed, const int64_t *d_keys, float alpha, float epsilon,
+                        int32_t *d_done, void *stream) {
+  int rc = check_tree(t, "fpc_tree_root_noise");
+  if (rc != FPC_OK) return rc;
+  if (!(alpha > 0.0f) || !std::isfinite(alpha))
+    return fail(FPC_ERR_ARG, "fpc_tree_root_noise: alpha must be positive and finite, got " + std::to_string(alpha));
+  if (!(epsilon >= 0.0f && epsilon <= 1.0f))
+    return fail(FPC_ERR_ARG, "fpc_tree_root_noise: epsilon outside [0, 1]: " + std::to_string(epsilon));
+  if (t->n_games == 0) return FPC_OK;
+  if (!d_keys || !d_done) return fail(FPC_ERR_ARG, "fpc_tree_root_noise: null keys / done");
+  const int blocks = (t->n_games + SEL_WARPS - 1) / SEL_WARPS;
+  tree_root_noise_kernel<<<blocks, SEL_WARPS * 32, 0, (cudaStream_t)stream>>>(*t, seed, d_keys, (double)alpha,
+                                                                              (double)epsilon, d_done);
+  return cuda_check(cudaGetLastError(), "tree_root_noise_kernel launch");
 }
 
 }  // extern "C"

@@ -25,7 +25,8 @@ NODES_PER_SIM = 96
 class BatchedMCTS:
     def __init__(self, R: int, n_games: int, neural_net, args: dict, device: str | torch.device = "cuda",
                  batch_rotation: bool = False, node_cap: int | None = None, cuda_graph: bool = False,
-                 reuse_tree: bool = False, leaves_per_game: int = 1, virtual_loss: int = 1):
+                 reuse_tree: bool = False, leaves_per_game: int = 1, virtual_loss: int = 1, root_noise: bool = False,
+                 noise_seed: int = 0):
         """args: the reference's dict (`alphazero.py:291-306`): uses "C" and "num_searches".
         batch_rotation=True reproduces the reference bit for bit (a whole leaf batch is rotated by the
         colour of its first expandable state); False rotates every leaf by its own side to move.
@@ -39,7 +40,11 @@ class BatchedMCTS:
         its path so that later descents of the batch pick other leaves; a descent that ends on a leaf already taken in
         the batch is a collision and spends its slot without a visit (counted in `self.collisions`).  A search is then
         num_searches / L batches of n_games * L network rows; L must divide num_searches.  The first batch after a
-        reset reaches the unexpanded root in every slot: one leaf and L - 1 collisions.  L = 1 is the one-leaf path."""
+        reset reaches the unexpanded root in every slot: one leaf and L - 1 collisions.  L = 1 is the one-leaf path.
+        root_noise=True mixes AlphaZero's exploration noise into the root's children priors (outside the reference):
+        prior <- (1 - eps) * prior + eps * Dir(alpha) with alpha = args["dirichlet_alpha"] and eps =
+        args["dirichlet_epsilon"], both required then; once per root, i.e. per reset / advance (`add_root_noise`,
+        `search`).  A game's draws depend only on (noise_seed, its key).  root_noise=False changes nothing."""
         self.geom = GEOMETRIES[R]
         self.R, self.n = R, int(n_games)
         self.net = neural_net
@@ -120,18 +125,29 @@ class BatchedMCTS:
                                 ("priors", "slot_priors"), ("collisions", "collisions")):
                 setattr(b, field, getattr(self, name).data_ptr())
             self.batch = b
+        self.root_noise = bool(root_noise)
+        if self.root_noise:
+            missing = [key for key in ("dirichlet_alpha", "dirichlet_epsilon") if key not in args]
+            if missing:
+                raise ValueError(f"root_noise=True needs args {missing}")
+            self.noise_alpha, self.noise_eps = float(args["dirichlet_alpha"]), float(args["dirichlet_epsilon"])
+            self.noise_seed = int(noise_seed) & (2**64 - 1)
+            self.noise_done = torch.zeros(n, **i32)  # 1 once the current root was noised; zeroed by reset / advance
+            self._searches = 0
 
     def _stream(self):
         return torch.cuda.current_stream(self.device).cuda_stream
 
     def _close_batch(self) -> None:
         """Before the trees are replaced or re-rooted: clear the marks of a leaf batch that was selected and never
-        expanded, and restart the collision count."""
+        expanded, and restart the collision count and the root-noise marks."""
         if self._open:
             self.in_flight.zero_()
             self._open = False
         if self.batch is not None:
             self.collisions.zero_()
+        if self.root_noise:
+            self.noise_done.zero_()  # a new root: noised again by the next add_root_noise
 
     # ---- the three device steps ----------------------------------------------------------------
     def reset(self, root_boards: torch.Tensor) -> None:
@@ -182,6 +198,20 @@ class BatchedMCTS:
                 self._open = True
         return self.planes
 
+    def add_root_noise(self, keys) -> None:
+        """Dirichlet noise on the root's children priors of every game whose root is expanded, not dropped and not yet
+        noised since the last reset / advance (`fpc_tree_root_noise`); keys [n] i64 select the games' draws.  A caller
+        that drives select / expand_backup itself calls it before its first batch and again right after it: the second
+        call reaches the roots that the first batch expanded."""
+        if not self.root_noise:
+            raise _lib.FpcError("add_root_noise() needs BatchedMCTS(..., root_noise=True)")
+        keys = torch.as_tensor(keys, dtype=torch.int64).to(self.device).contiguous()
+        assert keys.shape == (self.n,)
+        with torch.cuda.device(self.device):
+            check(self.L.fpc_tree_root_noise(C.byref(self.desc), self.noise_seed, keys.data_ptr(), self.noise_alpha,
+                                             self.noise_eps, self.noise_done.data_ptr(), self._stream()))
+        self._noise_keys = keys  # keep alive until the kernel has run
+
     def close(self) -> None:
         if getattr(self, "_track", None):
             self.L.fpc_dense_track_destroy(self._track)
@@ -216,13 +246,18 @@ class BatchedMCTS:
         self.expand_backup(logits, value)
 
     @torch.no_grad()
-    def search(self, root_boards: torch.Tensor | None = None, record=None, check: bool = True) -> "BatchedMCTS":
+    def search(self, root_boards: torch.Tensor | None = None, record=None, check: bool = True,
+               noise_keys=None) -> "BatchedMCTS":
         """num_searches simulations from fresh roots at root_boards, or, with root_boards=None, on top of the current
         trees (after advance(), or to add simulations to a finished search).
         record: optional callable(sim, logits, value) called after every network forward (eager mode only), e.g.
         to keep the outputs of some games for a replay on the CPU oracle (with L leaf slots per game: sim = the batch,
         rows g*L + j).  check: raise on tree errors (arena full ...)
-        instead of leaving them in `self.error`."""
+        instead of leaving them in `self.error`.
+        noise_keys: with root_noise=True, the [n] i64 keys of this search's root noise (default arange(n) + n * s for
+        this instance's s-th search).  add_root_noise runs before the first batch (roots that already have children:
+        a kept subtree) and right after it (roots the first batch expanded), outside the CUDA graph; a root noised since
+        the last reset / advance is not noised again."""
         if root_boards is not None:
             self.reset(root_boards)
         elif not self._has_tree:
@@ -231,12 +266,25 @@ class BatchedMCTS:
         if sims % self.leaves:
             raise ValueError(f"leaves_per_game={self.leaves} does not divide num_searches={sims}")
         sims //= self.leaves  # network batches
+        keys = None
+        if self.root_noise:
+            keys = noise_keys
+            if keys is None:
+                keys = torch.arange(self.n, dtype=torch.int64, device=self.device) + self.n * self._searches
+            self._searches += 1
+            self.add_root_noise(keys)
+
+        def after_batch(done):
+            if done == 1 and keys is not None:
+                self.add_root_noise(keys)
+
         done = 0
         if self.cuda_graph and record is None:
             # eager warm-up (the first select writes the planes in full; cuDNN / cuBLAS pick their kernels), then capture
             while self._graph is None and done < min(3, sims):
                 self.simulate()
                 done += 1
+                after_batch(done)
             if self._graph is None and done < sims:
                 torch.cuda.synchronize(self.device)
                 g = torch.cuda.CUDAGraph()
@@ -246,6 +294,7 @@ class BatchedMCTS:
             while done < sims:
                 self._graph.replay()
                 done += 1
+                after_batch(done)
         else:
             for sim in range(sims):
                 planes = self.select()
@@ -253,6 +302,7 @@ class BatchedMCTS:
                 if record is not None:
                     record(sim, logits, value)
                 self.expand_backup(logits, value)
+                after_batch(sim + 1)
         if check:
             self.check_errors()
         return self

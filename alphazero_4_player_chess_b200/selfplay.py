@@ -25,13 +25,16 @@ from .mcts import BatchedMCTS
 class SelfPlay:
     def __init__(self, R: int, n_games: int, neural_net, args: dict, start_record, device="cuda",
                  batch_rotation: bool = False, reuse_tree: bool = False, leaves_per_game: int = 1,
-                 virtual_loss: int = 1):
+                 virtual_loss: int = 1, root_noise: bool = False, noise_seed: int = 0):
         """args: the reference's dict (`alphazero.py:291-306`); uses C, num_searches, temperature,
         max_game_length, heuristic_weight.  reuse_tree=True keeps the played move's subtree for the next move's search
         (`BatchedMCTS.advance`) where the reference starts every move from a fresh root: num_searches simulations are
         still added per move, on top of the visits carried over, and the policy targets are the root children's visit
         counts including those.  leaves_per_game / virtual_loss: leaf-parallel search (BatchedMCTS), num_searches / L
-        network batches of n_games * L leaf slots per move."""
+        network batches of n_games * L leaf slots per move.  root_noise / noise_seed: Dirichlet noise on every move's
+        root priors (BatchedMCTS; args then needs dirichlet_alpha and dirichlet_epsilon), keyed by g * max_game_length + t
+        for game g at ply t, so the noise of a game does not depend on the batch it plays in; play() with the same
+        noise_seed draws the same noise again."""
         self.geom = GEOMETRIES[R]
         self.R, self.n, self.args = R, int(n_games), args
         self.device = torch.device(device)
@@ -39,7 +42,7 @@ class SelfPlay:
         self.reuse_tree = bool(reuse_tree)
         self.mcts = BatchedMCTS(R, self.n, neural_net, args, device=self.device, batch_rotation=batch_rotation,
                                 reuse_tree=self.reuse_tree, leaves_per_game=leaves_per_game,
-                                virtual_loss=virtual_loss)
+                                virtual_loss=virtual_loss, root_noise=root_noise, noise_seed=noise_seed)
         self.start = torch.as_tensor(start_record, dtype=torch.uint8)
         T = int(args["max_game_length"])
         i32 = dict(dtype=torch.int32, device=self.device)
@@ -82,10 +85,16 @@ class SelfPlay:
             else:
                 self.mcts.reset(self.env.boards)
             self.mcts.dropped.copy_((~running).int())  # finished games take no part in the search
-            for _ in range(int(self.args["num_searches"]) // self.mcts.leaves):
+            keys = None
+            if self.mcts.root_noise:
+                keys = torch.arange(n, dtype=torch.int64, device=self.device) * T + t
+                self.mcts.add_root_noise(keys)  # the roots a kept subtree brought
+            for b in range(int(self.args["num_searches"]) // self.mcts.leaves):
                 planes = self.mcts.select()
                 logits, value = self.mcts.net(planes)
                 self.mcts.expand_backup(logits, value)
+                if b == 0 and keys is not None:
+                    self.mcts.add_root_noise(keys)  # the roots the first batch expanded
             flat, visits, _, _ = self.mcts.root_children()
             self.hist_boards[t].copy_(self.env.boards)
             self.hist_flat[t].copy_(flat)

@@ -345,6 +345,31 @@ int fpc_tree_select_leaves(const fpc_tree *t, const fpc_leaf_batch *b, int batch
 int fpc_tree_expand_backup_leaves(const fpc_tree *t, const fpc_leaf_batch *b, const float *d_logits,
                                   const float *d_values, void *stream);
 
+/* ---- Dirichlet exploration noise at the root ------------------------------------------------------------------------
+ *
+ * AlphaZero's root noise, outside the reference (its args carry dirichlet_alpha / dirichlet_epsilon, alphazero.py:291-306,
+ * and mcts.py:45 defines add_dirichlet_noise, which nothing calls).  For every game g with d_done[g] == 0,
+ * dropped[g] == 0 and k = n_children[0] > 0, the root's children c_i = first_child[0] + i, i = 0 .. k-1 (slab order):
+ *   gamma_i ~ Gamma(alpha, 1) as below;  eta_i = gamma_i / S with S = sum_i gamma_i in f64 (S == 0, possible only
+ *   when every draw underflows at alpha below ~0.05: eta_i = 1/k);
+ *   prior[c_i] = (float)((1 - (double)epsilon) * (double)prior[c_i] + (double)epsilon * eta_i);  d_done[g] = 1.
+ * Nothing else is written, and games that fail the condition are left exactly as they are, so a second call with the
+ * same d_done changes nothing.  The order of the f64 sum is fixed by the kernel (a restatement that sums in another
+ * order may differ in the last bits of S).
+ *
+ * The draws are counter-based: those of game g depend only on (seed, d_keys[g], i), never on g's place in the batch,
+ * the launch shape or the GPU.  With mix64 of csrc/fpc_device.cuh, uniform j of child i is, in double arithmetic,
+ *   U(i, j) = ((double)(mix64(seed, (uint64_t)d_keys[g], (uint64_t)i << 32 | j) >> 11) + 0.5) * 2^-53   (never 0).
+ * Gamma (Marsaglia-Tsang, f64): a = alpha < 1 ? alpha + 1 : alpha, d = a - 1/3, c = 1/sqrt(9d).  Attempt t = 0 .. 63:
+ *   x = sqrt(-2 ln U(i, 3t)) * cos(2pi * U(i, 3t+1))  (Box-Muller, 2pi = 6.283185307179586);  v = 1 + c*x;
+ *   v <= 0: rejected;  else V = v^3, accepted when ln U(i, 3t+2) < x*x/2 + d - d*V + d*ln V, giving d*V.
+ * After 64 rejections the draw is d itself.  For alpha < 1 the result is multiplied by U(i, 192)^(1/alpha).
+ *
+ * alpha not positive and finite, epsilon outside [0, 1], null d_keys / d_done and a bad tree are FPC_ERR_ARG, before
+ * any launch.  d_keys [n_games] i64, d_done [n_games] i32. */
+int fpc_tree_root_noise(const fpc_tree *t, uint64_t seed, const int64_t *d_keys, float alpha, float epsilon,
+                        int32_t *d_done, void *stream);
+
 /* ---- host-buffer operations (per-object calls of the binding; e2e measurement) ------------- */
 
 typedef struct fpc_ctx fpc_ctx;
