@@ -60,6 +60,8 @@ SIGNATURES = {
     "fpc_tree_select_leaves": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp]),
     "fpc_tree_expand_backup_leaves": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "fpc_tree_root_noise": (_i, [_vp, _u64, _vp, C.c_float, C.c_float, _vp, _vp]),
+    "fpc_tree_select_gumbel": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp]),
+    "fpc_tree_gumbel_result": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "fpc_ctx_create": (_vp, [_i, _i, _i]),
     "fpc_ctx_destroy": (None, [_vp]),
     "fpc_ctx_stream": (_vp, [_vp]),
@@ -108,6 +110,12 @@ class LeafBatchDesc(C.Structure):
                 [(name, C.c_void_p) for name in
                  ("in_flight", "slot_node", "slot_kind", "leaf_boards", "leaf_flat", "leaf_counts", "leaf_status", "k",
                   "priors", "collisions")])
+
+
+class GumbelDesc(C.Structure):
+    """struct fpc_gumbel (include/fpc.h): the Gumbel root search's parameters and per-game device arrays."""
+    _fields_ = [("seed", C.c_uint64), ("keys", C.c_void_p), ("max_considered", C.c_int32), ("n_sims", C.c_int32),
+                ("scale", C.c_double), ("c_visit", C.c_double), ("c_scale", C.c_double), ("root_value", C.c_void_p)]
 
 
 _LIB = None

@@ -252,17 +252,12 @@ __global__ void __launch_bounds__(ADV_THREADS) tree_advance_kernel(const fpc_tre
   }
 }
 
-// Node::ChooseLeaf's descent (node.cpp:21-26) + Node::SelectChild (node.cpp:49-78).
-template <class G>
-__global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_kernel(const fpc_tree T) {
-  __shared__ alignas(16) uint8_t recs[SEL_WARPS][256];
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  const int g = blockIdx.x * SEL_WARPS + wib;
-  if (g >= T.n_games) return;
-  if (T.dropped[g]) {
-    if (lane == 0) T.leaf[g] = -1;
-    return;
-  }
+// Node::ChooseLeaf's descent (node.cpp:21-26) + Node::SelectChild (node.cpp:49-78), then the leaf's board materialised
+// into leaf_boards.  One warp of game g; `b` is the warp's 256-byte record scratch in shared memory.  root_step(node, nc,
+// fc, nv) may replace the root's step: it receives the root (node 0) and its (n_children, first_child, visits), may move
+// them to the node the descent continues from, and returns false when it has dropped the game.
+template <class G, class RootStep>
+__device__ __forceinline__ void descend(const fpc_tree &T, int g, int lane, uint8_t *b, RootStep root_step) {
   const size_t slab = (size_t)g * T.node_cap;
   const int32_t *visits = T.visits + slab, *first_child = T.first_child + slab, *n_children = T.n_children + slab;
   const double *value_sum = T.value_sum + slab;
@@ -271,6 +266,7 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_kernel(const fpc_
   // its child's own child range, and the winner's (first_child, n_children, visits) travel with the arg-max.
   int node = 0;
   int nc = n_children[0], fc = first_child[0], nv = visits[0];
+  if (!root_step(node, nc, fc, nv)) return;
   while (nc > 0) {
     const double lg = log(sqrt((double)nv));
     double best = -CUDART_INF;
@@ -311,7 +307,6 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_kernel(const fpc_
   // materialise the leaf's board: parent's board + MakeMove(Move(flat_index)) (node.cpp:87-92)
   uint8_t *pool = T.boards + (size_t)g * T.board_cap * G::REC;
   int bi = T.board_idx[slab + node];
-  uint8_t *b = recs[wib];
   if (bi < 0) {
     const int pb = T.board_idx[slab + T.parent[slab + node]];
     if (lane < G::REC / 16) reinterpret_cast<uint4 *>(b)[lane] = reinterpret_cast<const uint4 *>(pool + (size_t)pb * G::REC)[lane];
@@ -347,6 +342,19 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_kernel(const fpc_
     T.leaf[g] = node;
     T.k[g] = b[G::OFF_TURN] & 3;
   }
+}
+
+template <class G>
+__global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_kernel(const fpc_tree T) {
+  __shared__ alignas(16) uint8_t recs[SEL_WARPS][256];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int g = blockIdx.x * SEL_WARPS + wib;
+  if (g >= T.n_games) return;
+  if (T.dropped[g]) {
+    if (lane == 0) T.leaf[g] = -1;
+    return;
+  }
+  descend<G>(T, g, lane, recs[wib], [](int &, int &, int &, int &) { return true; });
 }
 
 // The reference rotates a whole leaf batch by the colour of states[0] (src/cpp/board.cpp:354-355,
@@ -1056,6 +1064,198 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_root_noise_kernel(const f
   if (lane == 0) done[g] = 1;
 }
 
+// ---- Gumbel root search (fpc_tree_select_gumbel / fpc_tree_gumbel_result; the semantics are stated in include/fpc.h) --
+// One warp per game, root child i on lane i % 32 in register i / 32.  Every f64 sum runs lane-wise in ascending i, then
+// over the xor butterfly 16 .. 1; products and sums are spelled __dmul_rn / __dadd_rn so that no FMA contraction changes
+// the bits a restatement computes.
+constexpr int GB_PER = (MAX_MOVES + 31) / 32;
+constexpr int GUMBEL_J = INT32_MIN;  // the draws' uniform j = 2^31: a stream disjoint from the root noise's j <= 192
+constexpr double GUMBEL_FLOOR = -1e9;
+
+// mctx's get_sequence_of_considered_visits(m, n_sims)[s] in closed form, extended past n_sims.  Once c is 2 it stays 2,
+// and every later phase adds one visit per two simulations.
+__device__ __forceinline__ int considered_visits(int s, int m, int n_sims) {
+  if (m <= 1) return s;
+  int l2 = 0;
+  while ((1 << l2) < m) ++l2;
+  int c = m, v = 0;
+  while (c > 2) {
+    const int e = max(1, n_sims / (l2 * c));
+    if (s < e * c) return v + s / c;
+    s -= e * c;
+    v += e;
+    c = max(2, c / 2);
+  }
+  return v + s / 2;
+}
+
+// Game g's k > 0 root children (the first at fc): n = N_i and z = l_i + sigma_i in this lane's registers, nmax = max N_i;
+// returns s = sum N_i.  The select (write_root_value) records the root's value_sum as root_value when s == 0.
+__device__ __forceinline__ int gumbel_logits(const fpc_tree &T, const fpc_gumbel &B, int g, int lane, int fc, int k,
+                                             bool write_root_value, int (&n)[GB_PER], double (&z)[GB_PER], int &nmax) {
+  const size_t slab = (size_t)g * T.node_cap;
+  double q[GB_PER];
+  int s = 0;
+  nmax = INT32_MIN;
+  double lmax = -CUDART_INF, wq = 0.0, ws = 0.0;
+#pragma unroll
+  for (int r = 0; r < GB_PER; ++r) {
+    const int i = lane + 32 * r;
+    n[r] = -1, q[r] = 0.0;
+    if (i < k) {
+      const size_t c = slab + fc + i;
+      const double p = (double)T.prior[c];
+      n[r] = T.visits[c] - 1;  // children are created with visit_count 1 (node.h:28)
+      lmax = fmax(lmax, log(p));
+      s += n[r];
+      nmax = max(nmax, n[r]);
+      if (n[r] > 0) {
+        q[r] = T.value_sum[c] / (double)n[r];
+        const double w = fmax(p, 0x1p-126);
+        wq = __dadd_rn(wq, __dmul_rn(w, q[r]));
+        ws = __dadd_rn(ws, w);
+      }
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    s += __shfl_xor_sync(FULL, s, o);
+    nmax = max(nmax, __shfl_xor_sync(FULL, nmax, o));
+    lmax = fmax(lmax, __shfl_xor_sync(FULL, lmax, o));
+    wq = __dadd_rn(wq, __shfl_xor_sync(FULL, wq, o));
+    ws = __dadd_rn(ws, __shfl_xor_sync(FULL, ws, o));
+  }
+  const double root = s == 0 ? T.value_sum[slab] : B.root_value[g];
+  if (write_root_value && s == 0 && lane == 0) B.root_value[g] = root;
+  const double w_mean = ws > 0.0 ? wq / ws : 0.0;
+  const double v_mix = __dadd_rn(-root, __dmul_rn((double)s, w_mean)) / (1.0 + (double)s);
+  double lo = CUDART_INF, hi = -CUDART_INF;
+#pragma unroll
+  for (int r = 0; r < GB_PER; ++r) {
+    if (lane + 32 * r < k) {
+      if (n[r] <= 0) q[r] = v_mix;  // completed Q
+      lo = fmin(lo, q[r]);
+      hi = fmax(hi, q[r]);
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    lo = fmin(lo, __shfl_xor_sync(FULL, lo, o));
+    hi = fmax(hi, __shfl_xor_sync(FULL, hi, o));
+  }
+  const double span = fmax(hi - lo, 1e-8);
+  const double a = __dmul_rn(B.c_visit + (double)nmax, B.c_scale);
+  // log p_i is taken again here rather than kept in registers across the divisions above
+#pragma unroll
+  for (int r = 0; r < GB_PER; ++r) {
+    const int i = lane + 32 * r;
+    z[r] = i < k ? __dadd_rn(log((double)T.prior[slab + fc + i]) - lmax, __dmul_rn(a, (q[r] - lo) / span)) : -CUDART_INF;
+  }
+  return s;
+}
+
+// The child index maximising max(GUMBEL_FLOOR, g_i + z_i) over the children with N_i == cv (the first maximum in
+// ascending i), or -1 when there is none.
+__device__ __forceinline__ int gumbel_argmax(const fpc_gumbel &B, uint64_t key, int lane, int k, int cv,
+                                             const int (&n)[GB_PER], const double (&z)[GB_PER]) {
+  double best = -CUDART_INF;
+  int best_i = 0x7fffffff;
+#pragma unroll
+  for (int r = 0; r < GB_PER; ++r) {
+    const int i = lane + 32 * r;
+    if (i < k && n[r] == cv) {
+      const double gum = -log(-log(noise_uniform(B.seed, key, i, GUMBEL_J)));
+      const double x = __dadd_rn(__dmul_rn(B.scale, gum), z[r]);
+      const double score = x > GUMBEL_FLOOR ? x : GUMBEL_FLOOR;
+      if (score > best) {  // strict: the first maximum wins
+        best = score;
+        best_i = i;
+      }
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const double ob = __shfl_xor_sync(FULL, best, o);
+    const int oi = __shfl_xor_sync(FULL, best_i, o);
+    if (oi != 0x7fffffff && (best_i == 0x7fffffff || ob > best || (ob == best && oi < best_i))) {
+      best = ob;
+      best_i = oi;
+    }
+  }
+  return best_i == 0x7fffffff ? -1 : best_i;
+}
+
+// fpc_tree_select with the Gumbel root step: the root's child by sequential halving, then Node::SelectChild below it.
+template <class G>
+__global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_gumbel_kernel(const fpc_tree T, const fpc_gumbel B) {
+  __shared__ alignas(16) uint8_t recs[SEL_WARPS][256];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int g = blockIdx.x * SEL_WARPS + wib;
+  if (g >= T.n_games) return;
+  if (T.dropped[g]) {
+    if (lane == 0) T.leaf[g] = -1;
+    return;
+  }
+  descend<G>(T, g, lane, recs[wib], [&](int &node, int &nc, int &fc, int &nv) {
+    if (nc <= 0) return true;  // an unexpanded root is the leaf, as in fpc_tree_select
+    int n[GB_PER], nmax;
+    double z[GB_PER];
+    const int s = gumbel_logits(T, B, g, lane, fc, nc, true, n, z, nmax);
+    const int i = gumbel_argmax(B, (uint64_t)B.keys[g], lane, nc, considered_visits(s, min(B.max_considered, nc), B.n_sims), n, z);
+    if (i < 0) {  // a root visit left the schedule: drop the game as a failed SelectChild does
+      if (lane == 0) {
+        T.error[g] |= ERR_NO_CHILD;
+        T.leaf[g] = -1;
+        T.dropped[g] = 1;
+      }
+      return false;
+    }
+    const size_t slab = (size_t)g * T.node_cap;
+    node = fc + i;
+    nc = T.n_children[slab + node], fc = T.first_child[slab + node], nv = T.visits[slab + node];
+    return true;
+  });
+}
+
+// The action (the considered child at cv = Nmax with the best score) and the improved policy softmax(l + sigma).
+__global__ void __launch_bounds__(SEL_WARPS * 32) tree_gumbel_result_kernel(const fpc_tree T, const fpc_gumbel B,
+                                                                             int32_t *action, float *policy) {
+  const int lane = threadIdx.x & 31;
+  const int g = blockIdx.x * SEL_WARPS + (threadIdx.x >> 5);
+  if (g >= T.n_games) return;
+  const size_t slab = (size_t)g * T.node_cap;
+  const int k = T.n_children[slab], fc = T.first_child[slab];
+  float *row = policy + (size_t)g * MAX_MOVES;
+  if (k <= 0) {
+    for (int i = lane; i < MAX_MOVES; i += 32) row[i] = 0.0f;
+    if (lane == 0) action[g] = -1;
+    return;
+  }
+  int n[GB_PER], nmax;
+  double z[GB_PER];
+  gumbel_logits(T, B, g, lane, fc, k, false, n, z, nmax);
+  const int best = gumbel_argmax(B, (uint64_t)B.keys[g], lane, k, nmax, n, z);
+  double zmax = -CUDART_INF, sum = 0.0;
+#pragma unroll
+  for (int r = 0; r < GB_PER; ++r)
+    if (lane + 32 * r < k) zmax = fmax(zmax, z[r]);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) zmax = fmax(zmax, __shfl_xor_sync(FULL, zmax, o));
+#pragma unroll
+  for (int r = 0; r < GB_PER; ++r) {
+    z[r] = lane + 32 * r < k ? exp(z[r] - zmax) : 0.0;
+    sum = __dadd_rn(sum, z[r]);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) sum = __dadd_rn(sum, __shfl_xor_sync(FULL, sum, o));
+#pragma unroll
+  for (int r = 0; r < GB_PER; ++r) {
+    const int i = lane + 32 * r;
+    if (i < MAX_MOVES) row[i] = (float)(z[r] / sum);
+  }
+  if (lane == 0) action[g] = best < 0 ? -1 : T.move_flat[slab + fc + best];
+}
+
 static int check_tree(const fpc_tree *t, const char *who) {
   if (!t) return fail(FPC_ERR_ARG, std::string(who) + ": null tree");
   if (!fpc_supported(t->R) || t->n_games < 0 || t->node_cap < 1 || t->board_cap < 1)
@@ -1089,6 +1289,43 @@ static int launch_advance(const fpc_tree &t, const int32_t *actions, const uint8
     CK(cudaFuncSetAttribute(tree_advance_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   tree_advance_kernel<G><<<t.n_games, ADV_THREADS, smem, st>>>(t, actions, roots, max_nodes, max_boards, kept);
   return cuda_check(cudaGetLastError(), "tree_advance_kernel launch");
+}
+
+static int check_gumbel(const fpc_tree *t, const fpc_gumbel *gb, const char *who) {
+  if (!gb) return fail(FPC_ERR_ARG, std::string(who) + ": null gumbel");
+  if (gb->max_considered < 1 || gb->max_considered > FPC_MAX_MOVES)
+    return fail(FPC_ERR_ARG, std::string(who) + ": max_considered " + std::to_string(gb->max_considered) + " outside 1 .. " +
+                                 std::to_string(FPC_MAX_MOVES));
+  if (gb->n_sims < 0) return fail(FPC_ERR_ARG, std::string(who) + ": negative n_sims");
+  const double params[3] = {gb->scale, gb->c_visit, gb->c_scale};
+  const char *names[3] = {"scale", "c_visit", "c_scale"};
+  for (int i = 0; i < 3; ++i)
+    if (!(params[i] >= 0.0) || !std::isfinite(params[i]))
+      return fail(FPC_ERR_ARG, std::string(who) + ": " + names[i] + " must be non-negative and finite");
+  if (t->n_games > 0 && (!gb->keys || !gb->root_value)) return fail(FPC_ERR_ARG, std::string(who) + ": null keys / root_value");
+  return FPC_OK;
+}
+
+// What fpc_tree_select does after its descent: the rules kernel on the leaf batch (legal moves + GetGameResult) and the
+// planes, rotated by the first live leaf's colour with batch_rotation.
+static int observe_leaves(const fpc_tree *t, int batch_rotation, float *d_planes, int flags, fpc_dense_track *track,
+                          void *stream) {
+  if (batch_rotation) {
+    // the batch rotation is that of the first NON-terminal leaf: results first, then k, then the planes
+    int rc = fpc_observe(t->R, t->leaf_boards, t->n_games, nullptr, t->leaf_flat, t->leaf_counts, t->leaf_status, nullptr,
+                         nullptr, 0, nullptr, 0, stream);
+    if (rc != FPC_OK) return rc;
+    rc = dispatch(t->R, [&](auto g) {
+      tree_batch_k_kernel<decltype(g)><<<1, 1024, 0, (cudaStream_t)stream>>>(*t);
+      return cuda_check(cudaGetLastError(), "tree_batch_k_kernel launch");
+    });
+    if (rc != FPC_OK) return rc;
+    return fpc_observe_tracked(track, t->R, t->leaf_boards, t->n_games, nullptr, nullptr, nullptr, nullptr, d_planes, t->k, 0,
+                               nullptr, flags, stream);
+  }
+  // legal moves + GetGameResult + planes of the leaf batch: the environment's rules kernel
+  return fpc_observe_tracked(track, t->R, t->leaf_boards, t->n_games, nullptr, t->leaf_flat, t->leaf_counts, t->leaf_status,
+                             d_planes, t->k, 0, nullptr, flags, stream);
 }
 
 }  // namespace fpc
@@ -1137,22 +1374,34 @@ int fpc_tree_select(const fpc_tree *t, int batch_rotation, float *d_planes, int 
     return cuda_check(cudaGetLastError(), "tree_descend_kernel launch");
   });
   if (rc != FPC_OK) return rc;
-  if (batch_rotation) {
-    // the batch rotation is that of the first NON-terminal leaf: results first, then k, then the planes
-    rc = fpc_observe(t->R, t->leaf_boards, t->n_games, nullptr, t->leaf_flat, t->leaf_counts, t->leaf_status, nullptr,
-                     nullptr, 0, nullptr, 0, stream);
-    if (rc != FPC_OK) return rc;
-    rc = dispatch(t->R, [&](auto g) {
-      tree_batch_k_kernel<decltype(g)><<<1, 1024, 0, st>>>(*t);
-      return cuda_check(cudaGetLastError(), "tree_batch_k_kernel launch");
-    });
-    if (rc != FPC_OK) return rc;
-    return fpc_observe_tracked(track, t->R, t->leaf_boards, t->n_games, nullptr, nullptr, nullptr, nullptr, d_planes, t->k, 0,
-                               nullptr, flags, stream);
-  }
-  // legal moves + GetGameResult + planes of the leaf batch: the environment's rules kernel
-  return fpc_observe_tracked(track, t->R, t->leaf_boards, t->n_games, nullptr, t->leaf_flat, t->leaf_counts, t->leaf_status,
-                             d_planes, t->k, 0, nullptr, flags, stream);
+  return observe_leaves(t, batch_rotation, d_planes, flags, track, stream);
+}
+
+int fpc_tree_select_gumbel(const fpc_tree *t, const fpc_gumbel *gb, int batch_rotation, float *d_planes, int flags,
+                           fpc_dense_track *track, void *stream) {
+  int rc = check_tree(t, "fpc_tree_select_gumbel");
+  if (rc == FPC_OK) rc = check_gumbel(t, gb, "fpc_tree_select_gumbel");
+  if (rc != FPC_OK) return rc;
+  if (t->n_games == 0) return FPC_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int blocks = (t->n_games + SEL_WARPS - 1) / SEL_WARPS;
+  rc = dispatch(t->R, [&](auto g) {
+    tree_descend_gumbel_kernel<decltype(g)><<<blocks, SEL_WARPS * 32, 0, st>>>(*t, *gb);
+    return cuda_check(cudaGetLastError(), "tree_descend_gumbel_kernel launch");
+  });
+  if (rc != FPC_OK) return rc;
+  return observe_leaves(t, batch_rotation, d_planes, flags, track, stream);
+}
+
+int fpc_tree_gumbel_result(const fpc_tree *t, const fpc_gumbel *gb, int32_t *d_action, float *d_policy, void *stream) {
+  int rc = check_tree(t, "fpc_tree_gumbel_result");
+  if (rc == FPC_OK) rc = check_gumbel(t, gb, "fpc_tree_gumbel_result");
+  if (rc != FPC_OK) return rc;
+  if (t->n_games == 0) return FPC_OK;
+  if (!d_action || !d_policy) return fail(FPC_ERR_ARG, "fpc_tree_gumbel_result: null action / policy");
+  const int blocks = (t->n_games + SEL_WARPS - 1) / SEL_WARPS;
+  tree_gumbel_result_kernel<<<blocks, SEL_WARPS * 32, 0, (cudaStream_t)stream>>>(*t, *gb, d_action, d_policy);
+  return cuda_check(cudaGetLastError(), "tree_gumbel_result_kernel launch");
 }
 
 int fpc_tree_expand_backup(const fpc_tree *t, const float *d_logits, const float *d_values, void *stream) {

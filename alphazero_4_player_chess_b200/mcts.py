@@ -14,19 +14,22 @@ import ctypes as C
 import torch
 
 from . import _lib
-from ._lib import FPC_MAX_MOVES, MAX_LEAVES_PER_GAME, LeafBatchDesc, TreeDesc, check
+from ._lib import FPC_MAX_MOVES, MAX_LEAVES_PER_GAME, GumbelDesc, LeafBatchDesc, TreeDesc, check
 from .geometry import GEOMETRIES, NUM_STATE_CHANNELS
 
 ERR_NODE_CAP, ERR_BOARD_CAP, ERR_NO_CHILD, ERR_MOVE = 1, 2, 4, 8
 # node slots per simulation: a leaf adds at most FPC_MAX_MOVES children; the legal-move average is ~19-38 at 14x14
 NODES_PER_SIM = 96
+# sigma(q) = (GUMBEL_C_VISIT + max N) * GUMBEL_C_SCALE * q: the constants of Danihelka et al. (ICLR 2022) and mctx
+GUMBEL_C_VISIT, GUMBEL_C_SCALE = 50.0, 0.1
 
 
 class BatchedMCTS:
     def __init__(self, R: int, n_games: int, neural_net, args: dict, device: str | torch.device = "cuda",
                  batch_rotation: bool = False, node_cap: int | None = None, cuda_graph: bool = False,
                  reuse_tree: bool = False, leaves_per_game: int = 1, virtual_loss: int = 1, root_noise: bool = False,
-                 noise_seed: int = 0):
+                 noise_seed: int = 0, gumbel: bool = False, gumbel_seed: int = 0, gumbel_considered: int = 16,
+                 gumbel_scale: float = 1.0):
         """args: the reference's dict (`alphazero.py:291-306`): uses "C" and "num_searches".
         batch_rotation=True reproduces the reference bit for bit (a whole leaf batch is rotated by the
         colour of its first expandable state); False rotates every leaf by its own side to move.
@@ -44,7 +47,15 @@ class BatchedMCTS:
         root_noise=True mixes AlphaZero's exploration noise into the root's children priors (outside the reference):
         prior <- (1 - eps) * prior + eps * Dir(alpha) with alpha = args["dirichlet_alpha"] and eps =
         args["dirichlet_epsilon"], both required then; once per root, i.e. per reset / advance (`add_root_noise`,
-        `search`).  A game's draws depend only on (noise_seed, its key).  root_noise=False changes nothing."""
+        `search`).  A game's draws depend only on (noise_seed, its key).  root_noise=False changes nothing.
+        gumbel=True replaces the root's step by Gumbel AlphaZero's (Danihelka et al., ICLR 2022; outside the reference):
+        gumbel_considered root moves sampled without replacement by Gumbel-top-k on the prior logits, the simulations
+        spent on them by sequential halving, and `gumbel_result` gives the surviving move and the improved policy
+        softmax(logits + sigma(completed Q)) (include/fpc.h states the recipe).  Below the root the descent is the
+        reference's SelectChild.  A game's draws depend only on (gumbel_seed, its key); gumbel_scale=0 makes the search
+        deterministic.  The schedule is planned for num_searches - 1 root visits (the first batch expands the root) and
+        indexed by the root's own visits, so gumbel=True refuses reuse_tree, root_noise and leaves_per_game > 1, and
+        search(None) cannot continue a finished search.  gumbel=False changes nothing."""
         self.geom = GEOMETRIES[R]
         self.R, self.n = R, int(n_games)
         self.net = neural_net
@@ -125,6 +136,22 @@ class BatchedMCTS:
                                 ("priors", "slot_priors"), ("collisions", "collisions")):
                 setattr(b, field, getattr(self, name).data_ptr())
             self.batch = b
+        self.gumbel = bool(gumbel)
+        if self.gumbel:
+            for refused, what in ((reuse_tree, "reuse_tree=True"), (root_noise, "root_noise=True"),
+                                  (self.leaves > 1, "leaves_per_game > 1")):
+                if refused:
+                    raise ValueError(f"gumbel=True does not combine with {what}")
+            # fixed addresses: a captured CUDA graph of simulate() reads the keys and writes root_value in place
+            self.gumbel_keys = torch.zeros(n, dtype=torch.int64, device=dev)
+            self.root_value = torch.zeros(n, dtype=torch.float64, device=dev)
+            gd = GumbelDesc()
+            gd.seed = int(gumbel_seed) & (2**64 - 1)
+            gd.keys, gd.root_value = self.gumbel_keys.data_ptr(), self.root_value.data_ptr()
+            gd.max_considered, gd.n_sims = int(gumbel_considered), max(0, sims - 1)
+            gd.scale, gd.c_visit, gd.c_scale = float(gumbel_scale), GUMBEL_C_VISIT, GUMBEL_C_SCALE
+            self.gumbel_desc = gd
+            self._gumbel_searches = 0
         self.root_noise = bool(root_noise)
         if self.root_noise:
             missing = [key for key in ("dirichlet_alpha", "dirichlet_epsilon") if key not in args]
@@ -188,7 +215,11 @@ class BatchedMCTS:
         # the planes tensor is resident and only read by the network between selects: after the first full encode
         # through this instance's handle it is updated in place (FPC_FLAG_INCREMENTAL)
         with torch.cuda.device(self.device):
-            if self.batch is None:
+            if self.gumbel:
+                check(self.L.fpc_tree_select_gumbel(C.byref(self.desc), C.byref(self.gumbel_desc), int(self.batch_rotation),
+                                                    self.planes.data_ptr(), _lib.FLAG_INCREMENTAL, self._track,
+                                                    self._stream()))
+            elif self.batch is None:
                 check(self.L.fpc_tree_select(C.byref(self.desc), int(self.batch_rotation), self.planes.data_ptr(),
                                              _lib.FLAG_INCREMENTAL, self._track, self._stream()))
             else:
@@ -211,6 +242,20 @@ class BatchedMCTS:
             check(self.L.fpc_tree_root_noise(C.byref(self.desc), self.noise_seed, keys.data_ptr(), self.noise_alpha,
                                              self.noise_eps, self.noise_done.data_ptr(), self._stream()))
         self._noise_keys = keys  # keep alive until the kernel has run
+
+    def gumbel_result(self):
+        """(action [n] i32, policy [n, FPC_MAX_MOVES] f32) of the current search (`fpc_tree_gumbel_result`): the flat
+        action of the root child the halving leaves standing, and the improved policy softmax(logits + sigma(completed
+        Q)) with its columns aligned with root_children().  A root without children gets action -1 and a zero row; a
+        dropped game's result comes from the visits it has."""
+        if not self.gumbel:
+            raise _lib.FpcError("gumbel_result() needs BatchedMCTS(..., gumbel=True)")
+        action = torch.empty(self.n, dtype=torch.int32, device=self.device)
+        policy = torch.empty((self.n, FPC_MAX_MOVES), dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.L.fpc_tree_gumbel_result(C.byref(self.desc), C.byref(self.gumbel_desc), action.data_ptr(),
+                                                policy.data_ptr(), self._stream()))
+        return action, policy
 
     def close(self) -> None:
         if getattr(self, "_track", None):
@@ -247,7 +292,7 @@ class BatchedMCTS:
 
     @torch.no_grad()
     def search(self, root_boards: torch.Tensor | None = None, record=None, check: bool = True,
-               noise_keys=None) -> "BatchedMCTS":
+               noise_keys=None, gumbel_keys=None) -> "BatchedMCTS":
         """num_searches simulations from fresh roots at root_boards, or, with root_boards=None, on top of the current
         trees (after advance(), or to add simulations to a finished search).
         record: optional callable(sim, logits, value) called after every network forward (eager mode only), e.g.
@@ -257,7 +302,11 @@ class BatchedMCTS:
         noise_keys: with root_noise=True, the [n] i64 keys of this search's root noise (default arange(n) + n * s for
         this instance's s-th search).  add_root_noise runs before the first batch (roots that already have children:
         a kept subtree) and right after it (roots the first batch expanded), outside the CUDA graph; a root noised since
-        the last reset / advance is not noised again."""
+        the last reset / advance is not noised again.
+        gumbel_keys: with gumbel=True, the [n] i64 keys of this search's Gumbel draws, copied into `self.gumbel_keys`
+        (default arange(n) + n * s for this instance's s-th search)."""
+        if self.gumbel and root_boards is None:
+            raise _lib.FpcError("search(None) with gumbel=True: a finished halving schedule cannot be continued")
         if root_boards is not None:
             self.reset(root_boards)
         elif not self._has_tree:
@@ -266,6 +315,11 @@ class BatchedMCTS:
         if sims % self.leaves:
             raise ValueError(f"leaves_per_game={self.leaves} does not divide num_searches={sims}")
         sims //= self.leaves  # network batches
+        if self.gumbel:
+            if gumbel_keys is None:
+                gumbel_keys = torch.arange(self.n, dtype=torch.int64, device=self.device) + self.n * self._gumbel_searches
+            self._gumbel_searches += 1
+            self.gumbel_keys.copy_(torch.as_tensor(gumbel_keys, dtype=torch.int64).reshape(self.n))
         keys = None
         if self.root_noise:
             keys = noise_keys

@@ -25,7 +25,8 @@ from .mcts import BatchedMCTS
 class SelfPlay:
     def __init__(self, R: int, n_games: int, neural_net, args: dict, start_record, device="cuda",
                  batch_rotation: bool = False, reuse_tree: bool = False, leaves_per_game: int = 1,
-                 virtual_loss: int = 1, root_noise: bool = False, noise_seed: int = 0):
+                 virtual_loss: int = 1, root_noise: bool = False, noise_seed: int = 0, gumbel: bool = False,
+                 gumbel_seed: int = 0, gumbel_considered: int = 16, gumbel_scale: float = 1.0):
         """args: the reference's dict (`alphazero.py:291-306`); uses C, num_searches, temperature,
         max_game_length, heuristic_weight.  reuse_tree=True keeps the played move's subtree for the next move's search
         (`BatchedMCTS.advance`) where the reference starts every move from a fresh root: num_searches simulations are
@@ -34,7 +35,10 @@ class SelfPlay:
         network batches of n_games * L leaf slots per move.  root_noise / noise_seed: Dirichlet noise on every move's
         root priors (BatchedMCTS; args then needs dirichlet_alpha and dirichlet_epsilon), keyed by g * max_game_length + t
         for game g at ply t, so the noise of a game does not depend on the batch it plays in; play() with the same
-        noise_seed draws the same noise again."""
+        noise_seed draws the same noise again.  gumbel / gumbel_seed / gumbel_considered / gumbel_scale: Gumbel root
+        search (BatchedMCTS), keyed like the noise by g * max_game_length + t; every move plays the action of
+        `gumbel_result` (temperature is then unused) and the replay's policy targets are its improved policy, kept in
+        `hist_policy` and returned as replay["child_policy"]."""
         self.geom = GEOMETRIES[R]
         self.R, self.n, self.args = R, int(n_games), args
         self.device = torch.device(device)
@@ -42,7 +46,8 @@ class SelfPlay:
         self.reuse_tree = bool(reuse_tree)
         self.mcts = BatchedMCTS(R, self.n, neural_net, args, device=self.device, batch_rotation=batch_rotation,
                                 reuse_tree=self.reuse_tree, leaves_per_game=leaves_per_game,
-                                virtual_loss=virtual_loss, root_noise=root_noise, noise_seed=noise_seed)
+                                virtual_loss=virtual_loss, root_noise=root_noise, noise_seed=noise_seed, gumbel=gumbel,
+                                gumbel_seed=gumbel_seed, gumbel_considered=gumbel_considered, gumbel_scale=gumbel_scale)
         self.start = torch.as_tensor(start_record, dtype=torch.uint8)
         T = int(args["max_game_length"])
         i32 = dict(dtype=torch.int32, device=self.device)
@@ -51,6 +56,8 @@ class SelfPlay:
         self.hist_visits = torch.zeros((T, self.n, FPC_MAX_MOVES), **i32)
         self.hist_valid = torch.zeros((T, self.n), dtype=torch.bool, device=self.device)
         self.hist_action = torch.full((T, self.n), -1, **i32)
+        if self.mcts.gumbel:
+            self.hist_policy = torch.zeros((T, self.n, FPC_MAX_MOVES), dtype=torch.float32, device=self.device)
 
     # ---- one move for every running game -----------------------------------------------------------
     def sample_actions(self, flat: torch.Tensor, visits: torch.Tensor, running: torch.Tensor) -> torch.Tensor:
@@ -85,6 +92,8 @@ class SelfPlay:
             else:
                 self.mcts.reset(self.env.boards)
             self.mcts.dropped.copy_((~running).int())  # finished games take no part in the search
+            if self.mcts.gumbel:
+                self.mcts.gumbel_keys.copy_(torch.arange(n, dtype=torch.int64, device=self.device) * T + t)
             keys = None
             if self.mcts.root_noise:
                 keys = torch.arange(n, dtype=torch.int64, device=self.device) * T + t
@@ -99,7 +108,12 @@ class SelfPlay:
             self.hist_boards[t].copy_(self.env.boards)
             self.hist_flat[t].copy_(flat)
             self.hist_visits[t].copy_(visits)
-            actions = self.sample_actions(flat, visits, running)
+            if self.mcts.gumbel:
+                actions, policy = self.mcts.gumbel_result()
+                self.hist_policy[t].copy_(policy)
+                actions = torch.where(running, actions, torch.full_like(actions, -1))
+            else:
+                actions = self.sample_actions(flat, visits, running)
             moved = running & (actions >= 0)
             self.hist_valid[t].copy_(moved)
             self.hist_action[t].copy_(actions)
@@ -126,6 +140,7 @@ class SelfPlay:
         cut = torch.where(entry_team == curr_team[None, :], heur[None, :], -heur[None, :])
         value = torch.where(running[None, :], cut, win)
         sel = self.hist_valid
+        extra = {"child_policy": self.hist_policy[sel]} if self.mcts.gumbel else {}  # [M, FPC_MAX_MOVES] improved policy
         return {
             "boards": self.hist_boards[sel],        # [M, record] the replay states
             "child_flat": self.hist_flat[sel],      # [M, FPC_MAX_MOVES] flat action indices of the root's children
@@ -133,13 +148,16 @@ class SelfPlay:
             "value": value[sel],                    # [M]
             "finished": ~running,
             "losing_team": losing_team,
+            **extra,
         }
 
     def policy_targets(self, replay: dict) -> torch.Tensor:
-        """Dense [M, A*R*R] action-probability targets (`alphazero.py:104-110`)."""
+        """Dense [M, A*R*R] action-probability targets: the normalised visit counts (`alphazero.py:104-110`), or the
+        Gumbel search's improved policy when the replay has child_policy."""
         m = replay["child_flat"].shape[0]
+        weights = replay["child_policy"] if "child_policy" in replay else replay["child_visits"].float()
         probs = torch.zeros((m, self.geom.action_space_size), dtype=torch.float32, device=self.device)
-        probs.scatter_add_(1, replay["child_flat"].long(), replay["child_visits"].float())
+        probs.scatter_add_(1, replay["child_flat"].long(), weights)
         return probs / probs.sum(dim=1, keepdim=True).clamp_min(1e-30)
 
     def encoded_states(self, replay: dict) -> torch.Tensor:

@@ -20,28 +20,37 @@ from .geometry import GEOMETRIES
 class ReplayStore:
     """Ring buffer of replay entries as device tensors (`src/py/replay_buffer.py:4-20` keeps Python tuples)."""
 
-    def __init__(self, capacity: int, record_bytes: int, max_children: int, device):
+    def __init__(self, capacity: int, record_bytes: int, max_children: int, device, child_policy: bool = False):
+        """child_policy=True also keeps an f32 policy target per child (the Gumbel search's improved policy)."""
         self.capacity, self.size, self.head = int(capacity), 0, 0
         self.boards = torch.zeros((self.capacity, record_bytes), dtype=torch.uint8, device=device)
         self.child_flat = torch.zeros((self.capacity, max_children), dtype=torch.int32, device=device)
         self.child_visits = torch.zeros((self.capacity, max_children), dtype=torch.int32, device=device)
         self.value = torch.zeros(self.capacity, dtype=torch.float32, device=device)
+        self.child_policy = (torch.zeros((self.capacity, max_children), dtype=torch.float32, device=device)
+                             if child_policy else None)
 
-    def add(self, boards, child_flat, child_visits, value) -> None:
+    def add(self, boards, child_flat, child_visits, value, child_policy=None) -> None:
         m = boards.shape[0]
         if m == 0:
             return
         if m >= self.capacity:
             boards, child_flat, child_visits, value = (t[-self.capacity:] for t in (boards, child_flat, child_visits, value))
+            child_policy = child_policy[-self.capacity:] if child_policy is not None else None
             m = self.capacity
         idx = (self.head + torch.arange(m, device=self.boards.device)) % self.capacity
         self.boards[idx], self.child_flat[idx], self.child_visits[idx], self.value[idx] = boards, child_flat, child_visits, value
+        if self.child_policy is not None:
+            self.child_policy[idx] = child_policy
         self.head = (self.head + m) % self.capacity
         self.size = min(self.capacity, self.size + m)
 
     def sample(self, batch: int):
+        """(boards, child_flat, child_visits, value) of `batch` entries drawn with replacement, and child_policy after
+        them when the store keeps it."""
         idx = torch.randint(0, self.size, (batch,), device=self.boards.device)
-        return self.boards[idx], self.child_flat[idx], self.child_visits[idx], self.value[idx]
+        out = (self.boards[idx], self.child_flat[idx], self.child_visits[idx], self.value[idx])
+        return out if self.child_policy is None else out + (self.child_policy[idx],)
 
     def __len__(self) -> int:
         return self.size
@@ -57,8 +66,11 @@ class Learner:
         g = selfplay.geom
         dev = selfplay.device
         self.geom = GEOMETRIES[g.R]
-        self.train_buf = ReplayStore(args["replay_buffer_capacity"], g.record_bytes, selfplay.hist_flat.shape[-1], dev)
-        self.valid_buf = ReplayStore(args["validation_buffer_capacity"], g.record_bytes, selfplay.hist_flat.shape[-1], dev)
+        # a self-play that records an improved policy (Gumbel search) trains on it: the stores keep it beside the visits
+        pol = hasattr(selfplay, "hist_policy")
+        self.train_buf = ReplayStore(args["replay_buffer_capacity"], g.record_bytes, selfplay.hist_flat.shape[-1], dev, pol)
+        self.valid_buf = ReplayStore(args["validation_buffer_capacity"], g.record_bytes, selfplay.hist_flat.shape[-1], dev,
+                                     pol)
         self.ddp = None
         if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
             ids = [dev.index] if dev.type == "cuda" else None
@@ -71,11 +83,14 @@ class Learner:
         cap_t, cap_v = self.args["replay_buffer_capacity"], self.args["validation_buffer_capacity"]
         to_train = torch.rand(m, device=replay["boards"].device) < cap_t / (cap_t + cap_v)
         for buf, sel in ((self.train_buf, to_train), (self.valid_buf, ~to_train)):
-            buf.add(replay["boards"][sel], replay["child_flat"][sel], replay["child_visits"][sel], replay["value"][sel])
+            policy = replay["child_policy"][sel] if buf.child_policy is not None else None
+            buf.add(replay["boards"][sel], replay["child_flat"][sel], replay["child_visits"][sel], replay["value"][sel], policy)
 
     def _batch(self, buf: ReplayStore):
-        boards, flat, visits, value = buf.sample(int(self.args["batch_size"]))
+        boards, flat, visits, value, *policy = buf.sample(int(self.args["batch_size"]))
         fake = {"boards": boards, "child_flat": flat, "child_visits": visits}
+        if policy:
+            fake["child_policy"] = policy[0]
         return self.sp.encoded_states(fake), self.sp.policy_targets(fake), value
 
     def _loss(self, net, planes, policy_t, value_t):

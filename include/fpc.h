@@ -370,6 +370,60 @@ int fpc_tree_expand_backup_leaves(const fpc_tree *t, const fpc_leaf_batch *b, co
 int fpc_tree_root_noise(const fpc_tree *t, uint64_t seed, const int64_t *d_keys, float alpha, float epsilon,
                         int32_t *d_done, void *stream);
 
+/* ---- Gumbel root search: sequential halving and an improved policy ---------------------------------------------------
+ *
+ * Gumbel AlphaZero's root (Danihelka et al., "Policy improvement by planning with Gumbel", ICLR 2022; mctx's
+ * gumbel_muzero_policy), outside the reference.  Only the root's step changes: below it the descent is Node::SelectChild
+ * exactly as in fpc_tree_select.  For game g with k = n_children[0] > 0 children c_i = first_child[0] + i, i = 0 .. k-1
+ * (slab order), all in f64:
+ *   N_i = visits[c_i] - 1 (children are created with visit_count 1), s = sum N_i, Nmax = max N_i;
+ *   q_i = value_sum[c_i] / N_i for N_i > 0 (the frame SelectChild maximises at the root);
+ *   v = -(s == 0 ? value_sum[0] : root_value[g]): the root's network value in the frame of q_i;
+ *   l_i = log p_i - max_j log p_j with p_i = (double)prior[c_i];
+ *   g_i = scale * (-log(-log U_i)), U_i = ((double)(mix64(seed, (uint64_t)keys[g], (uint64_t)i << 32 | 2^31) >> 11)
+ *         + 0.5) * 2^-53 (the root noise's uniform U(i, j) at j = 2^31, a stream disjoint from its j <= 192);
+ *   completed Q (mctx's qtransform_completed_by_mix_value): w_i = max(p_i, 2^-126);
+ *         W = (sum_{N_i>0} w_i*q_i) / (sum_{N_i>0} w_i), 0 when no child is visited;
+ *         v_mix = (v + s*W) / (1 + s);  cq_i = N_i > 0 ? q_i : v_mix;
+ *         r_i = (cq_i - min cq) / max(max cq - min cq, 1e-8);  sigma_i = ((c_visit + Nmax) * c_scale) * r_i;
+ *   z_i = l_i + sigma_i;  score_i = max(-1e9, g_i + z_i);
+ *   cv(s) = mctx's get_sequence_of_considered_visits(m', n_sims)[s], m' = min(max_considered, k), extended past n_sims:
+ *         m' <= 1: s.  Else L2 = ceil(log2 m'), c = m', v = 0; loop: e = max(1, n_sims / (L2*c)) (integer division);
+ *         s < e*c: cv = v + s / c; else s -= e*c, v += e, c = max(2, c / 2).
+ * Every sum, min and max above runs in one order: child i on lane i % 32, each lane over its children in ascending i,
+ * then the 32 lane results combined by the xor butterfly over offsets 16, 8, 4, 2, 1 (x = x + x[lane ^ o]).  No
+ * product is fused into a sum.
+ *
+ * fpc_tree_select_gumbel: fpc_tree_select with this root step.  A game that is dropped gets leaf -1; one whose root is
+ * not expanded is selected exactly as fpc_tree_select selects it.  Otherwise, when s == 0, root_value[g] =
+ * value_sum[0] (a fresh root holds exactly its network value once its expansion has backed it up); the root's child is
+ * c_i for the i maximising score_i over {i : N_i == cv(s)}, the first maximum in ascending i winning, and the descent
+ * continues from it with Node::SelectChild, then materialises, observes and encodes the leaf as fpc_tree_select does.
+ * While every root visit followed the schedule that set is never empty; if it is, error bit 2 is set and the game
+ * dropped, as for a failed SelectChild.  The reference's terminal rule is unchanged: a terminal leaf drops the root for
+ * the rest of the search.  Continuing a search past its n_sims follows the extended schedule (c = 2 from then on).
+ *
+ * fpc_tree_gumbel_result: for every game (dropped ones too: the result comes from the visits they have), with cv = Nmax
+ * and the same score, d_action[g] = move_flat of the best child, and d_policy[g][i] = (float)(e_i / E) with
+ * e_i = exp(z_i - max_j z_j), E = sum e_i (the order above), 0 for i >= k: softmax(l + sigma), the improved policy.  A
+ * game with k == 0 gets action -1 and a zero row.  Nothing else is written.
+ *
+ * max_considered outside 1 .. FPC_MAX_MOVES, n_sims < 0, scale / c_visit / c_scale negative or not finite, null keys /
+ * root_value / d_action / d_policy and a bad tree are FPC_ERR_ARG, before any launch.  keys [n_games] i64, root_value
+ * [n_games] f64, d_action [n_games] i32, d_policy [n_games][FPC_MAX_MOVES] f32. */
+typedef struct fpc_gumbel {
+  uint64_t seed;
+  const int64_t *keys;     /* per-game keys of the draws: a game's g_i depend only on (seed, key, i) */
+  int32_t max_considered;  /* m, the candidates of the first halving phase */
+  int32_t n_sims;          /* simulations the schedule is planned for */
+  double scale;            /* Gumbel scale; 0 = a deterministic search */
+  double c_visit, c_scale; /* sigma's constants (the paper's 50 and 0.1) */
+  double *root_value;      /* [n_games] the root's value_sum when s was 0, written by the select */
+} fpc_gumbel;
+int fpc_tree_select_gumbel(const fpc_tree *t, const fpc_gumbel *gb, int batch_rotation, float *d_planes, int flags,
+                           fpc_dense_track *track, void *stream);
+int fpc_tree_gumbel_result(const fpc_tree *t, const fpc_gumbel *gb, int32_t *d_action, float *d_policy, void *stream);
+
 /* ---- host-buffer operations (per-object calls of the binding; e2e measurement) ------------- */
 
 typedef struct fpc_ctx fpc_ctx;
