@@ -8,6 +8,7 @@
 #include <cfloat>
 #include <cmath>
 #include <string>
+#include <type_traits>
 
 #include "../../include/fpc.h"
 #include "fpc_device.cuh"
@@ -252,12 +253,17 @@ __global__ void __launch_bounds__(ADV_THREADS) tree_advance_kernel(const fpc_tre
   }
 }
 
+// descend's default step below the root: Node::SelectChild.
+struct SelectChild {};
+
 // Node::ChooseLeaf's descent (node.cpp:21-26) + Node::SelectChild (node.cpp:49-78), then the leaf's board materialised
 // into leaf_boards.  One warp of game g; `b` is the warp's 256-byte record scratch in shared memory.  root_step(node, nc,
 // fc, nv) may replace the root's step: it receives the root (node 0) and its (n_children, first_child, visits), may move
-// them to the node the descent continues from, and returns false when it has dropped the game.
-template <class G, class RootStep>
-__device__ __forceinline__ void descend(const fpc_tree &T, int g, int lane, uint8_t *b, RootStep root_step) {
+// them to the node the descent continues from, and returns false when it has dropped the game.  step(node, nc, fc, nv)
+// may replace every later step in the same way, at a node with nc > 0 children; the default is SelectChild, spelled out
+// in the loop below.
+template <class G, class RootStep, class Step = SelectChild>
+__device__ __forceinline__ void descend(const fpc_tree &T, int g, int lane, uint8_t *b, RootStep root_step, Step step = {}) {
   const size_t slab = (size_t)g * T.node_cap;
   const int32_t *visits = T.visits + slab, *first_child = T.first_child + slab, *n_children = T.n_children + slab;
   const double *value_sum = T.value_sum + slab;
@@ -268,6 +274,10 @@ __device__ __forceinline__ void descend(const fpc_tree &T, int g, int lane, uint
   int nc = n_children[0], fc = first_child[0], nv = visits[0];
   if (!root_step(node, nc, fc, nv)) return;
   while (nc > 0) {
+    if constexpr (!std::is_same_v<Step, SelectChild>) {
+      if (!step(node, nc, fc, nv)) return;
+      continue;
+    }
     const double lg = log(sqrt((double)nv));
     double best = -CUDART_INF;
     int best_i = 0x7fffffff, b_nc = 0, b_fc = 0, b_nv = 0;
@@ -1089,10 +1099,26 @@ __device__ __forceinline__ int considered_visits(int s, int m, int n_sims) {
   return v + s / 2;
 }
 
-// Game g's k > 0 root children (the first at fc): n = N_i and z = l_i + sigma_i in this lane's registers, nmax = max N_i;
-// returns s = sum N_i.  The select (write_root_value) records the root's value_sum as root_value when s == 0.
+// The root's network value u: value_sum[0] when s == 0, else root_value[g]; the select (write) records it as
+// root_value when s == 0.
+struct RootValue {
+  const fpc_tree &T;
+  const fpc_gumbel &B;
+  int g, lane;
+  bool write;
+  __device__ __forceinline__ double operator()(int s, size_t slab) const {
+    const double root = s == 0 ? T.value_sum[slab] : B.root_value[g];
+    if (write && s == 0 && lane == 0) B.root_value[g] = root;
+    return root;
+  }
+};
+
+// Game g's node with k > 0 children (the first at fc): n = N_i and z = l_i + sigma_i in this lane's registers,
+// nmax = max N_i; returns s = sum N_i.  value(s, slab) is the node's network value u (v = -u), which the caller reads,
+// and caches when s == 0: RootValue at the root, node_value below it.
+template <class Value>
 __device__ __forceinline__ int gumbel_logits(const fpc_tree &T, const fpc_gumbel &B, int g, int lane, int fc, int k,
-                                             bool write_root_value, int (&n)[GB_PER], double (&z)[GB_PER], int &nmax) {
+                                             Value value, int (&n)[GB_PER], double (&z)[GB_PER], int &nmax) {
   const size_t slab = (size_t)g * T.node_cap;
   double q[GB_PER];
   int s = 0;
@@ -1125,8 +1151,7 @@ __device__ __forceinline__ int gumbel_logits(const fpc_tree &T, const fpc_gumbel
     wq = __dadd_rn(wq, __shfl_xor_sync(FULL, wq, o));
     ws = __dadd_rn(ws, __shfl_xor_sync(FULL, ws, o));
   }
-  const double root = s == 0 ? T.value_sum[slab] : B.root_value[g];
-  if (write_root_value && s == 0 && lane == 0) B.root_value[g] = root;
+  const double root = value(s, slab);
   const double w_mean = ws > 0.0 ? wq / ws : 0.0;
   const double v_mix = __dadd_rn(-root, __dmul_rn((double)s, w_mean)) / (1.0 + (double)s);
   double lo = CUDART_INF, hi = -CUDART_INF;
@@ -1185,6 +1210,46 @@ __device__ __forceinline__ int gumbel_argmax(const fpc_gumbel &B, uint64_t key, 
   return best_i == 0x7fffffff ? -1 : best_i;
 }
 
+// The Gumbel root step (descend's root_step): the root's child by sequential halving.
+__device__ __forceinline__ bool gumbel_root_step(const fpc_tree &T, const fpc_gumbel &B, int g, int lane, int &node,
+                                                 int &nc, int &fc, int &nv) {
+  if (nc <= 0) return true;  // an unexpanded root is the leaf, as in fpc_tree_select
+  int n[GB_PER], nmax;
+  double z[GB_PER];
+  const int s = gumbel_logits(T, B, g, lane, fc, nc, RootValue{T, B, g, lane, true}, n, z, nmax);
+  const int i = gumbel_argmax(B, (uint64_t)B.keys[g], lane, nc, considered_visits(s, min(B.max_considered, nc), B.n_sims), n, z);
+  if (i < 0) {  // a root visit left the schedule: drop the game as a failed SelectChild does
+    if (lane == 0) {
+      T.error[g] |= ERR_NO_CHILD;
+      T.leaf[g] = -1;
+      T.dropped[g] = 1;
+    }
+    return false;
+  }
+  const size_t slab = (size_t)g * T.node_cap;
+  node = fc + i;
+  nc = T.n_children[slab + node], fc = T.first_child[slab + node], nv = T.visits[slab + node];
+  return true;
+}
+
+// e_i = exp(z_i - max_j z_j) in place of z (0 for i >= k); returns E = sum e_i, both in the stated order.
+__device__ __forceinline__ double softmax_terms(int lane, int k, double (&z)[GB_PER]) {
+  double zmax = -CUDART_INF, sum = 0.0;
+#pragma unroll
+  for (int r = 0; r < GB_PER; ++r)
+    if (lane + 32 * r < k) zmax = fmax(zmax, z[r]);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) zmax = fmax(zmax, __shfl_xor_sync(FULL, zmax, o));
+#pragma unroll
+  for (int r = 0; r < GB_PER; ++r) {
+    z[r] = lane + 32 * r < k ? exp(z[r] - zmax) : 0.0;
+    sum = __dadd_rn(sum, z[r]);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) sum = __dadd_rn(sum, __shfl_xor_sync(FULL, sum, o));
+  return sum;
+}
+
 // fpc_tree_select with the Gumbel root step: the root's child by sequential halving, then Node::SelectChild below it.
 template <class G>
 __global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_gumbel_kernel(const fpc_tree T, const fpc_gumbel B) {
@@ -1196,25 +1261,77 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_gumbel_kernel(con
     if (lane == 0) T.leaf[g] = -1;
     return;
   }
-  descend<G>(T, g, lane, recs[wib], [&](int &node, int &nc, int &fc, int &nv) {
-    if (nc <= 0) return true;  // an unexpanded root is the leaf, as in fpc_tree_select
-    int n[GB_PER], nmax;
-    double z[GB_PER];
-    const int s = gumbel_logits(T, B, g, lane, fc, nc, true, n, z, nmax);
-    const int i = gumbel_argmax(B, (uint64_t)B.keys[g], lane, nc, considered_visits(s, min(B.max_considered, nc), B.n_sims), n, z);
-    if (i < 0) {  // a root visit left the schedule: drop the game as a failed SelectChild does
-      if (lane == 0) {
-        T.error[g] |= ERR_NO_CHILD;
-        T.leaf[g] = -1;
-        T.dropped[g] = 1;
-      }
-      return false;
-    }
-    const size_t slab = (size_t)g * T.node_cap;
-    node = fc + i;
-    nc = T.n_children[slab + node], fc = T.first_child[slab + node], nv = T.visits[slab + node];
-    return true;
-  });
+  descend<G>(T, g, lane, recs[wib],
+             [&](int &node, int &nc, int &fc, int &nv) { return gumbel_root_step(T, B, g, lane, node, nc, fc, nv); });
+}
+
+// fpc_tree_select with the Gumbel root step and Gumbel MuZero's interior step below it: at node x the child maximising
+// pi'_i - N_i / (1 + s), pi' = softmax(l + sigma(completed Q)) with x's own network value, cached in node_value[x] the
+// first time the descent passes x (s == 0).  x's value_sum and node_value are requested in the children's memory
+// round; the winner's child range is loaded after the arg-max.
+template <class G>
+__global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_gumbel_interior_kernel(const fpc_tree T, const fpc_gumbel B,
+                                                                                       double *node_value) {
+  __shared__ alignas(16) uint8_t recs[SEL_WARPS][256];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int g = blockIdx.x * SEL_WARPS + wib;
+  if (g >= T.n_games) return;
+  if (T.dropped[g]) {
+    if (lane == 0) T.leaf[g] = -1;
+    return;
+  }
+  const size_t slab = (size_t)g * T.node_cap;
+  double *cache = node_value + slab;
+  descend<G>(
+      T, g, lane, recs[wib],
+      [&](int &node, int &nc, int &fc, int &nv) { return gumbel_root_step(T, B, g, lane, node, nc, fc, nv); },
+      [&](int &node, int &nc, int &fc, int &) {  // nv (SelectChild's parent count) is not used below the root
+        const int x = node;
+        const double own = T.value_sum[slab + x], cached = cache[x];  // requested with the children's statistics
+        int n[GB_PER], nmax;
+        double z[GB_PER];
+        const int s = gumbel_logits(T, B, g, lane, fc, nc,
+                                    [&](int s, size_t) {
+                                      if (s == 0 && lane == 0) cache[x] = own;
+                                      return s == 0 ? own : cached;
+                                    },
+                                    n, z, nmax);
+        const double E = softmax_terms(lane, nc, z);
+        const double d = 1.0 + (double)s;
+        double best = -CUDART_INF;
+        int best_i = 0x7fffffff;
+#pragma unroll
+        for (int r = 0; r < GB_PER; ++r) {
+          const int i = lane + 32 * r;
+          if (i < nc) {
+            const double score = __dsub_rn(z[r] / E, (double)n[r] / d);
+            if (score > best) {  // strict: the first maximum wins
+              best = score;
+              best_i = i;
+            }
+          }
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+          const double ob = __shfl_xor_sync(FULL, best, o);
+          const int oi = __shfl_xor_sync(FULL, best_i, o);
+          if (oi != 0x7fffffff && (best_i == 0x7fffffff || ob > best || (ob == best && oi < best_i))) {
+            best = ob;
+            best_i = oi;
+          }
+        }
+        if (best_i == 0x7fffffff) {  // NaN scores
+          if (lane == 0) {
+            T.error[g] |= ERR_NO_CHILD;
+            T.leaf[g] = -1;
+            T.dropped[g] = 1;
+          }
+          return false;
+        }
+        node = fc + best_i;
+        nc = T.n_children[slab + node], fc = T.first_child[slab + node];
+        return true;
+      });
 }
 
 // The action (the considered child at cv = Nmax with the best score) and the improved policy softmax(l + sigma).
@@ -1233,21 +1350,9 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_gumbel_result_kernel(cons
   }
   int n[GB_PER], nmax;
   double z[GB_PER];
-  gumbel_logits(T, B, g, lane, fc, k, false, n, z, nmax);
+  gumbel_logits(T, B, g, lane, fc, k, RootValue{T, B, g, lane, false}, n, z, nmax);
   const int best = gumbel_argmax(B, (uint64_t)B.keys[g], lane, k, nmax, n, z);
-  double zmax = -CUDART_INF, sum = 0.0;
-#pragma unroll
-  for (int r = 0; r < GB_PER; ++r)
-    if (lane + 32 * r < k) zmax = fmax(zmax, z[r]);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) zmax = fmax(zmax, __shfl_xor_sync(FULL, zmax, o));
-#pragma unroll
-  for (int r = 0; r < GB_PER; ++r) {
-    z[r] = lane + 32 * r < k ? exp(z[r] - zmax) : 0.0;
-    sum = __dadd_rn(sum, z[r]);
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) sum = __dadd_rn(sum, __shfl_xor_sync(FULL, sum, o));
+  const double sum = softmax_terms(lane, k, z);
 #pragma unroll
   for (int r = 0; r < GB_PER; ++r) {
     const int i = lane + 32 * r;
@@ -1388,6 +1493,23 @@ int fpc_tree_select_gumbel(const fpc_tree *t, const fpc_gumbel *gb, int batch_ro
   rc = dispatch(t->R, [&](auto g) {
     tree_descend_gumbel_kernel<decltype(g)><<<blocks, SEL_WARPS * 32, 0, st>>>(*t, *gb);
     return cuda_check(cudaGetLastError(), "tree_descend_gumbel_kernel launch");
+  });
+  if (rc != FPC_OK) return rc;
+  return observe_leaves(t, batch_rotation, d_planes, flags, track, stream);
+}
+
+int fpc_tree_select_gumbel_interior(const fpc_tree *t, const fpc_gumbel *gb, double *d_node_value, int batch_rotation,
+                                    float *d_planes, int flags, fpc_dense_track *track, void *stream) {
+  int rc = check_tree(t, "fpc_tree_select_gumbel_interior");
+  if (rc == FPC_OK) rc = check_gumbel(t, gb, "fpc_tree_select_gumbel_interior");
+  if (rc != FPC_OK) return rc;
+  if (!d_node_value) return fail(FPC_ERR_ARG, "fpc_tree_select_gumbel_interior: null node_value");
+  if (t->n_games == 0) return FPC_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int blocks = (t->n_games + SEL_WARPS - 1) / SEL_WARPS;
+  rc = dispatch(t->R, [&](auto g) {
+    tree_descend_gumbel_interior_kernel<decltype(g)><<<blocks, SEL_WARPS * 32, 0, st>>>(*t, *gb, d_node_value);
+    return cuda_check(cudaGetLastError(), "tree_descend_gumbel_interior_kernel launch");
   });
   if (rc != FPC_OK) return rc;
   return observe_leaves(t, batch_rotation, d_planes, flags, track, stream);

@@ -26,7 +26,8 @@ class SelfPlay:
     def __init__(self, R: int, n_games: int, neural_net, args: dict, start_record, device="cuda",
                  batch_rotation: bool = False, reuse_tree: bool = False, leaves_per_game: int = 1,
                  virtual_loss: int = 1, root_noise: bool = False, noise_seed: int = 0, gumbel: bool = False,
-                 gumbel_seed: int = 0, gumbel_considered: int = 16, gumbel_scale: float = 1.0):
+                 gumbel_seed: int = 0, gumbel_considered: int = 16, gumbel_scale: float = 1.0,
+                 gumbel_interior: bool = False):
         """args: the reference's dict (`alphazero.py:291-306`); uses C, num_searches, temperature,
         max_game_length, heuristic_weight.  reuse_tree=True keeps the played move's subtree for the next move's search
         (`BatchedMCTS.advance`) where the reference starts every move from a fresh root: num_searches simulations are
@@ -38,7 +39,8 @@ class SelfPlay:
         noise_seed draws the same noise again.  gumbel / gumbel_seed / gumbel_considered / gumbel_scale: Gumbel root
         search (BatchedMCTS), keyed like the noise by g * max_game_length + t; every move plays the action of
         `gumbel_result` (temperature is then unused) and the replay's policy targets are its improved policy, kept in
-        `hist_policy` and returned as replay["child_policy"]."""
+        `hist_policy` and returned as replay["child_policy"].  gumbel_interior: Gumbel MuZero's interior selection below
+        the Gumbel root (BatchedMCTS); keys, actions and policy targets are as with gumbel alone."""
         self.geom = GEOMETRIES[R]
         self.R, self.n, self.args = R, int(n_games), args
         self.device = torch.device(device)
@@ -47,7 +49,8 @@ class SelfPlay:
         self.mcts = BatchedMCTS(R, self.n, neural_net, args, device=self.device, batch_rotation=batch_rotation,
                                 reuse_tree=self.reuse_tree, leaves_per_game=leaves_per_game,
                                 virtual_loss=virtual_loss, root_noise=root_noise, noise_seed=noise_seed, gumbel=gumbel,
-                                gumbel_seed=gumbel_seed, gumbel_considered=gumbel_considered, gumbel_scale=gumbel_scale)
+                                gumbel_seed=gumbel_seed, gumbel_considered=gumbel_considered, gumbel_scale=gumbel_scale,
+                                gumbel_interior=gumbel_interior)
         self.start = torch.as_tensor(start_record, dtype=torch.uint8)
         T = int(args["max_game_length"])
         i32 = dict(dtype=torch.int32, device=self.device)

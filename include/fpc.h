@@ -424,6 +424,35 @@ int fpc_tree_select_gumbel(const fpc_tree *t, const fpc_gumbel *gb, int batch_ro
                            fpc_dense_track *track, void *stream);
 int fpc_tree_gumbel_result(const fpc_tree *t, const fpc_gumbel *gb, int32_t *d_action, float *d_policy, void *stream);
 
+/* ---- Gumbel MuZero interior selection: the completed-Q improved policy below the Gumbel root -------------------------
+ *
+ * The second half of Gumbel MuZero (Danihelka et al., ICLR 2022; mctx's gumbel_muzero_interior_action_selection), outside
+ * the reference.  fpc_tree_select_gumbel_interior is fpc_tree_select_gumbel with its root step unchanged (the halving
+ * schedule, the draws, root_value) and this step at every node x the descent passes below the root, with
+ * k = n_children[x] > 0 children c_i = first_child[x] + i, i = 0 .. k-1, all in f64:
+ *   N_i, s, Nmax, q_i, l_i, w_i, W, v_mix, cq_i, r_i and sigma_i exactly as the root's recipe above states them, with x
+ *         in place of the root, the same c_visit / c_scale, and
+ *   u = (s == 0 ? value_sum[x] : d_node_value[g][x]), v = -u: x's network value in the frame of q_i.  When s == 0 the
+ *         select writes d_node_value[g][x] = value_sum[x]: x gained its children in the expansion that backed its own
+ *         network value up, and no descent has passed x since, so value_sum[x] is exactly that value (the root_value
+ *         rule, applied to every node);
+ *   z_i = l_i + sigma_i;  pi'_i = e_i / E with e_i = exp(z_i - max_j z_j), E = sum e_i (fpc_tree_gumbel_result's
+ *         soft-max, in its order, before its cast to f32);
+ *   score_i = pi'_i - (double)N_i / (1 + (double)s)  (both quotients rounded, then one rounded subtraction).
+ * The child is c_i for the first maximum of score_i in ascending i: no draws and no keys below the root, the step is
+ * deterministic.  If no score compares greater than -inf (NaN inputs), error bit 2 is set and the game dropped, as for a
+ * failed SelectChild.  Sums, maxima and minima run in the root's order (lane i % 32, lanes ascending, then the xor
+ * butterfly 16 .. 1) and no product is fused into a sum.  The terminal rule, the materialisation, the observe and the
+ * encode of the leaf are fpc_tree_select's.  fpc_tree_gumbel_result serves this search unchanged: the root's statistics
+ * are the same.
+ *
+ * The caller's contract for d_node_value [n_games][node_cap] f64: every simulation since the tree's reset went through
+ * this select.  An entry is then read only after this select wrote it, so the slab needs no initialisation and
+ * fpc_tree_reset does not touch it.  Null d_node_value, every refusal of fpc_tree_select_gumbel and a bad tree are
+ * FPC_ERR_ARG, before any launch. */
+int fpc_tree_select_gumbel_interior(const fpc_tree *t, const fpc_gumbel *gb, double *d_node_value, int batch_rotation,
+                                    float *d_planes, int flags, fpc_dense_track *track, void *stream);
+
 /* ---- host-buffer operations (per-object calls of the binding; e2e measurement) ------------- */
 
 typedef struct fpc_ctx fpc_ctx;
