@@ -14,12 +14,37 @@ torch's device RNG.  The deterministic pieces (advance, rewards) are checked aga
 tests/test_gpu_selfplay.py."""
 from __future__ import annotations
 
+import functools
+
 import torch
 
 from ._lib import FPC_MAX_MOVES
 from .env import BatchedEnv
-from .geometry import GEOMETRIES
+from .geometry import GEOMETRIES, Geometry
 from .mcts import BatchedMCTS
+
+
+@functools.lru_cache(maxsize=None)
+def _network_index(R: int, device: torch.device) -> torch.Tensor:
+    """[4, A*R*R] i64: row k maps a board-frame flat action index to the entry of the network's policy row that the
+    search reads for it when the network sees the position rotated by colour k (torch.rot90(., -k) over [A, R, R], as
+    tree_expand_backup_kernel un-rotates)."""
+    g = GEOMETRIES[R]
+    idx = torch.arange(g.action_space_size, dtype=torch.int64).view(g.num_action_channels, R, R)
+    return torch.stack([torch.rot90(idx, -k, (1, 2)).reshape(-1) for k in range(4)]).to(device)
+
+
+def policy_targets(geom: Geometry, boards: torch.Tensor, child_flat: torch.Tensor, weights: torch.Tensor) -> torch.Tensor:
+    """Dense [M, A*R*R] f32 policy targets in the network's frame: row i is weights[i] normalised, with the weight of
+    child child_flat[i, j] (a board-frame flat index) placed where the search reads that move in the network's row
+    when the position is encoded rotated by its own side to move k = boards[i, off_turn] (`BatchedEnv.encode(k=-1)`,
+    `BatchedMCTS(batch_rotation=False)`).  That is torch.rot90 of the board-frame target over [A, R, R] by +k.
+    Padding columns carry weight 0; a row whose weights are all zero stays zero."""
+    k = boards[:, geom.off_turn].long()
+    dest = _network_index(geom.R, child_flat.device)[k[:, None], child_flat.long()]
+    probs = torch.zeros((child_flat.shape[0], geom.action_space_size), dtype=torch.float32, device=child_flat.device)
+    probs.scatter_add_(1, dest, weights.to(torch.float32))
+    return probs / probs.sum(dim=1, keepdim=True).clamp_min(1e-30)
 
 
 class SelfPlay:
@@ -146,8 +171,8 @@ class SelfPlay:
         extra = {"child_policy": self.hist_policy[sel]} if self.mcts.gumbel else {}  # [M, FPC_MAX_MOVES] improved policy
         return {
             "boards": self.hist_boards[sel],        # [M, record] the replay states
-            "child_flat": self.hist_flat[sel],      # [M, FPC_MAX_MOVES] flat action indices of the root's children
-            "child_visits": self.hist_visits[sel],  # [M, FPC_MAX_MOVES] their visit counts (policy target = normalised)
+            "child_flat": self.hist_flat[sel],      # [M, FPC_MAX_MOVES] board-frame flat indices of the root's children
+            "child_visits": self.hist_visits[sel],  # [M, FPC_MAX_MOVES] their visit counts (targets: policy_targets)
             "value": value[sel],                    # [M]
             "finished": ~running,
             "losing_team": losing_team,
@@ -155,17 +180,18 @@ class SelfPlay:
         }
 
     def policy_targets(self, replay: dict) -> torch.Tensor:
-        """Dense [M, A*R*R] action-probability targets: the normalised visit counts (`alphazero.py:104-110`), or the
-        Gumbel search's improved policy when the replay has child_policy."""
-        m = replay["child_flat"].shape[0]
-        weights = replay["child_policy"] if "child_policy" in replay else replay["child_visits"].float()
-        probs = torch.zeros((m, self.geom.action_space_size), dtype=torch.float32, device=self.device)
-        probs.scatter_add_(1, replay["child_flat"].long(), weights)
-        return probs / probs.sum(dim=1, keepdim=True).clamp_min(1e-30)
+        """Dense [M, A*R*R] action-probability targets in the network's frame, the frame of `encoded_states`
+        (module-level `policy_targets`): the normalised visit counts (`alphazero.py:104-110`), or the Gumbel search's
+        improved policy when the replay has child_policy.  The reference scatters the visits at the board-frame index
+        (`alphazero.py:109`) while its network sees rotated planes; here the targets follow the rotation.  A self-play
+        run with batch_rotation=True read its leaves in the colour of each batch's first state, so these own-colour
+        targets match what its search read only for Red-led batches."""
+        weights = replay["child_policy"] if "child_policy" in replay else replay["child_visits"]
+        return policy_targets(self.geom, replay["boards"], replay["child_flat"], weights)
 
     def encoded_states(self, replay: dict) -> torch.Tensor:
         """`GetEncodedState(entry.state)` for every replay entry (`alphazero.py:71-75`): each state rotated by its
-        own side to move, [M,24,R,R] f32."""
+        own side to move, [M,24,R,R] f32, the network's frame of `policy_targets`."""
         boards = replay["boards"].contiguous()
         env = BatchedEnv(self.R, boards.shape[0], device=self.device)
         env.load(boards)

@@ -7,7 +7,8 @@ expanded per mini-batch by the CUDA encoder), the optimiser step is plain PyTorc
 than one GPU each rank plays its own shard of games and gradients are averaged by
 `DistributedDataParallel` (NCCL all-reduce) -- the only bulk cross-GPU traffic of the whole system.
 The loss is the reference's: cross-entropy(policy logits, visit distribution) + MSE(value, outcome),
-Adam + StepLR(1000, 0.1)."""
+Adam + StepLR(1000, 0.1).  Planes and policy targets are both in the network's frame, each entry rotated by its own
+side to move (`SelfPlay.encoded_states`, `SelfPlay.policy_targets`), where the reference trains on board-frame targets."""
 from __future__ import annotations
 
 import torch
@@ -18,10 +19,11 @@ from .geometry import GEOMETRIES
 
 
 class ReplayStore:
-    """Ring buffer of replay entries as device tensors (`src/py/replay_buffer.py:4-20` keeps Python tuples)."""
+    """Ring buffer of replay entries as device tensors (`src/py/replay_buffer.py:4-20` keeps Python tuples): board
+    records, the root children's board-frame flat indices and visit counts, and values."""
 
     def __init__(self, capacity: int, record_bytes: int, max_children: int, device, child_policy: bool = False):
-        """child_policy=True also keeps an f32 policy target per child (the Gumbel search's improved policy)."""
+        """child_policy=True also keeps an f32 policy weight per child (the Gumbel search's improved policy)."""
         self.capacity, self.size, self.head = int(capacity), 0, 0
         self.boards = torch.zeros((self.capacity, record_bytes), dtype=torch.uint8, device=device)
         self.child_flat = torch.zeros((self.capacity, max_children), dtype=torch.int32, device=device)
@@ -87,6 +89,7 @@ class Learner:
             buf.add(replay["boards"][sel], replay["child_flat"][sel], replay["child_visits"][sel], replay["value"][sel], policy)
 
     def _batch(self, buf: ReplayStore):
+        """(planes, policy targets, values) of one drawn mini-batch; planes and targets in the network's frame."""
         boards, flat, visits, value, *policy = buf.sample(int(self.args["batch_size"]))
         fake = {"boards": boards, "child_flat": flat, "child_visits": visits}
         if policy:

@@ -20,6 +20,7 @@ from tests.gumbel_oracle import GumbelTree
 from tests.reuse_oracle import search_on
 from tests.test_gpu_mcts import assert_trees_equal, search_roots
 from tests.test_gpu_mcts_noise import same_trees
+from tests.test_gpu_puct_kernels import rot_index
 from tests.util import mixed_positions, oracle_for
 
 pytestmark = pytest.mark.gpu
@@ -145,10 +146,11 @@ def test_refused_combinations_and_arguments():
 
 
 @pytest.mark.parametrize("name,R,n,T", [("EIGHT_SIMPLE", 8, 24, 40), ("STANDARD", 14, 8, 6)])
-def test_gumbel_selfplay_replays_on_the_oracle_and_repeats(monkeypatch, name, R, n, T):
+def test_gumbel_selfplay_replays_on_the_oracle_and_targets_the_networks_frame(monkeypatch, name, R, n, T):
     """The self-play replay check of tests/test_gpu_selfplay.py (boards, legality, results, rewards, policy targets
     summing to 1) with SelfPlay(gumbel=True), run twice: the same seeds give the same games.  Every ply plays the action
-    of that ply's gumbel_result, its improved policy is the replay's policy target."""
+    of that ply's gumbel_result, its improved policy is the replay's policy target, placed in the network's frame: child
+    `flat` of a position with colour k to move at rot_index(k)[flat]."""
     made, results = [], []
 
     def factory(R_, n_, net, args, start, **kw):
@@ -181,7 +183,12 @@ def test_gumbel_selfplay_replays_on_the_oracle_and_repeats(monkeypatch, name, R,
     assert torch.allclose(pol.sum(dim=1), torch.ones(len(pol), device="cuda"), atol=1e-5)
     mask = cp > 0  # the root's children (padding columns are zero)
     assert bool(mask.any(dim=1).all())
-    assert torch.allclose(torch.gather(pol, 1, flat)[mask], cp[mask], rtol=1e-5, atol=1e-7)
+    # the targets are in the network's frame: the search reads child `flat` of a position with colour k to move at
+    # rot_index(k)[flat] of the row
+    A, ks = a.geom.num_action_channels, replay["boards"][:, a.geom.off_turn].long()
+    rot = torch.stack([torch.from_numpy(rot_index(R, A, k)) for k in range(4)]).cuda()
+    at = rot[ks[:, None], flat]
+    assert torch.allclose(torch.gather(pol, 1, at)[mask], cp[mask], rtol=1e-5, atol=1e-7)
 
 
 def test_learner_trains_on_a_gumbel_replay():
