@@ -309,7 +309,7 @@ class BatchedMCTS:
 
     @torch.no_grad()
     def search(self, root_boards: torch.Tensor | None = None, record=None, check: bool = True,
-               noise_keys=None, gumbel_keys=None) -> "BatchedMCTS":
+               noise_keys=None, gumbel_keys=None, dropped=None) -> "BatchedMCTS":
         """num_searches simulations from fresh roots at root_boards, or, with root_boards=None, on top of the current
         trees (after advance(), or to add simulations to a finished search).
         record: optional callable(sim, logits, value) called after every network forward (eager mode only), e.g.
@@ -321,13 +321,17 @@ class BatchedMCTS:
         a kept subtree) and right after it (roots the first batch expanded), outside the CUDA graph; a root noised since
         the last reset / advance is not noised again.
         gumbel_keys: with gumbel=True, the [n] i64 keys of this search's Gumbel draws, copied into `self.gumbel_keys`
-        (default arange(n) + n * s for this instance's s-th search)."""
+        (default arange(n) + n * s for this instance's s-th search).
+        dropped: optional [n] bool mask of games that sit this search out (finished games), set after the reset as a
+        caller driving select / expand_backup itself would set `self.dropped`."""
         if self.gumbel and root_boards is None:
             raise _lib.FpcError("search(None) with gumbel=True: a finished halving schedule cannot be continued")
         if root_boards is not None:
             self.reset(root_boards)
         elif not self._has_tree:
             raise _lib.FpcError("search(None) continues the current trees, but there are none: pass root_boards")
+        if dropped is not None:
+            self.dropped.copy_(torch.as_tensor(dropped).reshape(self.n))
         sims = int(self.args["num_searches"])
         if sims % self.leaves:
             raise ValueError(f"leaves_per_game={self.leaves} does not divide num_searches={sims}")

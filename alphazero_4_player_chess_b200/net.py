@@ -29,6 +29,7 @@ class PolicyValueNet(nn.Module):
     def __init__(self, R: int, blocks: int = 10, hidden: int = 128, device: str | torch.device = "cuda"):
         super().__init__()
         g = GEOMETRIES[R]
+        self.R = R
         self.device = torch.device(device)
         self.stem = _conv_bn_relu(NUM_STATE_CHANNELS, hidden)
         self.tower = nn.Sequential(*[_Residual(hidden) for _ in range(blocks)])
@@ -70,7 +71,7 @@ class InferenceNet:
         precision, NOT the reference's arithmetic: bench.py reports it beside the strict fp32 line, never instead."""
         self.dtype = torch.bfloat16 if bf16 else torch.float32
         self.module = net
-        self.device = net.device
+        self.R, self.device = getattr(net, "R", None), net.device
         self.fused = bool(fused) and self.device.type == "cuda" and self._fused_ops_work()
         self.split = bool(split_policy_linear) and not bf16 and self.device.type == "cuda"
         self.refresh()
@@ -165,7 +166,7 @@ class AutocastNet:
 
     def __init__(self, net: PolicyValueNet):
         self.net = net
-        self.device = net.device
+        self.R, self.device = getattr(net, "R", None), net.device
 
     @torch.no_grad()
     def __call__(self, planes: torch.Tensor):
