@@ -1361,6 +1361,58 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_gumbel_result_kernel(cons
   if (lane == 0) action[g] = best < 0 ? -1 : T.move_flat[slab + fc + best];
 }
 
+// ---- Keyed move sampling from the root's visit counts (fpc_tree_sample_root; the recipe is stated in include/fpc.h) --
+constexpr int SAMPLE_J = INT32_MIN + 1;  // uniform j = 2^31 + 1: disjoint from the root noise's j <= 192 and Gumbel's 2^31
+
+// One warp per game: the lanes compute the weights of children i = lane, lane + 32, ... into shared memory, then lane 0
+// runs the prefix sum in ascending i (the one order the header states) and picks the child.
+__global__ void __launch_bounds__(SEL_WARPS * 32) tree_sample_root_kernel(const fpc_tree T, uint64_t seed, const int64_t *keys,
+                                                                           double temperature, int32_t *action) {
+  __shared__ double s_w[SEL_WARPS][MAX_MOVES];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int g = blockIdx.x * SEL_WARPS + warp;
+  if (g >= T.n_games) return;
+  const size_t slab = (size_t)g * T.node_cap;
+  const int k = T.dropped[g] ? 0 : min(T.n_children[slab], MAX_MOVES);
+  if (k <= 0) {
+    if (lane == 0) action[g] = -1;
+    return;
+  }
+  const int fc = T.first_child[slab];
+  long long vsum = 0;
+  for (int i = lane; i < k; i += 32) vsum += max(T.visits[slab + fc + i], 0);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) vsum += __shfl_xor_sync(FULL, vsum, o);
+  const double V = (double)vsum, inv_t = 1.0 / temperature;
+  for (int i = lane; i < k; i += 32) {
+    const double v = (double)max(T.visits[slab + fc + i], 0);
+    s_w[warp][i] = temperature == 1.0 ? v : pow(v / V, inv_t);
+  }
+  __syncwarp();
+  if (lane != 0) return;
+  double W = 0.0;
+  int last = -1;
+  for (int i = 0; i < k; ++i) {
+    W = __dadd_rn(W, s_w[warp][i]);
+    if (s_w[warp][i] > 0.0) last = i;
+  }
+  if (!(W > 0.0)) {  // no visits, or every weight underflowed
+    action[g] = -1;
+    return;
+  }
+  const double u = __dmul_rn(noise_uniform(seed, (uint64_t)keys[g], 0, SAMPLE_J), W);
+  int pick = last;  // U*W rounded up to W: the last child with weight
+  double P = 0.0;
+  for (int i = 0; i < k; ++i) {
+    P = __dadd_rn(P, s_w[warp][i]);
+    if (P > u) {
+      pick = i;
+      break;
+    }
+  }
+  action[g] = T.move_flat[slab + fc + pick];
+}
+
 static int check_tree(const fpc_tree *t, const char *who) {
   if (!t) return fail(FPC_ERR_ARG, std::string(who) + ": null tree");
   if (!fpc_supported(t->R) || t->n_games < 0 || t->node_cap < 1 || t->board_cap < 1)
@@ -1600,6 +1652,20 @@ int fpc_tree_root_noise(const fpc_tree *t, uint64_t seed, const int64_t *d_keys,
   tree_root_noise_kernel<<<blocks, SEL_WARPS * 32, 0, (cudaStream_t)stream>>>(*t, seed, d_keys, (double)alpha,
                                                                               (double)epsilon, d_done);
   return cuda_check(cudaGetLastError(), "tree_root_noise_kernel launch");
+}
+
+int fpc_tree_sample_root(const fpc_tree *t, uint64_t seed, const int64_t *d_keys, double temperature, int32_t *d_action,
+                         void *stream) {
+  int rc = check_tree(t, "fpc_tree_sample_root");
+  if (rc != FPC_OK) return rc;
+  if (!(temperature > 0.0) || !std::isfinite(temperature))
+    return fail(FPC_ERR_ARG, "fpc_tree_sample_root: temperature must be positive and finite, got " +
+                                 std::to_string(temperature));
+  if (!d_keys || !d_action) return fail(FPC_ERR_ARG, "fpc_tree_sample_root: null keys / action");
+  if (t->n_games == 0) return FPC_OK;
+  const int blocks = (t->n_games + SEL_WARPS - 1) / SEL_WARPS;
+  tree_sample_root_kernel<<<blocks, SEL_WARPS * 32, 0, (cudaStream_t)stream>>>(*t, seed, d_keys, temperature, d_action);
+  return cuda_check(cudaGetLastError(), "tree_sample_root_kernel launch");
 }
 
 }  // extern "C"

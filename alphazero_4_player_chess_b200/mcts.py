@@ -274,6 +274,21 @@ class BatchedMCTS:
                                                 policy.data_ptr(), self._stream()))
         return action, policy
 
+    def sample_root(self, seed: int, keys, temperature: float) -> torch.Tensor:
+        """[n] i32: a move drawn from every game's root visit counts with the reference's distribution (visits / sum
+        raised to 1 / temperature, `alphazero.py:108-118`), by one counter-based uniform per (seed, keys[g])
+        (`fpc_tree_sample_root`), so that a game's move does not depend on the games it shares the batch with.  -1 for a
+        dropped game and for a root without children or visits.  A search drops a game whose descent reached a terminal
+        leaf, so a caller that wants a move for such a game sets `dropped` back first."""
+        keys = torch.as_tensor(keys, dtype=torch.int64).to(self.device).contiguous()
+        assert keys.shape == (self.n,)
+        action = torch.empty(self.n, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.L.fpc_tree_sample_root(C.byref(self.desc), int(seed) & (2**64 - 1), keys.data_ptr(),
+                                              float(temperature), action.data_ptr(), self._stream()))
+        self._sample_keys = keys  # keep alive until the kernel has run
+        return action
+
     def close(self) -> None:
         if getattr(self, "_track", None):
             self.L.fpc_dense_track_destroy(self._track)

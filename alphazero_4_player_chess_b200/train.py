@@ -59,11 +59,16 @@ class ReplayStore:
 
 
 class Learner:
-    def __init__(self, selfplay, model: torch.nn.Module, optimizer: torch.optim.Optimizer, args: dict):
+    def __init__(self, selfplay, model: torch.nn.Module, optimizer: torch.optim.Optimizer, args: dict,
+                 continuous: bool = False):
         """selfplay: a SelfPlay whose network wraps `model` for inference; args: the reference's dict
         (`alphazero.py:291-306`): batch_size, replay_buffer_capacity, validation_buffer_capacity, num_iterations,
-        num_games, num_parallel_games."""
+        num_games, num_parallel_games.  continuous=True plays each iteration's games with `SelfPlay.play_games`
+        (a slot takes the next game as soon as its own ends): num_games games for training, then num_parallel_games for
+        validation, the game ids continuing across iterations.  continuous=False plays rounds of `SelfPlay.play`, as the
+        reference does."""
         self.sp, self.model, self.opt, self.args = selfplay, model, optimizer, args
+        self.continuous = bool(continuous)
         self.sched = torch.optim.lr_scheduler.StepLR(optimizer, step_size=1000, gamma=0.1)  # alphazero.py:25-27
         g = selfplay.geom
         dev = selfplay.device
@@ -144,10 +149,13 @@ class Learner:
         out = []
         for _ in range(int(iterations if iterations is not None else self.args["num_iterations"])):
             self.model.eval()
-            for _ in range(max(1, int(self.args["num_games"]) // int(self.args["num_parallel_games"]))):
-                self.store(self.sp.play())
+            if self.continuous:
+                self.store(self.sp.play_games(int(self.args["num_games"])))
+            else:
+                for _ in range(max(1, int(self.args["num_games"]) // int(self.args["num_parallel_games"]))):
+                    self.store(self.sp.play())
             steps = self.train()
             self.model.eval()
-            self.store(self.sp.play())
+            self.store(self.sp.play_games(int(self.args["num_parallel_games"])) if self.continuous else self.sp.play())
             out.append({"train_steps": steps, "replay": len(self.train_buf), "validation": self.validate()})
         return out

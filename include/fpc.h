@@ -453,6 +453,28 @@ int fpc_tree_gumbel_result(const fpc_tree *t, const fpc_gumbel *gb, int32_t *d_a
 int fpc_tree_select_gumbel_interior(const fpc_tree *t, const fpc_gumbel *gb, double *d_node_value, int batch_rotation,
                                     float *d_planes, int flags, fpc_dense_track *track, void *stream);
 
+/* ---- Keyed move sampling from the root's visit counts ---------------------------------------------------------------
+ *
+ * The played move of the reference's self-play (alphazero.py:108-118: probs = visits / sum, probs ** (1/temperature),
+ * multinomial), drawn from a counter-based uniform so that a game's move depends only on (seed, d_keys[g]) and its own
+ * tree, never on its place in the batch.  For game g with dropped[g] == 0 and k = n_children[0] > 0, the root's children
+ * c_i = first_child[0] + i, i = 0 .. k-1 (slab order), with v_i = max(visits[c_i], 0) (the stored counts, including
+ * the 1 every child is created with) and V = sum v_i (exact, integer):
+ *   temperature == 1:  w_i = (double)v_i (the integers themselves: every sum below is exact);
+ *   otherwise:         w_i = pow((double)v_i / (double)V, 1.0 / temperature) in f64;
+ *   P_i = P_{i-1} + w_i with P_{-1} = 0, one rounded f64 addition per child in ascending i;  W = P_{k-1};
+ *   U = ((double)(mix64(seed, (uint64_t)d_keys[g], 2^31 + 1) >> 11) + 0.5) * 2^-53 (the root noise's uniform U(i, j)
+ *       at i = 0, j = SAMPLE_J = 2^31 + 1: a stream disjoint from the noise's j <= 192 and Gumbel's j = 2^31);
+ *   t = U * W (one rounded product);
+ *   d_action[g] = move_flat[c_i] for the smallest i with P_i > t; if none (t rounded up to W), the largest i with w_i > 0.
+ * A game that is dropped, whose root has no children, or whose W is not positive (no visits, or every w_i underflowed)
+ * gets d_action[g] = -1.  Nothing but d_action is written.
+ *
+ * temperature not positive and finite, null d_keys / d_action and a bad tree are FPC_ERR_ARG, before any launch.
+ * d_keys [n_games] i64, d_action [n_games] i32. */
+int fpc_tree_sample_root(const fpc_tree *t, uint64_t seed, const int64_t *d_keys, double temperature,
+                         int32_t *d_action, void *stream);
+
 /* ---- host-buffer operations (per-object calls of the binding; e2e measurement) ------------- */
 
 typedef struct fpc_ctx fpc_ctx;
