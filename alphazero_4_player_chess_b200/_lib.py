@@ -63,6 +63,8 @@ SIGNATURES = {
     "fpc_tree_select_gumbel": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp]),
     "fpc_tree_gumbel_result": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "fpc_tree_select_gumbel_interior": (_i, [_vp, _vp, _vp, _i, _vp, _i, _vp, _vp]),
+    "fpc_tree_select_gumbel_leaves": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp]),
+    "fpc_tree_gumbel_result_leaves": (_i, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "fpc_tree_sample_root": (_i, [_vp, _u64, _vp, C.c_double, _vp, _vp]),
     "fpc_ctx_create": (_vp, [_i, _i, _i]),
     "fpc_ctx_destroy": (None, [_vp]),

@@ -45,7 +45,7 @@ from .geometry import GEOMETRIES
 from .mcts import BatchedMCTS
 
 SEARCH_ARGS = ("cuda_graph", "leaves_per_game", "virtual_loss", "batch_rotation", "gumbel", "gumbel_seed",
-               "gumbel_considered", "gumbel_scale", "gumbel_interior", "node_cap")
+               "gumbel_considered", "gumbel_scale", "gumbel_interior", "gumbel_leaves", "node_cap")
 OPENING_TRIES = 16
 Z95 = 1.96
 

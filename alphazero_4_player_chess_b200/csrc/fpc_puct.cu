@@ -612,16 +612,15 @@ __global__ void __launch_bounds__(EXP_THREADS, 8) tree_expand_backup_kernel(cons
 // ---- leaf-parallel PUCT (fpc_tree_select_leaves / fpc_tree_expand_backup_leaves; semantics in include/fpc.h) -------
 constexpr int LB_PATH = 64;  // path nodes a descent keeps in shared memory for its marks; deeper ones are re-walked
 
-// One warp per game, its L descents one after the other: slot j must see the marks of slots < j.  Each level is one
-// memory round as in tree_descend_kernel, with in_flight read beside visits; after the first descent the upper levels
-// come from the cache.
-template <class G>
-__global__ void __launch_bounds__(SEL_WARPS * 32) leaves_descend_kernel(const fpc_tree T, const fpc_leaf_batch B) {
-  __shared__ alignas(16) uint8_t recs[SEL_WARPS][256];
-  __shared__ int paths[SEL_WARPS][LB_PATH];
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  const int g = blockIdx.x * SEL_WARPS + wib;
-  if (g >= T.n_games) return;
+// The L slots of game g, one after the other: slot j must see the marks of slots < j.  Each level is one memory round
+// as in tree_descend_kernel, with in_flight read beside visits; after the first descent the upper levels come from the
+// cache.  root_step(node, depth, nc, fc, nv) may replace the root's step: it receives the root (node 0, depth 0) with its
+// effective (n_children, first_child, visits), may move them to a child (recording it in path[depth]) and returns 0 or
+// the error bits that end the game.  step(node, nc, fc) may replace SelectChild at every later node with nc > 0
+// children: it returns the chosen child's index or -1.  Returns the number of slots that were filled.
+template <class G, class RootStep, class Step = SelectChild>
+__device__ __forceinline__ int leaves_select(const fpc_tree &T, const fpc_leaf_batch &B, int g, int lane, uint8_t *b, int *path,
+                                             RootStep root_step, Step step = {}) {
   const int L = B.L, VL = B.virtual_loss;
   const size_t s0 = (size_t)g * L, slab = (size_t)g * T.node_cap;
   const int32_t *visits = T.visits + slab, *first_child = T.first_child + slab, *n_children = T.n_children + slab;
@@ -629,16 +628,27 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) leaves_descend_kernel(const fp
   const float *prior = T.prior + slab;
   int32_t *in_flight = B.in_flight + slab;
   uint8_t *pool = T.boards + (size_t)g * T.board_cap * G::REC;
-  int *path = paths[wib];
-  uint8_t *b = recs[wib];
   int n_boards = T.n_boards[g], n_coll = 0, j = 0;
   bool live = !T.dropped[g];
   if (lane == 0) T.leaf[g] = -1;
   for (; live && j < L; ++j) {
-    int node = 0, depth = 0, err = 0;
+    int node = 0, depth = 0;
     int nc = n_children[0], fc = first_child[0], nv = visits[0] + VL * in_flight[0];
     if (lane == 0) path[0] = 0;
-    while (nc > 0) {
+    int err = root_step(node, depth, nc, fc, nv);
+    while (!err && nc > 0) {
+      if constexpr (!std::is_same_v<Step, SelectChild>) {
+        const int i = step(node, nc, fc);
+        if (i < 0) {
+          err = ERR_NO_CHILD;
+          break;
+        }
+        node = fc + i;
+        ++depth;
+        if (lane == 0 && depth < LB_PATH) path[depth] = node;
+        nc = n_children[node], fc = first_child[node];
+        continue;
+      }
       const double lg = log(sqrt((double)nv));
       double best = -CUDART_INF;
       int best_i = 0x7fffffff, b_nc = 0, b_fc = 0, b_nv = 0;
@@ -736,6 +746,17 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) leaves_descend_kernel(const fp
     T.n_boards[g] = n_boards;
     if (n_coll) B.collisions[g] += n_coll;
   }
+  return j;
+}
+
+template <class G>
+__global__ void __launch_bounds__(SEL_WARPS * 32) leaves_descend_kernel(const fpc_tree T, const fpc_leaf_batch B) {
+  __shared__ alignas(16) uint8_t recs[SEL_WARPS][256];
+  __shared__ int paths[SEL_WARPS][LB_PATH];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int g = blockIdx.x * SEL_WARPS + wib;
+  if (g >= T.n_games) return;
+  leaves_select<G>(T, B, g, lane, recs[wib], paths[wib], [](int &, int &, int &, int &, int &) { return 0; });
 }
 
 // tree_batch_k_kernel over the slots: k <- side to move of the first LEAF slot whose status says IN_PROGRESS
@@ -1115,13 +1136,16 @@ struct RootValue {
 
 // Game g's node with k > 0 children (the first at fc): n = N_i and z = l_i + sigma_i in this lane's registers,
 // nmax = max N_i; returns s = sum N_i.  value(s, slab) is the node's network value u (v = -u), which the caller reads,
-// and caches when s == 0: RootValue at the root, node_value below it.
+// and caches when s == 0: RootValue at the root, node_value below it.  With in_flight (a leaf batch's marks, slab of
+// game g) the statistics are the effective ones, N_i + VL*in_flight and W_i - VL*in_flight, while value() still receives
+// the committed s.
 template <class Value>
 __device__ __forceinline__ int gumbel_logits(const fpc_tree &T, const fpc_gumbel &B, int g, int lane, int fc, int k,
-                                             Value value, int (&n)[GB_PER], double (&z)[GB_PER], int &nmax) {
+                                             Value value, int (&n)[GB_PER], double (&z)[GB_PER], int &nmax,
+                                             const int32_t *in_flight = nullptr, int VL = 0) {
   const size_t slab = (size_t)g * T.node_cap;
   double q[GB_PER];
-  int s = 0;
+  int s = 0, s_committed = 0;
   nmax = INT32_MIN;
   double lmax = -CUDART_INF, wq = 0.0, ws = 0.0;
 #pragma unroll
@@ -1131,12 +1155,14 @@ __device__ __forceinline__ int gumbel_logits(const fpc_tree &T, const fpc_gumbel
     if (i < k) {
       const size_t c = slab + fc + i;
       const double p = (double)T.prior[c];
+      const int vl = in_flight ? VL * in_flight[fc + i] : 0;
       n[r] = T.visits[c] - 1;  // children are created with visit_count 1 (node.h:28)
+      if (in_flight) s_committed += n[r], n[r] += vl;
       lmax = fmax(lmax, log(p));
       s += n[r];
       nmax = max(nmax, n[r]);
       if (n[r] > 0) {
-        q[r] = T.value_sum[c] / (double)n[r];
+        q[r] = (in_flight ? T.value_sum[c] - (double)vl : T.value_sum[c]) / (double)n[r];
         const double w = fmax(p, 0x1p-126);
         wq = __dadd_rn(wq, __dmul_rn(w, q[r]));
         ws = __dadd_rn(ws, w);
@@ -1146,12 +1172,13 @@ __device__ __forceinline__ int gumbel_logits(const fpc_tree &T, const fpc_gumbel
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     s += __shfl_xor_sync(FULL, s, o);
+    if (in_flight) s_committed += __shfl_xor_sync(FULL, s_committed, o);
     nmax = max(nmax, __shfl_xor_sync(FULL, nmax, o));
     lmax = fmax(lmax, __shfl_xor_sync(FULL, lmax, o));
     wq = __dadd_rn(wq, __shfl_xor_sync(FULL, wq, o));
     ws = __dadd_rn(ws, __shfl_xor_sync(FULL, ws, o));
   }
-  const double root = value(s, slab);
+  const double root = value(in_flight ? s_committed : s, slab);
   const double w_mean = ws > 0.0 ? wq / ws : 0.0;
   const double v_mix = __dadd_rn(-root, __dmul_rn((double)s, w_mean)) / (1.0 + (double)s);
   double lo = CUDART_INF, hi = -CUDART_INF;
@@ -1250,6 +1277,49 @@ __device__ __forceinline__ double softmax_terms(int lane, int k, double (&z)[GB_
   return sum;
 }
 
+// Gumbel MuZero's interior step at node x of game g (k > 0 children, the first at fc): the index of the first maximum of
+// pi'_i - N_i / (1 + s), or -1 when no score compares greater than -inf.  x's network value is value_sum[x] when the
+// committed s is 0 (then cached in cache[x]), else cache[x]; both are requested in the children's memory round.  With
+// in_flight the statistics are a leaf batch's effective ones (gumbel_logits).
+__device__ __forceinline__ int interior_argmax(const fpc_tree &T, const fpc_gumbel &B, int g, int lane, int x, int fc, int k,
+                                               double *cache, const int32_t *in_flight = nullptr, int VL = 0) {
+  const size_t slab = (size_t)g * T.node_cap;
+  const double own = T.value_sum[slab + x], cached = cache[x];
+  int n[GB_PER], nmax;
+  double z[GB_PER];
+  const int s = gumbel_logits(T, B, g, lane, fc, k,
+                              [&](int s, size_t) {
+                                if (s == 0 && lane == 0) cache[x] = own;
+                                return s == 0 ? own : cached;
+                              },
+                              n, z, nmax, in_flight, VL);
+  const double E = softmax_terms(lane, k, z);
+  const double d = 1.0 + (double)s;
+  double best = -CUDART_INF;
+  int best_i = 0x7fffffff;
+#pragma unroll
+  for (int r = 0; r < GB_PER; ++r) {
+    const int i = lane + 32 * r;
+    if (i < k) {
+      const double score = __dsub_rn(z[r] / E, (double)n[r] / d);
+      if (score > best) {  // strict: the first maximum wins
+        best = score;
+        best_i = i;
+      }
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const double ob = __shfl_xor_sync(FULL, best, o);
+    const int oi = __shfl_xor_sync(FULL, best_i, o);
+    if (oi != 0x7fffffff && (best_i == 0x7fffffff || ob > best || (ob == best && oi < best_i))) {
+      best = ob;
+      best_i = oi;
+    }
+  }
+  return best_i == 0x7fffffff ? -1 : best_i;
+}
+
 // fpc_tree_select with the Gumbel root step: the root's child by sequential halving, then Node::SelectChild below it.
 template <class G>
 __global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_gumbel_kernel(const fpc_tree T, const fpc_gumbel B) {
@@ -1286,41 +1356,8 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_gumbel_interior_k
       T, g, lane, recs[wib],
       [&](int &node, int &nc, int &fc, int &nv) { return gumbel_root_step(T, B, g, lane, node, nc, fc, nv); },
       [&](int &node, int &nc, int &fc, int &) {  // nv (SelectChild's parent count) is not used below the root
-        const int x = node;
-        const double own = T.value_sum[slab + x], cached = cache[x];  // requested with the children's statistics
-        int n[GB_PER], nmax;
-        double z[GB_PER];
-        const int s = gumbel_logits(T, B, g, lane, fc, nc,
-                                    [&](int s, size_t) {
-                                      if (s == 0 && lane == 0) cache[x] = own;
-                                      return s == 0 ? own : cached;
-                                    },
-                                    n, z, nmax);
-        const double E = softmax_terms(lane, nc, z);
-        const double d = 1.0 + (double)s;
-        double best = -CUDART_INF;
-        int best_i = 0x7fffffff;
-#pragma unroll
-        for (int r = 0; r < GB_PER; ++r) {
-          const int i = lane + 32 * r;
-          if (i < nc) {
-            const double score = __dsub_rn(z[r] / E, (double)n[r] / d);
-            if (score > best) {  // strict: the first maximum wins
-              best = score;
-              best_i = i;
-            }
-          }
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-          const double ob = __shfl_xor_sync(FULL, best, o);
-          const int oi = __shfl_xor_sync(FULL, best_i, o);
-          if (oi != 0x7fffffff && (best_i == 0x7fffffff || ob > best || (ob == best && oi < best_i))) {
-            best = ob;
-            best_i = oi;
-          }
-        }
-        if (best_i == 0x7fffffff) {  // NaN scores
+        const int i = interior_argmax(T, B, g, lane, node, fc, nc, cache);
+        if (i < 0) {  // NaN scores
           if (lane == 0) {
             T.error[g] |= ERR_NO_CHILD;
             T.leaf[g] = -1;
@@ -1328,18 +1365,113 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_gumbel_interior_k
           }
           return false;
         }
-        node = fc + best_i;
+        node = fc + i;
         nc = T.n_children[slab + node], fc = T.first_child[slab + node];
         return true;
       });
 }
 
-// The action (the considered child at cv = Nmax with the best score) and the improved policy softmax(l + sigma).
-__global__ void __launch_bounds__(SEL_WARPS * 32) tree_gumbel_result_kernel(const fpc_tree T, const fpc_gumbel B,
-                                                                             int32_t *action, float *policy) {
-  const int lane = threadIdx.x & 31;
-  const int g = blockIdx.x * SEL_WARPS + (threadIdx.x >> 5);
+// ---- leaf-parallel Gumbel search (fpc_tree_select_gumbel_leaves / fpc_tree_gumbel_result_leaves; include/fpc.h) ----
+// One warp per game, its L slots in order through leaves_select.  The root's scores come from the committed statistics
+// once per batch (gumbel_logits and the draws: one reduction per game and batch); the schedule runs on issued[] (I_i in
+// register i / 32 of lane i % 32), so slot j's root child is the first maximum of score_i over {I_i == cv(sum I)}.  Below
+// it the descent is leaves_select's SelectChild with virtual loss, or with Interior the interior step over the effective
+// statistics.  A slot whose descent fails after its root step gives its issue back: only LEAF and COLLISION slots count.
+template <class G, bool Interior>
+__global__ void __launch_bounds__(SEL_WARPS * 32) gumbel_leaves_descend_kernel(const fpc_tree T, const fpc_gumbel Gb,
+                                                                              const fpc_leaf_batch B, int32_t *issued,
+                                                                              double *node_value) {
+  __shared__ alignas(16) uint8_t recs[SEL_WARPS][256];
+  __shared__ int paths[SEL_WARPS][LB_PATH];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int g = blockIdx.x * SEL_WARPS + wib;
   if (g >= T.n_games) return;
+  const size_t slab = (size_t)g * T.node_cap;
+  const int k = T.n_children[slab], fc0 = T.first_child[slab];
+  const bool root_open = !T.dropped[g] && k > 0;
+  int32_t *iss = issued + (size_t)g * MAX_MOVES;
+  const int32_t *in_flight = B.in_flight + slab;
+  int I[GB_PER];
+  double score[GB_PER];
+  int t = 0, mp = 0;
+  if (root_open) {
+    int n[GB_PER], nmax;
+    double z[GB_PER];
+    gumbel_logits(T, Gb, g, lane, fc0, k, RootValue{T, Gb, g, lane, true}, n, z, nmax);
+    const uint64_t key = (uint64_t)Gb.keys[g];
+#pragma unroll
+    for (int r = 0; r < GB_PER; ++r) {
+      const int i = lane + 32 * r;
+      I[r] = i < k ? iss[i] : 0;
+      t += I[r];
+      score[r] = -CUDART_INF;
+      if (i < k) {  // gumbel_argmax's score
+        const double gum = -log(-log(noise_uniform(Gb.seed, key, i, GUMBEL_J)));
+        const double x = __dadd_rn(__dmul_rn(Gb.scale, gum), z[r]);
+        score[r] = x > GUMBEL_FLOOR ? x : GUMBEL_FLOOR;
+      }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(FULL, t, o);
+    mp = min(Gb.max_considered, k);
+  }
+  int taken = 0, last = -1;
+  auto root_step = [&](int &node, int &depth, int &nc, int &fc, int &nv) -> int {
+    if (nc <= 0) return 0;  // an unexpanded root is every slot's endpoint: one LEAF, L - 1 COLLISIONs
+    const int cv = considered_visits(t, mp, Gb.n_sims);
+    double best = -CUDART_INF;
+    int best_i = 0x7fffffff;
+#pragma unroll
+    for (int r = 0; r < GB_PER; ++r) {
+      const int i = lane + 32 * r;
+      if (i < k && I[r] == cv && score[r] > best) {  // strict: the first maximum wins
+        best = score[r];
+        best_i = i;
+      }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const double ob = __shfl_xor_sync(FULL, best, o);
+      const int oi = __shfl_xor_sync(FULL, best_i, o);
+      if (oi != 0x7fffffff && (best_i == 0x7fffffff || ob > best || (ob == best && oi < best_i))) {
+        best = ob;
+        best_i = oi;
+      }
+    }
+    if (best_i == 0x7fffffff) return ERR_NO_CHILD;  // a root visit left the schedule
+#pragma unroll
+    for (int r = 0; r < GB_PER; ++r) I[r] += lane + 32 * r == best_i;
+    ++t, ++taken, last = best_i;
+    node = fc + best_i;
+    depth = 1;
+    if (lane == 0) paths[wib][1] = node;
+    nc = T.n_children[slab + node], fc = T.first_child[slab + node];
+    nv = T.visits[slab + node] + B.virtual_loss * in_flight[node];
+    return 0;
+  };
+  int filled;
+  if constexpr (Interior) {
+    double *cache = node_value + slab;
+    filled = leaves_select<G>(T, B, g, lane, recs[wib], paths[wib], root_step, [&](int node, int nc, int fc) {
+      return interior_argmax(T, Gb, g, lane, node, fc, nc, cache, in_flight, B.virtual_loss);
+    });
+  } else {
+    filled = leaves_select<G>(T, B, g, lane, recs[wib], paths[wib], root_step);
+  }
+  if (!root_open) return;
+  if (taken > filled) {  // the slot that failed below its root step is EMPTY: it issued no visit
+#pragma unroll
+    for (int r = 0; r < GB_PER; ++r) I[r] -= lane + 32 * r == last;
+  }
+#pragma unroll
+  for (int r = 0; r < GB_PER; ++r)
+    if (lane + 32 * r < k) iss[lane + 32 * r] = I[r];
+}
+
+// The action (the considered child at cv = Nmax with the best score) and the improved policy softmax(l + sigma).  With
+// issued (a leaf-parallel search's I_i) the survivors are {I_i == max I} instead.
+__device__ __forceinline__ void gumbel_result(const fpc_tree &T, const fpc_gumbel &B, int g, int lane, const int32_t *issued,
+                                              int32_t *action, float *policy) {
   const size_t slab = (size_t)g * T.node_cap;
   const int k = T.n_children[slab], fc = T.first_child[slab];
   float *row = policy + (size_t)g * MAX_MOVES;
@@ -1351,6 +1483,17 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_gumbel_result_kernel(cons
   int n[GB_PER], nmax;
   double z[GB_PER];
   gumbel_logits(T, B, g, lane, fc, k, RootValue{T, B, g, lane, false}, n, z, nmax);
+  if (issued) {
+    nmax = INT32_MIN;
+#pragma unroll
+    for (int r = 0; r < GB_PER; ++r) {
+      const int i = lane + 32 * r;
+      n[r] = i < k ? issued[(size_t)g * MAX_MOVES + i] : -1;
+      nmax = max(nmax, n[r]);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) nmax = max(nmax, __shfl_xor_sync(FULL, nmax, o));
+  }
   const int best = gumbel_argmax(B, (uint64_t)B.keys[g], lane, k, nmax, n, z);
   const double sum = softmax_terms(lane, k, z);
 #pragma unroll
@@ -1359,6 +1502,21 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_gumbel_result_kernel(cons
     if (i < MAX_MOVES) row[i] = (float)(z[r] / sum);
   }
   if (lane == 0) action[g] = best < 0 ? -1 : T.move_flat[slab + fc + best];
+}
+
+__global__ void __launch_bounds__(SEL_WARPS * 32) tree_gumbel_result_kernel(const fpc_tree T, const fpc_gumbel B,
+                                                                             int32_t *action, float *policy) {
+  const int g = blockIdx.x * SEL_WARPS + (threadIdx.x >> 5);
+  if (g >= T.n_games) return;
+  gumbel_result(T, B, g, threadIdx.x & 31, nullptr, action, policy);
+}
+
+__global__ void __launch_bounds__(SEL_WARPS * 32) tree_gumbel_result_leaves_kernel(const fpc_tree T, const fpc_gumbel B,
+                                                                                    const int32_t *issued, int32_t *action,
+                                                                                    float *policy) {
+  const int g = blockIdx.x * SEL_WARPS + (threadIdx.x >> 5);
+  if (g >= T.n_games) return;
+  gumbel_result(T, B, g, threadIdx.x & 31, issued, action, policy);
 }
 
 // ---- Keyed move sampling from the root's visit counts (fpc_tree_sample_root; the recipe is stated in include/fpc.h) --
@@ -1485,6 +1643,27 @@ static int observe_leaves(const fpc_tree *t, int batch_rotation, float *d_planes
                              d_planes, t->k, 0, nullptr, flags, stream);
 }
 
+// What fpc_tree_select_leaves does after its selection: the rules kernel on the slots and their planes, rotated by the
+// first LEAF slot in progress with batch_rotation.
+static int observe_slots(const fpc_tree *t, const fpc_leaf_batch *b, int batch_rotation, float *d_planes, int flags,
+                         fpc_dense_track *track, void *stream) {
+  const int n_slots = t->n_games * b->L;
+  if (batch_rotation) {
+    int rc = fpc_observe(t->R, b->leaf_boards, n_slots, nullptr, b->leaf_flat, b->leaf_counts, b->leaf_status, nullptr,
+                         nullptr, 0, nullptr, 0, stream);
+    if (rc != FPC_OK) return rc;
+    rc = dispatch(t->R, [&](auto g) {
+      leaves_batch_k_kernel<decltype(g)><<<1, 1024, 0, (cudaStream_t)stream>>>(*b, n_slots);
+      return cuda_check(cudaGetLastError(), "leaves_batch_k_kernel launch");
+    });
+    if (rc != FPC_OK) return rc;
+    return fpc_observe_tracked(track, t->R, b->leaf_boards, n_slots, nullptr, nullptr, nullptr, nullptr, d_planes, b->k, 0,
+                               nullptr, flags, stream);
+  }
+  return fpc_observe_tracked(track, t->R, b->leaf_boards, n_slots, nullptr, b->leaf_flat, b->leaf_counts, b->leaf_status,
+                             d_planes, b->k, 0, nullptr, flags, stream);
+}
+
 }  // namespace fpc
 
 using namespace fpc;
@@ -1598,27 +1777,47 @@ int fpc_tree_select_leaves(const fpc_tree *t, const fpc_leaf_batch *b, int batch
   if (rc != FPC_OK) return rc;
   if (t->n_games == 0) return FPC_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  const int n_slots = t->n_games * b->L;
   const int blocks = (t->n_games + SEL_WARPS - 1) / SEL_WARPS;
   rc = dispatch(t->R, [&](auto g) {
     leaves_descend_kernel<decltype(g)><<<blocks, SEL_WARPS * 32, 0, st>>>(*t, *b);
     return cuda_check(cudaGetLastError(), "leaves_descend_kernel launch");
   });
   if (rc != FPC_OK) return rc;
-  if (batch_rotation) {
-    rc = fpc_observe(t->R, b->leaf_boards, n_slots, nullptr, b->leaf_flat, b->leaf_counts, b->leaf_status, nullptr,
-                     nullptr, 0, nullptr, 0, stream);
-    if (rc != FPC_OK) return rc;
-    rc = dispatch(t->R, [&](auto g) {
-      leaves_batch_k_kernel<decltype(g)><<<1, 1024, 0, st>>>(*b, n_slots);
-      return cuda_check(cudaGetLastError(), "leaves_batch_k_kernel launch");
-    });
-    if (rc != FPC_OK) return rc;
-    return fpc_observe_tracked(track, t->R, b->leaf_boards, n_slots, nullptr, nullptr, nullptr, nullptr, d_planes, b->k, 0,
-                               nullptr, flags, stream);
-  }
-  return fpc_observe_tracked(track, t->R, b->leaf_boards, n_slots, nullptr, b->leaf_flat, b->leaf_counts, b->leaf_status,
-                             d_planes, b->k, 0, nullptr, flags, stream);
+  return observe_slots(t, b, batch_rotation, d_planes, flags, track, stream);
+}
+
+int fpc_tree_select_gumbel_leaves(const fpc_tree *t, const fpc_gumbel *gb, const fpc_leaf_batch *b, int32_t *d_issued,
+                                  double *d_node_value, int batch_rotation, float *d_planes, int flags,
+                                  fpc_dense_track *track, void *stream) {
+  int rc = check_tree(t, "fpc_tree_select_gumbel_leaves");
+  if (rc == FPC_OK) rc = check_gumbel(t, gb, "fpc_tree_select_gumbel_leaves");
+  if (rc == FPC_OK) rc = check_batch(t, b, "fpc_tree_select_gumbel_leaves");
+  if (rc != FPC_OK) return rc;
+  if (t->n_games == 0) return FPC_OK;
+  if (!d_issued) return fail(FPC_ERR_ARG, "fpc_tree_select_gumbel_leaves: null issued");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int blocks = (t->n_games + SEL_WARPS - 1) / SEL_WARPS;
+  rc = dispatch(t->R, [&](auto g) {
+    if (d_node_value)
+      gumbel_leaves_descend_kernel<decltype(g), true><<<blocks, SEL_WARPS * 32, 0, st>>>(*t, *gb, *b, d_issued, d_node_value);
+    else
+      gumbel_leaves_descend_kernel<decltype(g), false><<<blocks, SEL_WARPS * 32, 0, st>>>(*t, *gb, *b, d_issued, nullptr);
+    return cuda_check(cudaGetLastError(), "gumbel_leaves_descend_kernel launch");
+  });
+  if (rc != FPC_OK) return rc;
+  return observe_slots(t, b, batch_rotation, d_planes, flags, track, stream);
+}
+
+int fpc_tree_gumbel_result_leaves(const fpc_tree *t, const fpc_gumbel *gb, const int32_t *d_issued, int32_t *d_action,
+                                  float *d_policy, void *stream) {
+  int rc = check_tree(t, "fpc_tree_gumbel_result_leaves");
+  if (rc == FPC_OK) rc = check_gumbel(t, gb, "fpc_tree_gumbel_result_leaves");
+  if (rc != FPC_OK) return rc;
+  if (t->n_games == 0) return FPC_OK;
+  if (!d_issued || !d_action || !d_policy) return fail(FPC_ERR_ARG, "fpc_tree_gumbel_result_leaves: null issued / action / policy");
+  const int blocks = (t->n_games + SEL_WARPS - 1) / SEL_WARPS;
+  tree_gumbel_result_leaves_kernel<<<blocks, SEL_WARPS * 32, 0, (cudaStream_t)stream>>>(*t, *gb, d_issued, d_action, d_policy);
+  return cuda_check(cudaGetLastError(), "tree_gumbel_result_leaves_kernel launch");
 }
 
 int fpc_tree_expand_backup_leaves(const fpc_tree *t, const fpc_leaf_batch *b, const float *d_logits,

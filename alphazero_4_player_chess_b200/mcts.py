@@ -29,7 +29,7 @@ class BatchedMCTS:
                  batch_rotation: bool = False, node_cap: int | None = None, cuda_graph: bool = False,
                  reuse_tree: bool = False, leaves_per_game: int = 1, virtual_loss: int = 1, root_noise: bool = False,
                  noise_seed: int = 0, gumbel: bool = False, gumbel_seed: int = 0, gumbel_considered: int = 16,
-                 gumbel_scale: float = 1.0, gumbel_interior: bool = False):
+                 gumbel_scale: float = 1.0, gumbel_interior: bool = False, gumbel_leaves: int = 1):
         """args: the reference's dict (`alphazero.py:291-306`): uses "C" and "num_searches".
         batch_rotation=True reproduces the reference bit for bit (a whole leaf batch is rotated by the
         colour of its first expandable state); False rotates every leaf by its own side to move.
@@ -60,7 +60,16 @@ class BatchedMCTS:
         the child maximising pi'_i - N_i / (1 + sum_j N_j), pi' = softmax(logits + sigma(completed Q)) computed at that
         node with its own network value (`fpc_tree_select_gumbel_interior`), instead of SelectChild.  It costs one f64
         per node slot (`node_value`, n_games x node_cap): 25 MB at 1,024 games x 32 simulations, 403 MB at 8,192 x 64.
-        gumbel_interior=False changes nothing."""
+        gumbel_interior=False changes nothing.
+        gumbel_leaves=L > 1 (with gumbel=True, root-only or interior) runs the Gumbel search leaf-parallel
+        (`fpc_tree_select_gumbel_leaves`): num_searches / L batches of n_games * L network rows, the L slots of a game
+        taking the halving schedule's next L root visits, each continued below its root child with `virtual_loss` (or
+        the interior step over the same effective statistics).  The schedule is indexed by `issued`, the visits it
+        handed out per root child, so a collision (counted in `collisions`) costs that child a visit but never derails
+        the schedule, and `gumbel_result` keeps the children with the most issued visits.  The first batch expands the
+        root (one leaf, L - 1 collisions), so the schedule is planned for num_searches - L root visits: at 32
+        simulations and L = 8 the root gets at most 24, against 31 at L = 1.  L must divide num_searches.
+        gumbel_leaves=1 is the sequential Gumbel search, call for call."""
         self.geom = GEOMETRIES[R]
         self.R, self.n = R, int(n_games)
         self.net = neural_net
@@ -73,6 +82,13 @@ class BatchedMCTS:
         self._graph = None
         self.L = _lib.lib()
         sims = int(args["num_searches"])
+        self.gumbel_leaves = int(gumbel_leaves)
+        if not 1 <= self.gumbel_leaves <= MAX_LEAVES_PER_GAME:
+            raise ValueError(f"gumbel_leaves must be in 1 .. {MAX_LEAVES_PER_GAME}, got {self.gumbel_leaves}")
+        if self.gumbel_leaves > 1 and not gumbel:
+            raise ValueError("gumbel_leaves > 1 needs gumbel=True")
+        if sims % self.gumbel_leaves:
+            raise ValueError(f"gumbel_leaves={self.gumbel_leaves} does not divide num_searches={sims}")
         self.leaves, self.virtual_loss = int(leaves_per_game), int(virtual_loss)
         if not 1 <= self.leaves <= MAX_LEAVES_PER_GAME:
             raise ValueError(f"leaves_per_game must be in 1 .. {MAX_LEAVES_PER_GAME}, got {self.leaves}")
@@ -80,6 +96,10 @@ class BatchedMCTS:
             raise ValueError(f"virtual_loss must be at least 1, got {self.virtual_loss}")
         if sims % self.leaves:
             raise ValueError(f"leaves_per_game={self.leaves} does not divide num_searches={sims}")
+        gumbel_refused = ((reuse_tree, "reuse_tree=True"), (root_noise, "root_noise=True"),
+                          (self.leaves > 1, "leaves_per_game > 1"))
+        if self.gumbel_leaves > 1:
+            self.leaves = self.gumbel_leaves  # the leaf batch below, with the Gumbel select (`select`)
         self._open = False  # a leaf batch was selected and not yet expanded: its in_flight marks are still set
         reuse = 2 if reuse_tree else 1
         self.node_cap = int(node_cap) if node_cap else 1 + reuse * NODES_PER_SIM * sims
@@ -146,8 +166,7 @@ class BatchedMCTS:
         if self.gumbel_interior and not self.gumbel:
             raise ValueError("gumbel_interior=True needs gumbel=True")
         if self.gumbel:
-            for refused, what in ((reuse_tree, "reuse_tree=True"), (root_noise, "root_noise=True"),
-                                  (self.leaves > 1, "leaves_per_game > 1")):
+            for refused, what in gumbel_refused:
                 if refused:
                     raise ValueError(f"gumbel=True does not combine with {what}")
             # fixed addresses: a captured CUDA graph of simulate() reads the keys and writes root_value in place
@@ -156,13 +175,17 @@ class BatchedMCTS:
             gd = GumbelDesc()
             gd.seed = int(gumbel_seed) & (2**64 - 1)
             gd.keys, gd.root_value = self.gumbel_keys.data_ptr(), self.root_value.data_ptr()
-            gd.max_considered, gd.n_sims = int(gumbel_considered), max(0, sims - 1)
+            # the schedule's root visits: the first batch expands the root and spends all its L slots there
+            gd.max_considered, gd.n_sims = int(gumbel_considered), max(0, sims - self.leaves)
             gd.scale, gd.c_visit, gd.c_scale = float(gumbel_scale), GUMBEL_C_VISIT, GUMBEL_C_SCALE
             self.gumbel_desc = gd
             if self.gumbel_interior:
                 # each node's network value, cached by the select at the node's first pass; every entry is written
                 # before it is read, so it needs no initialisation (fixed address, like root_value)
                 self.node_value = torch.empty((n, nc), dtype=torch.float64, device=dev)
+            if self.batch is not None:
+                # I_i: the root visits the halving schedule issued to child i since the reset (fixed address)
+                self.issued = torch.zeros((n, FPC_MAX_MOVES), **i32)
             self._gumbel_searches = 0
         self.root_noise = bool(root_noise)
         if self.root_noise:
@@ -185,6 +208,8 @@ class BatchedMCTS:
             self._open = False
         if self.batch is not None:
             self.collisions.zero_()
+            if self.gumbel:
+                self.issued.zero_()  # a new root: the schedule starts again
         if self.root_noise:
             self.noise_done.zero_()  # a new root: noised again by the next add_root_noise
 
@@ -227,7 +252,14 @@ class BatchedMCTS:
         # the planes tensor is resident and only read by the network between selects: after the first full encode
         # through this instance's handle it is updated in place (FPC_FLAG_INCREMENTAL)
         with torch.cuda.device(self.device):
-            if self.gumbel_interior:
+            if self.gumbel and self.batch is not None:
+                node_value = self.node_value.data_ptr() if self.gumbel_interior else None
+                check(self.L.fpc_tree_select_gumbel_leaves(C.byref(self.desc), C.byref(self.gumbel_desc), C.byref(self.batch),
+                                                           self.issued.data_ptr(), node_value, int(self.batch_rotation),
+                                                           self.planes.data_ptr(), _lib.FLAG_INCREMENTAL, self._track,
+                                                           self._stream()))
+                self._open = True
+            elif self.gumbel_interior:
                 check(self.L.fpc_tree_select_gumbel_interior(C.byref(self.desc), C.byref(self.gumbel_desc),
                                                              self.node_value.data_ptr(), int(self.batch_rotation),
                                                              self.planes.data_ptr(), _lib.FLAG_INCREMENTAL,
@@ -264,14 +296,20 @@ class BatchedMCTS:
         """(action [n] i32, policy [n, FPC_MAX_MOVES] f32) of the current search (`fpc_tree_gumbel_result`): the flat
         action of the root child the halving leaves standing, and the improved policy softmax(logits + sigma(completed
         Q)) with its columns aligned with root_children().  A root without children gets action -1 and a zero row; a
-        dropped game's result comes from the visits it has."""
+        dropped game's result comes from the visits it has.  With gumbel_leaves > 1 the survivors are the children with
+        the most issued visits (`fpc_tree_gumbel_result_leaves`)."""
         if not self.gumbel:
             raise _lib.FpcError("gumbel_result() needs BatchedMCTS(..., gumbel=True)")
         action = torch.empty(self.n, dtype=torch.int32, device=self.device)
         policy = torch.empty((self.n, FPC_MAX_MOVES), dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
-            check(self.L.fpc_tree_gumbel_result(C.byref(self.desc), C.byref(self.gumbel_desc), action.data_ptr(),
-                                                policy.data_ptr(), self._stream()))
+            if self.batch is not None:
+                check(self.L.fpc_tree_gumbel_result_leaves(C.byref(self.desc), C.byref(self.gumbel_desc),
+                                                           self.issued.data_ptr(), action.data_ptr(), policy.data_ptr(),
+                                                           self._stream()))
+            else:
+                check(self.L.fpc_tree_gumbel_result(C.byref(self.desc), C.byref(self.gumbel_desc), action.data_ptr(),
+                                                    policy.data_ptr(), self._stream()))
         return action, policy
 
     def sample_root(self, seed: int, keys, temperature: float) -> torch.Tensor:

@@ -54,7 +54,7 @@ class SelfPlay:
                  batch_rotation: bool = False, reuse_tree: bool = False, leaves_per_game: int = 1,
                  virtual_loss: int = 1, root_noise: bool = False, noise_seed: int = 0, gumbel: bool = False,
                  gumbel_seed: int = 0, gumbel_considered: int = 16, gumbel_scale: float = 1.0,
-                 gumbel_interior: bool = False, sample_seed: int = 0):
+                 gumbel_interior: bool = False, gumbel_leaves: int = 1, sample_seed: int = 0):
         """args: the reference's dict (`alphazero.py:291-306`); uses C, num_searches, temperature,
         max_game_length, heuristic_weight.  reuse_tree=True keeps the played move's subtree for the next move's search
         (`BatchedMCTS.advance`) where the reference starts every move from a fresh root: num_searches simulations are
@@ -67,7 +67,9 @@ class SelfPlay:
         search (BatchedMCTS), keyed like the noise by g * max_game_length + t; every move plays the action of
         `gumbel_result` (temperature is then unused) and the replay's policy targets are its improved policy, kept in
         `hist_policy` and returned as replay["child_policy"].  gumbel_interior: Gumbel MuZero's interior selection below
-        the Gumbel root (BatchedMCTS); keys, actions and policy targets are as with gumbel alone.  sample_seed: the seed of
+        the Gumbel root (BatchedMCTS); keys, actions and policy targets are as with gumbel alone.  gumbel_leaves: the
+        leaf-parallel Gumbel search (BatchedMCTS), num_searches / L network batches of n_games * L rows per move, with
+        `virtual_loss` below the root.  sample_seed: the seed of
         play_games' keyed move sampling (`BatchedMCTS.sample_root`); play() samples with torch's RNG and ignores it."""
         self.geom = GEOMETRIES[R]
         self.R, self.n, self.args = R, int(n_games), args
@@ -78,7 +80,7 @@ class SelfPlay:
                                 reuse_tree=self.reuse_tree, leaves_per_game=leaves_per_game,
                                 virtual_loss=virtual_loss, root_noise=root_noise, noise_seed=noise_seed, gumbel=gumbel,
                                 gumbel_seed=gumbel_seed, gumbel_considered=gumbel_considered, gumbel_scale=gumbel_scale,
-                                gumbel_interior=gumbel_interior)
+                                gumbel_interior=gumbel_interior, gumbel_leaves=gumbel_leaves)
         self.start = torch.as_tensor(start_record, dtype=torch.uint8)
         self.sample_seed = int(sample_seed)
         self.next_game = 0  # the first game id of the next play_games(first_game=None)

@@ -453,6 +453,51 @@ int fpc_tree_gumbel_result(const fpc_tree *t, const fpc_gumbel *gb, int32_t *d_a
 int fpc_tree_select_gumbel_interior(const fpc_tree *t, const fpc_gumbel *gb, double *d_node_value, int batch_rotation,
                                     float *d_planes, int flags, fpc_dense_track *track, void *stream);
 
+/* ---- leaf-parallel Gumbel search: several halving steps per game in one network batch ------------------------------
+ *
+ * The Gumbel search (root-only, or with the interior step when d_node_value is not NULL) over the leaf batch above:
+ * num_searches / L batches of n_games*L network rows, slot s = g*L + j, slot kinds LEAF / COLLISION / EMPTY, committed
+ * by fpc_tree_expand_backup_leaves unchanged.  Within one round of a halving phase the schedule visits distinct root
+ * children, so those visits share a batch with no virtual loss at the root.  One more per-game array:
+ *   d_issued [n_games][FPC_MAX_MOVES] i32: I_i, the LEAF and COLLISION slots that took root child i since the tree's
+ *   reset.  At L = 1, and in any batch without collisions, I_i = N_i (visits - 1).  The caller zeroes it whenever it
+ *   resets the tree, as it zeroes in_flight once.
+ *
+ * fpc_tree_select_gumbel_leaves, game g (a dropped game: every slot EMPTY):
+ *   1. root not expanded: every slot reaches the root, one LEAF and L-1 COLLISIONs (the leaf batch's first-batch rule);
+ *      d_issued is not touched;
+ *   2. root expanded: score_i = max(-1e9, g_i + l_i + sigma_i) is computed ONCE per batch from the committed statistics,
+ *      exactly as fpc_tree_select_gumbel computes it (N_i, Nmax committed; root_value[g] = value_sum[0] when s == 0).
+ *      Then for slots j = 0 .. L-1 in ascending order: t = sum_i I_i, cv(t) from the schedule above planned for
+ *      gb->n_sims (a caller plans num_searches - L: the first batch expands the root); the slot's root child is the
+ *      first maximum of score_i over {i : I_i == cv(t)}; I_i += 1; the descent continues below that child with the leaf
+ *      batch's rule: effective statistics N + VL*in_flight and W - VL*in_flight, an endpoint with in_flight > 0 is a
+ *      COLLISION, in_flight += 1 along the whole path, the root included.  The schedule runs on I, not on N, so a
+ *      collision only lowers N_i and the candidate set is never empty; if it is anyway, or any later step of the
+ *      descent fails, the leaf batch's descent-error rule applies (the error bits of fpc_tree_select, e.g. bit 2; the
+ *      game is dropped; this slot and every later one are EMPTY) and the failed slot adds nothing to I;
+ *   3. below the root with d_node_value: the interior step of fpc_tree_select_gumbel_interior over the effective
+ *      statistics (N_eff, q from W_eff, s_eff, Nmax_eff).  x's network value follows the COMMITTED s = sum (visits - 1)
+ *      of x's children: s == 0: u = value_sum[x] and d_node_value[g][x] = value_sum[x] is written; else u =
+ *      d_node_value[g][x].  Pending descents do not touch value_sum, so the caching argument above still holds.  Without
+ *      d_node_value the descent below the root is Node::SelectChild with virtual loss, as in fpc_tree_select_leaves;
+ *   4. the rules kernel, the encoder, batch_rotation, leaf[g] and collisions as in fpc_tree_select_leaves.
+ * Sums, maxima and minima run in the Gumbel order (lane i % 32, lanes ascending, then the xor butterfly 16 .. 1) and no
+ * product is fused into a sum.  Called at L = 1 this select writes what fpc_tree_select_gumbel (or _interior) writes in
+ * every tree array.
+ *
+ * fpc_tree_gumbel_result_leaves: fpc_tree_gumbel_result's recipe with the survivors {i : I_i == max I} in place of
+ * {i : N_i == Nmax}, so a visit lost to a collision cannot demote a survivor; the improved policy softmax(l + sigma)
+ * comes from the committed statistics, unchanged.  It equals fpc_tree_gumbel_result whenever I == N.
+ *
+ * Every refusal of fpc_tree_select_gumbel and of fpc_tree_select_leaves, null d_issued, and for the result null
+ * d_action / d_policy are FPC_ERR_ARG, before any launch. */
+int fpc_tree_select_gumbel_leaves(const fpc_tree *t, const fpc_gumbel *gb, const fpc_leaf_batch *b, int32_t *d_issued,
+                                  double *d_node_value, int batch_rotation, float *d_planes, int flags,
+                                  fpc_dense_track *track, void *stream);
+int fpc_tree_gumbel_result_leaves(const fpc_tree *t, const fpc_gumbel *gb, const int32_t *d_issued, int32_t *d_action,
+                                  float *d_policy, void *stream);
+
 /* ---- Keyed move sampling from the root's visit counts ---------------------------------------------------------------
  *
  * The played move of the reference's self-play (alphazero.py:108-118: probs = visits / sum, probs ** (1/temperature),
