@@ -17,7 +17,9 @@
 namespace fpc {
 
 constexpr int SEL_WARPS = 4;
-constexpr int ERR_NODE_CAP = 1, ERR_BOARD_CAP = 2, ERR_NO_CHILD = 4, ERR_MOVE = 8;
+constexpr int ERR_NODE_CAP = 1, ERR_BOARD_CAP = 2, ERR_NO_CHILD = 4, ERR_MOVE = 8, ERR_OVERFLOW = 16;
+// a leaf the network evaluates: in progress, with its whole legal list
+constexpr int NOT_EXPANDABLE = FPC_STATUS_RESULT_MASK | FPC_STATUS_OVERFLOW;
 
 // A fresh root for game g: node 0 = `root` (one record), visit_count 1, no children; per-game state cleared.  Run by
 // every thread of one CTA.
@@ -369,7 +371,7 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) tree_descend_kernel(const fpc_
 
 // The reference rotates a whole leaf batch by the colour of states[0] (src/cpp/board.cpp:354-355,
 // mcts.py:69), states = the leaves that are NOT terminal (mcts.py:18-26 drops terminal leaves before the batch is
-// built): k[g] <- side to move of the first leaf whose status (already computed) says IN_PROGRESS.
+// built): k[g] <- side to move of the first leaf whose status (already computed) says IN_PROGRESS without overflow.
 template <class G>
 __global__ void __launch_bounds__(1024) tree_batch_k_kernel(const fpc_tree T) {
   __shared__ int first;
@@ -377,7 +379,7 @@ __global__ void __launch_bounds__(1024) tree_batch_k_kernel(const fpc_tree T) {
   __syncthreads();
   int mine = 0x7fffffff;
   for (int g = threadIdx.x; g < T.n_games; g += blockDim.x)
-    if (T.leaf[g] >= 0 && (T.leaf_status[g] & FPC_STATUS_RESULT_MASK) == 0) {
+    if (T.leaf[g] >= 0 && (T.leaf_status[g] & NOT_EXPANDABLE) == 0) {
       mine = g;
       break;
     }
@@ -427,6 +429,13 @@ __global__ void __launch_bounds__(EXP_THREADS, 8) tree_expand_backup_kernel(cons
     prev_in[q] = (i > 0 && i < MAX_MOVES) ? T.leaf_flat[(size_t)g * MAX_MOVES + i - 1] : -1;
   }
   if (leaf < 0) return;
+  if (status & FPC_STATUS_OVERFLOW) {  // a partial legal list: no children, no backup, the game drops
+    if (tid == 0) {
+      T.error[g] |= ERR_OVERFLOW;
+      T.dropped[g] = 1;
+    }
+    return;
+  }
   const size_t slab = (size_t)g * T.node_cap;
   // The latency-bound tail is prepared while the logits stream: one thread (of the last warp) walks the leaf's ancestors
   // now -- a chain of dependent loads -- so that the backup at the end is one parallel round of updates; thread 0 has
@@ -759,7 +768,8 @@ __global__ void __launch_bounds__(SEL_WARPS * 32) leaves_descend_kernel(const fp
   leaves_select<G>(T, B, g, lane, recs[wib], paths[wib], [](int &, int &, int &, int &, int &) { return 0; });
 }
 
-// tree_batch_k_kernel over the slots: k <- side to move of the first LEAF slot whose status says IN_PROGRESS
+// tree_batch_k_kernel over the slots: k <- side to move of the first LEAF slot whose status says IN_PROGRESS without
+// overflow
 template <class G>
 __global__ void __launch_bounds__(1024) leaves_batch_k_kernel(const fpc_leaf_batch B, int n_slots) {
   __shared__ int first;
@@ -767,7 +777,7 @@ __global__ void __launch_bounds__(1024) leaves_batch_k_kernel(const fpc_leaf_bat
   __syncthreads();
   int mine = 0x7fffffff;
   for (int s = threadIdx.x; s < n_slots; s += blockDim.x)
-    if (B.slot_kind[s] == FPC_SLOT_LEAF && (B.leaf_status[s] & FPC_STATUS_RESULT_MASK) == 0) {
+    if (B.slot_kind[s] == FPC_SLOT_LEAF && (B.leaf_status[s] & NOT_EXPANDABLE) == 0) {
       mine = s;
       break;
     }
@@ -789,7 +799,7 @@ __global__ void __launch_bounds__(EXP_THREADS, 8) leaves_priors_kernel(const fpc
   __shared__ double s_msum;
   const size_t s = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (B.slot_kind[s] != FPC_SLOT_LEAF || (B.leaf_status[s] & FPC_STATUS_RESULT_MASK) != 0) return;
+  if (B.slot_kind[s] != FPC_SLOT_LEAF || (B.leaf_status[s] & NOT_EXPANDABLE) != 0) return;
   const int cnt = B.leaf_counts[s];
   const int k = B.k[s] & 3;
   constexpr int PER = (MAX_MOVES + EXP_THREADS - 1) / EXP_THREADS;
@@ -893,7 +903,7 @@ __global__ void __launch_bounds__(LB_THREADS) leaves_commit_kernel(const fpc_tre
   __shared__ unsigned long long s_ent[LB_ENTRIES];
   __shared__ int s_node[FPC_MAX_LEAVES_PER_GAME], s_cnt[FPC_MAX_LEAVES_PER_GAME], s_base[FPC_MAX_LEAVES_PER_GAME];
   __shared__ float s_val[FPC_MAX_LEAVES_PER_GAME];
-  __shared__ int8_t s_what[FPC_MAX_LEAVES_PER_GAME];  // 0 no backup, 1 terminal LEAF, 2 LEAF in progress
+  __shared__ int8_t s_what[FPC_MAX_LEAVES_PER_GAME];  // 0 no backup, 1 terminal LEAF, 2 LEAF in progress, 3 overflow
   __shared__ int s_ne;
   const int g = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int L = B.L;
@@ -901,11 +911,11 @@ __global__ void __launch_bounds__(LB_THREADS) leaves_commit_kernel(const fpc_tre
   if (tid == 0) s_ne = 0;
   for (int j = tid; j < L; j += LB_THREADS) {
     const int kind = B.slot_kind[s0 + j];
-    const int result = B.leaf_status[s0 + j] & FPC_STATUS_RESULT_MASK;
+    const int status = B.leaf_status[s0 + j], result = status & FPC_STATUS_RESULT_MASK;
     int what = 0;
     float v = 0.0f;
     if (kind == FPC_SLOT_LEAF) {
-      what = result ? 1 : 2;
+      what = (status & FPC_STATUS_OVERFLOW) ? 3 : result ? 1 : 2;
       v = result == 3 ? 0.0f : result ? -1.0f : values[s0 + j];
     }
     s_node[j] = kind == FPC_SLOT_EMPTY ? -1 : B.slot_node[s0 + j];
@@ -930,10 +940,11 @@ __global__ void __launch_bounds__(LB_THREADS) leaves_commit_kernel(const fpc_tre
     int nn = T.n_nodes[g], err = 0, drop = 0;
     for (int j = 0; j < L; ++j) {
       s_base[j] = -1;
-      drop |= s_what[j] == 1;
+      drop |= s_what[j] == 1 || s_what[j] == 3;
+      if (s_what[j] == 3) err |= ERR_OVERFLOW;
       if (s_what[j] != 2) continue;
       if (nn + s_cnt[j] > T.node_cap) {
-        err = ERR_NODE_CAP;
+        err |= ERR_NODE_CAP;
       } else {
         s_base[j] = nn;
         nn += s_cnt[j];
@@ -974,7 +985,7 @@ __global__ void __launch_bounds__(LB_THREADS) leaves_commit_kernel(const fpc_tre
   }
   // the paths, one thread per slot: clear the marks; gather the backup entries of the LEAF slots
   for (int j = tid; j < L; j += LB_THREADS) {
-    const bool backup = s_what[j] != 0;
+    const bool backup = s_what[j] == 1 || s_what[j] == 2;
     unsigned par = 0;
     for (int node = s_node[j]; node >= 0; node = T.parent[slab + node], par ^= 1u) {
       B.in_flight[slab + node] = 0;
@@ -989,7 +1000,7 @@ __global__ void __launch_bounds__(LB_THREADS) leaves_commit_kernel(const fpc_tre
   if (ne > LB_ENTRIES) {  // Node::Backpropagate slot by slot
     if (tid == 0)
       for (int j = 0; j < L; ++j) {
-        if (!s_what[j]) continue;
+        if (s_what[j] != 1 && s_what[j] != 2) continue;
         double v = (double)s_val[j];
         for (int node = s_node[j]; node >= 0; node = T.parent[slab + node]) {
           T.value_sum[slab + node] += v;

@@ -539,6 +539,14 @@ __device__ void rules_warp(const ObserveParams &P, RulesScratch<G> &s, const int
           }
         }
         const int cnt = lo.cnt + hi.cnt;  // <= 26: two rays of at most 13 squares
+        // a king capture counts whether or not this round fits the buffer (only the last square of a run can hold a piece)
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const Run2 &r = h ? hi : lo;
+          const int to0 = from + r.delta * (r.first + 1);
+          const int last = r.promo ? to0 : to0 + r.delta * (r.cnt - 1);
+          takes_king |= r.cnt > 0 && (last == ek1 || last == ek2);
+        }
         int excl = 0, total = 0;
 #pragma unroll
         for (int bit = 0; bit < 5; ++bit) {
@@ -558,8 +566,6 @@ __device__ void rules_warp(const ObserveParams &P, RulesScratch<G> &s, const int
             const int to0 = from + r.delta * (r.first + 1);
             uint32_t mv = pack_compact<G>(from, to0, r.plane0 + r.first, r.promo ? KNIGHT : NO_PIECE, 0);
             const uint32_t inc = r.promo ? 1u << 14 : KEY_STEP + (uint32_t)r.delta;
-            const int last = r.promo ? to0 : to0 + r.delta * (r.cnt - 1);  // only the last square of a run can hold a piece
-            takes_king |= last == ek1 || last == ek2;
             for (int j = 0; j < r.cnt; ++j, mv += inc) s.moves[at++] = mv;
           }
           n_moves += total;

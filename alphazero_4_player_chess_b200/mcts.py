@@ -17,8 +17,9 @@ from . import _lib
 from ._lib import FPC_MAX_MOVES, MAX_LEAVES_PER_GAME, GumbelDesc, LeafBatchDesc, TreeDesc, check
 from .geometry import GEOMETRIES, NUM_STATE_CHANNELS
 
-ERR_NODE_CAP, ERR_BOARD_CAP, ERR_NO_CHILD, ERR_MOVE = 1, 2, 4, 8
-# node slots per simulation: a leaf adds at most FPC_MAX_MOVES children; the legal-move average is ~19-38 at 14x14
+ERR_NODE_CAP, ERR_BOARD_CAP, ERR_NO_CHILD, ERR_MOVE, ERR_OVERFLOW = 1, 2, 4, 8, 16
+# node slots per simulation: a leaf adds at most FPC_MAX_MOVES children; the legal-move average is ~19-38 at 14x14.
+# Crowded positions (100-300 legal moves) outgrow this default within a few simulations: pass node_cap for them.
 NODES_PER_SIM = 96
 # sigma(q) = (GUMBEL_C_VISIT + max N) * GUMBEL_C_SCALE * q: the constants of Danihelka et al. (ICLR 2022) and mctx
 GUMBEL_C_VISIT, GUMBEL_C_SCALE = 50.0, 0.1
@@ -439,7 +440,8 @@ class BatchedMCTS:
     def check_errors(self) -> None:
         e = int(self.error.max().item())
         if e:
-            raise _lib.FpcError(f"tree error bits {e:#x} (1 node_cap, 2 board_cap, 4 no child selectable, 8 move)")
+            raise _lib.FpcError(f"tree error bits {e:#x} (1 node_cap, 2 board_cap, 4 no child selectable, 8 move, "
+                                  f"16 leaf with more than {FPC_MAX_MOVES} legal moves)")
 
     def root_children(self):
         """(flat [n,FPC_MAX_MOVES] i32, visits [n,FPC_MAX_MOVES] i32, prior f32, count [n]) of the root's

@@ -54,7 +54,15 @@ extern "C" {
 #define FPC_STATUS_RESULT_MASK 0x3     /* GameResult: 0 IN_PROGRESS 1 WIN_RY 2 WIN_BG 3 STALEMATE */
 #define FPC_STATUS_IN_CHECK 0x100      /* side to move is in check (set only when it has no legal move) */
 #define FPC_STATUS_CAN_TAKE_KING 0x200 /* some legal move captures a king (SURVEY 8a row 8) */
-#define FPC_STATUS_OVERFLOW 0x400      /* move buffer overflow */
+#define FPC_STATUS_OVERFLOW 0x400      /* more than FPC_MAX_MOVES legal moves (the reference aborts, engine/board.h:482-486).
+                                          Legal moves are counted, not pseudo-legal ones: a position with more than
+                                          FPC_MAX_MOVES pseudo-legal but at most FPC_MAX_MOVES legal moves gets its full
+                                          list.  When set: counts <= FPC_MAX_MOVES; the moves / flat indices listed are a
+                                          strictly ascending subset of the canonical legal list, not necessarily a prefix
+                                          (whole generation rounds that do not fit are dropped); the mask has ones at
+                                          exactly the listed flat indices; FPC_STATUS_CAN_TAKE_KING and FPC_STATUS_CHECK
+                                          are those of the full legal list; the result is IN_PROGRESS unless the mover
+                                          has no king.  The search treats such a leaf as an error (fpc_tree error bit 4). */
 #define FPC_STATUS_FINISHED 0x800      /* playout only: the game in this slot ended and was re-seeded */
 #define FPC_STATUS_CHECK 0x1000        /* side to move is in check (engine/board.cpp:941-960), legal moves or not */
 
@@ -228,7 +236,9 @@ typedef struct fpc_tree {
   int32_t *dropped;       /* 1 once a terminal leaf was reached: the root sits out the remaining
                              simulations (mcts.py:22-23) */
   int32_t *error;         /* bit 0 node_cap exceeded, bit 1 board_cap exceeded, bit 2 no child selectable
-                             (the reference throws, node.cpp:72-75), bit 3 index-built move failed */
+                             (the reference throws, node.cpp:72-75), bit 3 index-built move failed, bit 4 a leaf
+                             with FPC_STATUS_OVERFLOW (its legal list is partial; the reference aborts): the leaf is
+                             left unexpanded, nothing is backed up for it and the game is dropped */
   uint8_t *boards;        /* [n_games][board_cap][record] */
   /* the leaf batch: input of the rules kernel and of the network */
   uint8_t *leaf_boards;   /* [n_games][record] */
@@ -304,6 +314,8 @@ int fpc_tree_expand_backup(const fpc_tree *t, const float *d_logits, const float
  * Expand / backup, game g, slots in ascending j (the outputs of COLLISION and EMPTY slots are ignored):
  *   - LEAF, terminal: Backpropagate(0 | -1); the game is dropped after this batch (its later slots still count: they
  *     ran concurrently);
+ *   - LEAF with FPC_STATUS_OVERFLOW: error bit 4, no backup, no children; the game is dropped after this batch as for
+ *     a terminal leaf.  Such a slot is not the batch_rotation slot either;
  *   - LEAF, in progress: Backpropagate(value), then one child per non-zero prior appended at n_nodes, the priors
  *     bit-identical to fpc_tree_expand_backup's for the same logits, k and legal list.  The node_cap check is made per
  *     slot against the running n_nodes: a slot that does not fit sets error bit 0 and is backed up without children;

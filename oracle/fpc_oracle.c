@@ -437,12 +437,11 @@ static int cmp_key(const void *a, const void *b) {
   return (x[0] > y[0]) - (x[0] < y[0]);
 }
 
-/* src/cpp/board.cpp:94-118 GetLegalMoves, returned in canonical order
- * (ascending flat action index, then promotion type). */
-static int legal_moves(const Geo *g, const uint8_t *b, uint64_t *out, int cap) {
-  uint64_t pseudo[MAX_MOVES], keyed[MAX_MOVES][2];
-  int n = pseudo_moves(g, b, pseudo, MAX_MOVES), k = 0;
-  if (n > MAX_MOVES) abort(); /* engine/board.h:482-486 */
+/* The legal subset of pseudo[0 .. n-1] in canonical order (ascending flat action index, then promotion type);
+ * keyed has room for n entries.  Returns the legal count, writes at most cap moves. */
+static int legal_subset(const Geo *g, const uint8_t *b, const uint64_t *pseudo, int n, uint64_t (*keyed)[2],
+                        uint64_t *out, int cap) {
+  int k = 0;
   for (int i = 0; i < n; ++i)
     if (king_safe_after(g, b, pseudo[i])) {
       keyed[k][0] = (uint64_t)flat_index(g->R, pseudo[i]) * 8 + (uint64_t)MV_PROMO(pseudo[i]);
@@ -452,6 +451,14 @@ static int legal_moves(const Geo *g, const uint8_t *b, uint64_t *out, int cap) {
   qsort(keyed, (size_t)k, sizeof keyed[0], cmp_key);
   for (int i = 0; i < k && i < cap; ++i) out[i] = keyed[i][1];
   return k;
+}
+
+/* src/cpp/board.cpp:94-118 GetLegalMoves, returned in canonical order. */
+static int legal_moves(const Geo *g, const uint8_t *b, uint64_t *out, int cap) {
+  uint64_t pseudo[MAX_MOVES], keyed[MAX_MOVES][2];
+  int n = pseudo_moves(g, b, pseudo, MAX_MOVES);
+  if (n > MAX_MOVES) abort(); /* engine/board.h:482-486 */
+  return legal_subset(g, b, pseudo, n, keyed, out, cap);
 }
 
 /* engine/board.cpp:891-939 GetGameResult under the order-independent contract of SURVEY 8a
@@ -507,6 +514,18 @@ int fpo_pseudo_moves(int R, int IA, const uint8_t *rec, uint64_t *out, int cap) 
 int fpo_legal_moves(int R, int IA, const uint8_t *rec, uint64_t *out, int cap) {
   Geo g = geo(R, IA);
   return legal_moves(&g, rec, out, cap);
+}
+/* fpo_legal_moves without the reference's 300-move buffer: the full canonical legal list of a crowded position (the
+ * reference aborts above 300 pseudo-legal moves; the device rules kernel counts legal moves only).  *n_pseudo = the
+ * pseudo-legal count.  Returns the legal count (at most cap moves written), or -1 above WIDE_MOVES pseudo-legal moves. */
+#define WIDE_MOVES 1024
+int fpo_legal_moves_wide(int R, int IA, const uint8_t *rec, uint64_t *out, int cap, int *n_pseudo) {
+  uint64_t pseudo[WIDE_MOVES], keyed[WIDE_MOVES][2];
+  Geo g = geo(R, IA);
+  int n = pseudo_moves(&g, rec, pseudo, WIDE_MOVES);
+  if (n_pseudo) *n_pseudo = n;
+  if (n > WIDE_MOVES) return -1;
+  return legal_subset(&g, rec, pseudo, n, keyed, out, cap);
 }
 int fpo_is_attacked_by_team(int R, int IA, const uint8_t *rec, int team, int sq) {
   Geo g = geo(R, IA);

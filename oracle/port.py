@@ -33,6 +33,7 @@ def lib():
         L = C.CDLL(build())
         L.fpo_pseudo_moves.argtypes = [C.c_int, C.c_int, _u8p, _u64p, C.c_int]
         L.fpo_legal_moves.argtypes = [C.c_int, C.c_int, _u8p, _u64p, C.c_int]
+        L.fpo_legal_moves_wide.argtypes = [C.c_int, C.c_int, _u8p, _u64p, C.c_int, C.POINTER(C.c_int)]
         L.fpo_is_attacked_by_team.argtypes = [C.c_int, C.c_int, _u8p, C.c_int, C.c_int]
         L.fpo_king_in_check.argtypes = [C.c_int, C.c_int, _u8p, C.c_int]
         L.fpo_is_attacked_by_player.argtypes = [C.c_int, C.c_int, _u8p, C.c_int, C.c_int]
@@ -83,6 +84,16 @@ class Oracle:
         out = np.zeros(300, dtype=np.uint64)
         n = self.L.fpo_legal_moves(self.R, self.IA, np.ascontiguousarray(rec), out, 300)
         return out[:n].copy()
+
+    def legal_moves_wide(self, rec):
+        """(moves, n_pseudo): the full canonical legal list, also where the position has more than 300 pseudo-legal
+        or legal moves (legal_moves aborts there, as the reference does)."""
+        out = np.zeros(1024, dtype=np.uint64)
+        n_pseudo = C.c_int(0)
+        n = self.L.fpo_legal_moves_wide(self.R, self.IA, np.ascontiguousarray(rec), out, len(out), C.byref(n_pseudo))
+        if n < 0:
+            raise ValueError(f"more than {len(out)} pseudo-legal moves ({n_pseudo.value})")
+        return out[:n].copy(), n_pseudo.value
 
     def is_attacked_by_team(self, rec, team, sq) -> bool:
         return bool(self.L.fpo_is_attacked_by_team(self.R, self.IA, np.ascontiguousarray(rec), team, sq))

@@ -22,7 +22,7 @@ import torch
 from oracle.mcts_port import Tree
 
 EMPTY, LEAF, COLLISION = 0, 1, 2
-ERR_NODE_CAP, ERR_BOARD_CAP, ERR_NO_CHILD = 1, 2, 4
+ERR_NODE_CAP, ERR_BOARD_CAP, ERR_NO_CHILD, ERR_OVERFLOW = 1, 2, 4, 16
 
 
 def prepare(t: Tree) -> Tree:
@@ -78,12 +78,17 @@ def select_batch(t: Tree, L: int, vl: int, board_room: int | None = None):
     return slots + [(EMPTY, -1)] * (L - len(slots)), err
 
 
-def expand_backup_batch(t: Tree, slots, results, values, children, node_cap: int | None = None):
+def expand_backup_batch(t: Tree, slots, results, values, children, node_cap: int | None = None, overflow=None):
     """Slots in order; results[j] = GameResult of slot j's board, values[j] its value, children(j) -> (flats, priors)
-    of a leaf in progress.  Returns (error bits, whether the game drops)."""
+    of a leaf in progress, overflow[j] (default all False) whether slot j's board has more than 300 legal moves: such a
+    leaf gets error bit 4, no backup and no children, and the game drops.  Returns (error bits, whether the game drops)."""
     err, drop = 0, False
     for j, (kind, node) in enumerate(slots):
         if kind != LEAF:
+            continue
+        if overflow is not None and overflow[j]:
+            err |= ERR_OVERFLOW
+            drop = True
             continue
         if results[j]:
             t.backpropagate(node, 0.0 if results[j] == 3 else -1.0)
